@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- background-extraction frames/s (and BG-mix clips/s) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1]): the UCF101-shaped set -- 13,320 videos, T ~ U[120,240] frames
@@ -306,6 +306,24 @@ def extraction_leg(leg_name, spec, rank, world, dev, steps, barrier):
 
 
 
+DUMP_BYTES = 60_000_000      # --dump-outputs cap: rank 0's 1,665 backgrounds would be 1.5 GB as float32
+
+
+def dump_outputs(path, out, torch):
+    """Write what the last timed step returned to rank 0 -- its uint8 backgrounds [V, H*W*3] -- for a fixed, seeded sample
+    of videos, as float32 [k, H, W, 3] (exact for uint8) in path/backgrounds.npy: two builds run with the same arguments
+    can then be compared output for output.  Only the headline extraction is dumped; the BG-mix legs write nothing."""
+    import numpy as np
+    V = out.shape[0]
+    k = min(V, DUMP_BYTES // (4 * N_BYTES))
+    sel = np.sort(np.random.default_rng(0).choice(V, k, replace=False))
+    bg = out[torch.from_numpy(sel).to(out.device)].view(k, H, W, 3).float().cpu().numpy()
+    d = pathlib.Path(path)
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / "backgrounds.npy", bg)
+    log(f"dumped the backgrounds of videos {sel.tolist()} (of {V}) to {d / 'backgrounds.npy'}")
+
+
 def time_back_to_back(calls, flush, reps, torch):
     """Median ms per call of `calls` (each on its own input / output buffers, together far larger than L2) enqueued back to
     back inside one CUDA-event bracket, L2 flushed before every bracket: the steady-state cost of a batch in a training loop.
@@ -472,6 +490,9 @@ def run_ours(args):
     Ts = draw_T(rng, V)
     free, _total = torch.cuda.mem_get_info(dev)
     while int(Ts.sum()) * N_BYTES + (4 << 30) > free and V > 16:          # another tenant on the GPU: shrink, say so
+        if args.dump_outputs:
+            raise SystemExit("bench.py --dump-outputs: the shard does not fit in free device memory, and a smaller one "
+                             "would change the inputs the dumped outputs are compared on")
         V //= 2
         Ts = Ts[:V]
     offs = torch.from_numpy(np.concatenate([[0], np.cumsum(Ts)]).astype(np.int64))
@@ -520,6 +541,8 @@ def run_ours(args):
     # spot-check the timed path (outside the timed region) against the definition evaluated with plain torch:
     # (s[(T-1)//2] + s[T//2]) >> 1 over the sorted column -- what np.median(...).astype(uint8) gives
     ok = spot_check(frames, offs, Ts, out, int(np.argmin(Ts)), torch) and spot_check(frames, offs, Ts, out, int(np.argmax(Ts)), torch)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, torch)
 
     # ---- end to end through the C ABI with host buffers ----------------------------------------
     Ve = int(os.environ.get("BGD_BENCH_E2E_VIDEOS", 48))
@@ -858,7 +881,14 @@ def main():
     ap.add_argument("--workload", default=WL_NAME, choices=sorted(WORKLOADS))
     ap.add_argument("--content", default="random", choices=["random", "structured"], help="synthetic frame content of the main leg")
     ap.add_argument("--no-legs", dest="no_legs", action="store_true", help="skip the extra workload legs (hmdb51, sthv2, structured)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="after the timed extraction steps, write what the last one computed (a seeded sample of rank 0's "
+                         "backgrounds, float32) as DIR/backgrounds.npy; the BG-mix legs' outputs are not written")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computes; --impl reference keeps no outputs to write")
     _select_workload(args.workload)
     if args.impl == "reference":
         run_reference(args)

@@ -1,4 +1,3 @@
-import os
 import pathlib
 import sys
 
@@ -13,12 +12,13 @@ GOLDEN = ROOT / "tests" / "golden"
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
+    config.addinivalue_line("markers", "reference: runs the original project's code (its source tree at BGD_REFERENCE_ROOT)")
 
 
 def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.isfile("/root/reference/cil_tools/extract_background.py")
-    skip_ref = pytest.mark.skip(reason="/root/reference not present")
+    from oracle import _ref_import
+    have_ref = _ref_import.available()
+    skip_ref = pytest.mark.skip(reason="the original project's source tree is not present (BGD_REFERENCE_ROOT)")
     for item in items:
         if "reference" in item.keywords and not have_ref:
             item.add_marker(skip_ref)

@@ -98,6 +98,27 @@ def test_reference_splits():
     assert [len(r) for r in s] == [1, 1, 1, 0]
 
 
+@pytest.mark.parametrize("name", CASES)
+def test_stored_reference_video_agrees(name, tmp_path):
+    """The comparison of test_live_reference_agrees on the videos whose reference outputs are stored: the frames are
+    written as an FFV1 video, read back with cv2.VideoCapture as bg_extraction_tmf reads them (extract_background.py:
+    42-75), and the restatement of the decoded frames must give the reference's output."""
+    import cv2
+    from oracle import gen_golden
+    interval, max_frames = (int(v) for v in _NPZ[name + "/params"])
+    vid = str(tmp_path / "v.avi")
+    gen_golden.write_ffv1(vid, _NPZ[name + "/frames"])
+    cap = cv2.VideoCapture(vid)
+    decoded = []
+    ok, f = cap.read()
+    while ok:
+        decoded.append(f)
+        ok, f = cap.read()
+    cap.release()
+    np.testing.assert_array_equal(mo.bg_extraction_tmf_frames(np.array(decoded), interval, max_frames),
+                                  _NPZ[name + "/expected"])
+
+
 @pytest.mark.reference
 def test_live_reference_agrees(tmp_path):
     """Build container only: run the reference itself on a fresh random video."""

@@ -66,6 +66,22 @@ def test_against_numpy(T, avg):
         np.testing.assert_array_equal(so.cast_u8(got), exp.astype(np.uint8))
 
 
+@pytest.mark.parametrize("name", CASES)
+def test_stored_reference_file_agrees(name, tmp_path):
+    """The comparison of test_reference_function_end_to_end on the folders whose reference outputs are stored: the
+    restatement under the stored torch seed, written as sim_cam_motion_bg_extract writes it (:99, one channel swap), is
+    the reference's file byte for byte."""
+    import cv2
+    import torch
+    interval, max_frames, avg, seed = (int(v) for v in _NPZ[name + "/params"])
+    torch.manual_seed(seed)
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        img = so.sim_cam_background(_NPZ[name + "/frames"], interval, max_frames, avg)
+    assert cv2.imwrite(str(tmp_path / "o.jpg"), cv2.cvtColor(img, cv2.COLOR_BGR2RGB))
+    assert (tmp_path / "o.jpg").read_bytes() == _NPZ[name + "/jpeg"].tobytes()
+
+
 @pytest.mark.reference
 def test_reference_function_end_to_end(tmp_path):
     import cv2
