@@ -32,6 +32,13 @@ class RaggedSlot(_c.Structure):
                 ("xtab", _c.c_int32), ("ytab", _c.c_int32), ("kx", _c.c_int32), ("ky", _c.c_int32)]
 
 
+class CropDesc(_c.Structure):
+    """``bgd_crop_desc`` of include/bgdebias.h (48 bytes)."""
+    _fields_ = [("offset", _c.c_int64), ("H", _c.c_int32), ("W", _c.c_int32), ("top", _c.c_int32), ("left", _c.c_int32),
+                ("h", _c.c_int32), ("w", _c.c_int32), ("xtab", _c.c_int32), ("ytab", _c.c_int32), ("kx", _c.c_int32),
+                ("ky", _c.c_int32)]
+
+
 _ragged_common = [_c.c_int64, _c.c_int64, _c.c_int64, _c.c_int64,            # B, T, H, W
                   _vp, _vp, _c.c_int64, _vp,                                 # pool, slots, P, tables
                   _vp, _vp, _vp, _vp]                                        # bg_idx, top, left, apply
@@ -62,6 +69,8 @@ SIGNATURES = {
     "bgd_aa_resize_u8_f32": (_c.c_int, [_vp, _c.POINTER(RaggedSlot), _vp, _vp, _vp]),
     "bgd_bgmix_blend_ragged_f32": (_c.c_int, [_vp] + _ragged_common + [_vp, _f32p, _f32p, _c.c_double, _c.c_int, _vp, _vp]),
     "bgd_bgmix_blend_ragged_normfg_f32": (_c.c_int, [_vp] + _ragged_common + [_f32p, _f32p, _c.c_double, _c.c_int, _vp, _vp]),
+    "bgd_resized_crop_aa_u8_f32": (_c.c_int, [_vp, _c.c_int64, _vp, _c.c_int64, _vp, _c.c_int64, _c.c_int64, _c.c_int64,
+                                              _vp, _vp]),
     "bgd_resize_bilinear_u8": (_c.c_int, [_vp, _c.c_int64, _i64p, _c.c_int64, _c.c_int64, _c.c_int64, _c.c_int64, _vp, _vp]),
     "bgd_bgmix_resize_blend_f32_host": (_c.c_int, [_vp, _c.c_int64, _i64p, _c.c_int64, _c.c_int64, _c.c_int64, _c.c_int64,
                                                    _vp, _c.c_int64, _c.c_int64, _c.c_int64, _vp, _vp, _vp, _vp, _vp,

@@ -594,6 +594,16 @@ int bgd_bgmix_blend_ragged_normfg_f32(const float *d_fg_norm, int64_t B, int64_t
                                nullptr, h_bg_mean, h_bg_std, alpha, layout, d_out, static_cast<cudaStream_t>(stream));
 }
 
+int bgd_resized_crop_aa_u8_f32(const uint8_t *d_src, int64_t src_bytes, const bgd_crop_desc *h_desc, int64_t n,
+                               const int32_t *d_tables, int64_t table_words, int64_t out_h, int64_t out_w, float *d_out,
+                               void *stream)
+{
+    DeviceProps dp;
+    if (int rc = current_device_props(&dp)) return rc;
+    return launch_resized_crop_aa(d_src, src_bytes, h_desc, n, d_tables, table_words, out_h, out_w, d_out,
+                                  static_cast<cudaStream_t>(stream));
+}
+
 int bgd_resize_bilinear_u8(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t B, int64_t T, int64_t H,
                            int64_t W, uint8_t *d_out, void *stream)
 {

@@ -73,6 +73,9 @@ int launch_bgmix_ragged(const uint8_t *d_fg, const float *d_fg_norm, int64_t B, 
                         const float *d_lut, const float *h_mean, const float *h_std, double alpha, int layout, float *d_out,
                         cudaStream_t stream);
 int launch_aa_resize(const uint8_t *d_img, const bgd_ragged_slot *h_slot, const int32_t *d_tables, float *d_out, cudaStream_t stream);
+int launch_resized_crop_aa(const uint8_t *d_src, int64_t src_bytes, const bgd_crop_desc *h_desc, int64_t n,
+                           const int32_t *d_tables, int64_t table_words, int64_t out_h, int64_t out_w, float *d_out,
+                           cudaStream_t stream);
 int launch_sum_f32(const float *d_x, int64_t n, double *d_sum, cudaStream_t stream);
 int launch_nan_reduce(const float *d_frames, int64_t T, int64_t N, int avg_method, int zero_is_missing, uint8_t *d_out_u8,
                       float *d_out_f32, cudaStream_t stream);

@@ -26,6 +26,7 @@
 //
 // Blend arithmetic as in bgmix.cu (each operation rounded, no contraction):
 //   fg = lut[c][x];  bg = (resized - mean[c]) / std[c];  out = fg * f32(1 - alpha) + bg * f32(alpha)
+#include "aa_resample.cuh"
 #include "bgd_common.cuh"
 
 #include <algorithm>
@@ -52,44 +53,6 @@ struct RaggedParams {
     float w_fg, w_bg;
     int64_t out_stride_t, out_stride_c;
 };
-
-// one accumulation step of ATen's tap loop: step j (1-based) of n = size - 1 steps
-__device__ __forceinline__ float aa_step(float acc, float v, float w, int j, int n_unfused)
-{
-    return j <= n_unfused ? __fadd_rn(acc, __fmul_rn(v, w)) : __fmaf_rn(v, w, acc);
-}
-
-// horizontal pass at one output column of one source row (uint8 pixels)
-__device__ __forceinline__ float aa_row(const uint8_t *row, const int32_t *ent)
-{
-    const int mn = ent[0], size = ent[1];
-    const float *w = reinterpret_cast<const float *>(ent + 2);
-    float acc = __fmul_rn((float)__ldg(row + mn), __ldg(w));
-    const int n_unfused = ((size - 1) >> 2) << 2;
-    for (int j = 1; j < size; ++j) acc = aa_step(acc, (float)__ldg(row + mn + j), __ldg(w + j), j, n_unfused);
-    return acc;
-}
-
-// value of the resized image at (Y, X) of channel plane `img_c` ([h][w] uint8)
-__device__ __forceinline__ float aa_sample(const uint8_t *img_c, const bgd_ragged_slot &s, const int32_t *tables, int Y, int X)
-{
-    const int32_t *xe = s.xtab >= 0 ? tables + s.xtab + (int64_t)X * (2 + s.kx) : nullptr;
-    if (s.ytab < 0) {
-        const uint8_t *row = img_c + (int64_t)Y * s.w;
-        return xe ? aa_row(row, xe) : (float)__ldg(row + X);
-    }
-    const int32_t *ye = tables + s.ytab + (int64_t)Y * (2 + s.ky);
-    const int mn = ye[0], size = ye[1];
-    const float *w = reinterpret_cast<const float *>(ye + 2);
-    const int n_unfused = ((size - 1) >> 2) << 2;
-    float acc = 0.f;
-    for (int r = 0; r < size; ++r) {
-        const uint8_t *row = img_c + (int64_t)(mn + r) * s.w;
-        const float hv = xe ? aa_row(row, xe) : (float)__ldg(row + X);
-        acc = r == 0 ? __fmul_rn(hv, __ldg(w)) : aa_step(acc, hv, __ldg(w + r), r, n_unfused);
-    }
-    return acc;
-}
 
 __device__ __forceinline__ bgd_ragged_slot load_slot(const RaggedParams &prm, int64_t b, int &top, int &left)
 {
@@ -125,7 +88,8 @@ __global__ void __launch_bounds__(kThreads) bgmix_ragged_kernel(const RaggedPara
         for (int c = 0; c < 3; ++c)
 #pragma unroll
             for (int i = 0; i < PX; ++i) {
-                const float raw = aa_sample(img + (int64_t)c * s.h * s.w, s, prm.tables, top + y, left + x + i);
+                const float raw = aa_sample(img + (int64_t)c * s.h * s.w, s.w, prm.tables, s.xtab, s.kx, s.ytab, s.ky, top + y,
+                                            left + x + i);
                 g[c][i] = __fmul_rn(__fdiv_rn(__fsub_rn(raw, prm.mean[c]), prm.std[c]), prm.w_bg);
             }
     }
@@ -200,74 +164,21 @@ __global__ void __launch_bounds__(kThreads, BGD_RAGGED_MINBLOCKS) bgmix_ragged_t
         const bgd_ragged_slot s = load_slot(prm, b, top, left);
         const uint8_t *img = prm.pool + s.offset;
         const int Y0 = top + ty0, Ylast = top + min(ty0 + kTile, H) - 1;
-        int rmin = Y0, rend = Ylast + 1;
-        if (s.ytab >= 0) {
-            rmin = prm.tables[s.ytab + (int64_t)Y0 * (2 + s.ky)];
-            const int32_t *last = prm.tables + s.ytab + (int64_t)Ylast * (2 + s.ky);
-            rend = last[0] + last[1];
-        }
+        int rmin, rend;
+        aa_tile_rows(prm.tables, s.ytab, s.ky, Y0, Ylast, rmin, rend);
         const int nrows = rend - rmin;
         if (nrows <= kMaxSrcRows) {
             // horizontal pass: thread -> output column x of the tile, source rows r = warp, warp + 8, ...
             const int x = threadIdx.x & 31, X = left + tx0 + x, r_first = threadIdx.x >> 5;
             if (tx0 + x < W) {
                 const int32_t *xe = s.xtab >= 0 ? prm.tables + s.xtab + (int64_t)X * (2 + s.kx) : nullptr;
-                const int xmin = xe ? xe[0] : X, xsize = xe ? xe[1] : 1;
-                const int step = (kThreads / 32) * s.w;                        // bytes between this thread's source rows
-                if (xsize <= 3) {
-                    // up to 3 taps (any up-scaling): v0 w0, then fused multiply-adds -- ATen's order for fewer than 5 taps.
-                    // An absent tap has weight 0 and re-reads the pixel before it, which leaves the sum unchanged.
-                    const float *w = reinterpret_cast<const float *>(xe + 2);
-                    const float w0 = xe ? __ldg(w) : 1.f, w1 = xsize > 1 ? __ldg(w + 1) : 0.f, w2 = xsize > 2 ? __ldg(w + 2) : 0.f;
-                    const int o1 = xsize > 1 ? 1 : 0, o2 = xsize > 2 ? 2 : o1;
-#pragma unroll
-                    for (int c = 0; c < 3; ++c) {
-                        const uint8_t *q = img + ((int64_t)c * s.h + rmin + r_first) * s.w + xmin;
-                        float *dst = &s_h[c][r_first][x];
-#pragma unroll 4
-                        for (int r = r_first; r < nrows; r += kThreads / 32) {
-                            const float v0 = (float)__ldg(q), v1 = (float)__ldg(q + o1), v2 = (float)__ldg(q + o2);
-                            *dst = __fmaf_rn(v2, w2, __fmaf_rn(v1, w1, __fmul_rn(v0, w0)));
-                            q += step;
-                            dst += (kThreads / 32) * kTile;
-                        }
-                    }
-                } else {
-#pragma unroll
-                    for (int c = 0; c < 3; ++c) {
-                        const uint8_t *q = img + ((int64_t)c * s.h + rmin + r_first) * s.w;
-                        for (int r = r_first; r < nrows; r += kThreads / 32, q += step) s_h[c][r][x] = aa_row(q, xe);
-                    }
-                }
+                aa_tile_hpass<kThreads / 32>(s_h, img, (int64_t)s.h * s.w, s.w, xe, X, x, rmin, r_first, nrows);
             }
             __syncthreads();
             if (inside) {
                 const int Y = top + ty0 + ty;
-                if (s.ytab < 0) {
-#pragma unroll
-                    for (int c = 0; c < 3; ++c) {
-                        const float4 v = *reinterpret_cast<const float4 *>(&s_h[c][Y - rmin][tx]);
-                        g[c][0] = v.x; g[c][1] = v.y; g[c][2] = v.z; g[c][3] = v.w;
-                    }
-                } else {
-                    const int32_t *ye = prm.tables + s.ytab + (int64_t)Y * (2 + s.ky);
-                    const int r0 = ye[0] - rmin, size = ye[1];
-                    const float *w = reinterpret_cast<const float *>(ye + 2);
-                    const int n_unfused = ((size - 1) >> 2) << 2;
-#pragma unroll
-                    for (int c = 0; c < 3; ++c) {
-                        float4 v = *reinterpret_cast<const float4 *>(&s_h[c][r0][tx]);
-                        const float wy0 = __ldg(w);
-                        float a0 = __fmul_rn(v.x, wy0), a1 = __fmul_rn(v.y, wy0), a2 = __fmul_rn(v.z, wy0), a3 = __fmul_rn(v.w, wy0);
-                        for (int r = 1; r < size; ++r) {
-                            v = *reinterpret_cast<const float4 *>(&s_h[c][r0 + r][tx]);
-                            const float wr = __ldg(w + r);
-                            a0 = aa_step(a0, v.x, wr, r, n_unfused); a1 = aa_step(a1, v.y, wr, r, n_unfused);
-                            a2 = aa_step(a2, v.z, wr, r, n_unfused); a3 = aa_step(a3, v.w, wr, r, n_unfused);
-                        }
-                        g[c][0] = a0; g[c][1] = a1; g[c][2] = a2; g[c][3] = a3;
-                    }
-                }
+                const int32_t *ye = s.ytab >= 0 ? prm.tables + s.ytab + (int64_t)Y * (2 + s.ky) : nullptr;
+                aa_tile_vpass4(s_h, ye, Y, rmin, tx, g);
             }
         } else {
             __syncthreads();
@@ -276,7 +187,8 @@ __global__ void __launch_bounds__(kThreads, BGD_RAGGED_MINBLOCKS) bgmix_ragged_t
                 for (int c = 0; c < 3; ++c)
 #pragma unroll
                     for (int i = 0; i < 4; ++i)
-                        g[c][i] = aa_sample(img + (int64_t)c * s.h * s.w, s, prm.tables, top + ty0 + ty, left + tx0 + tx + i);
+                        g[c][i] = aa_sample(img + (int64_t)c * s.h * s.w, s.w, prm.tables, s.xtab, s.kx, s.ytab, s.ky,
+                                            top + ty0 + ty, left + tx0 + tx + i);
             }
         }
         if (inside) {
@@ -332,7 +244,8 @@ __global__ void __launch_bounds__(kThreads) bgmix_ragged_normfg_kernel(const Rag
         int top, left;
         const bgd_ragged_slot s = load_slot(prm, b, top, left);
         const int y = (int)(p / prm.W), x = (int)(p - (int64_t)y * prm.W);
-        const float raw = aa_sample(prm.pool + s.offset + c * (int64_t)s.h * s.w, s, prm.tables, top + y, left + x);
+        const float raw = aa_sample(prm.pool + s.offset + c * (int64_t)s.h * s.w, s.w, prm.tables, s.xtab, s.kx, s.ytab, s.ky,
+                                    top + y, left + x);
         g = __fmul_rn(__fdiv_rn(__fsub_rn(raw, prm.mean[c]), prm.std[c]), prm.w_bg);
     }
     const float *src = prm.fgn + (b * prm.T * 3 + c) * HW + p;
@@ -351,7 +264,7 @@ __global__ void __launch_bounds__(kThreads) aa_resize_kernel(const uint8_t *__re
     const int64_t p = (int64_t)blockIdx.x * kThreads + threadIdx.x;
     if (p >= n) return;
     const int c = blockIdx.y, Y = (int)(p / s.Wb), X = (int)(p - (int64_t)Y * s.Wb);
-    out[c * n + p] = aa_sample(img + (int64_t)c * s.h * s.w, s, tables, Y, X);
+    out[c * n + p] = aa_sample(img + (int64_t)c * s.h * s.w, s.w, tables, s.xtab, s.kx, s.ytab, s.ky, Y, X);
 }
 
 }  // namespace

@@ -165,32 +165,108 @@ def bg_extraction_tmf(data_path: pathlib.Path, dest: pathlib.Path,
 SIM_CAM_CROP = 100
 
 
-def sim_cam_frames(data_path: pathlib.Path, interval: int, max_frames: int) -> torch.Tensor:
-    """The reference's loop (extract_background.py:81-92) up to the NaN marking: every ``interval``-th image
-    of the sorted folder except the last, at most ``max_frames``, each through ``RandomResizedCrop(size=100)``
-    on the host (torchvision itself: same torch-RNG draws, same antialiased resize).  float32 ``[T,100,100,3]``."""
+def sim_cam_files(data_path: pathlib.Path, interval: int, max_frames: int) -> List[pathlib.Path]:
+    """The frames the reference's loop reads (extract_background.py:82-88): every ``interval``-th file of the sorted
+    folder except the last, at most ``max_frames`` of them."""
+    return sorted(pathlib.Path(data_path).glob('*'))[:-1:interval][:max_frames]
+
+
+def read_sim_cam_frames(data_path: pathlib.Path, interval: int, max_frames: int) -> List[torch.Tensor]:
+    """The decoded frames of a folder, uint8 ``[3, H, W]`` each: ``torchvision.io.read_image`` as the reference decodes
+    them (:89).  An empty folder, an unreadable file and an image without exactly 3 channels raise ``ValueError`` (the
+    reference fails on them too: nanmedian of nothing, read_image's error, cvtColor(BGR2RGB) on :99)."""
     from torchvision.io import read_image
-    from torchvision.transforms import Compose, RandomResizedCrop
-    cam_motion_pipeline = Compose([RandomResizedCrop(size=SIM_CAM_CROP)])
-    image_files = sorted(pathlib.Path(data_path).glob('*'))
-    out = []
-    for i, frame_f in enumerate(image_files[:-1:interval]):
-        if i == max_frames:
-            break
-        frame = read_image(str(frame_f)).float()
-        out.append(cam_motion_pipeline(frame).permute(1, 2, 0).contiguous())
-    if not out:
-        raise ValueError(f"no frames under {data_path}")       # reference: nanmedian of [] raises
-    return torch.stack(out)
+    frames = []
+    for f in sim_cam_files(data_path, interval, max_frames):
+        try:
+            img = read_image(str(f))
+        except RuntimeError as e:
+            raise ValueError(f"{f}: cannot decode ({e})") from e
+        if img.dim() != 3 or img.shape[0] != 3:
+            raise ValueError(f"{f}: {tuple(img.shape)} is not a 3-channel image")
+        frames.append(img)
+    if not frames:
+        raise ValueError(f"no frames under {data_path}")
+    return frames
+
+
+def crop_draws(sizes) -> List[tuple]:
+    """``(top, left, h, w)`` per frame of frame sizes ``(H, W)`` in order: the draws ``RandomResizedCrop(100)`` makes
+    for those frames (:81,90) -- ``get_params`` with torchvision's default scale and ratio on the global torch RNG,
+    which depends on the frame size only.  Call it on one thread, in the reference's frame order."""
+    from torchvision.transforms import RandomResizedCrop
+    rrc = RandomResizedCrop(SIM_CAM_CROP)
+    return [tuple(int(v) for v in rrc.get_params(torch.empty(1, 1, 1).expand(3, int(H), int(W)), rrc.scale, rrc.ratio))
+            for H, W in sizes]
+
+
+def crop_descriptors(frames, draws, tables) -> torch.Tensor:
+    """int64 ``[n, 11]`` descriptors of ``torch.ops.bgdebias.resized_crop_aa`` for ``frames`` = ``(byte offset, H, W)``
+    and ``draws`` = ``(top, left, h, w)``; ``tables`` (:class:`pool.AATables`) gains the weight tables they need."""
+    rows = []
+    for (off, H, W), (i, j, h, w) in zip(frames, draws):
+        xtab, kx = tables.lookup(w, SIM_CAM_CROP)
+        ytab, ky = tables.lookup(h, SIM_CAM_CROP)
+        rows.append((off, H, W, i, j, h, w, xtab, ytab, kx, ky))
+    return torch.tensor(rows, dtype=torch.int64).reshape(-1, 11)
+
+
+def _frame_layout(start: int, frames) -> list:
+    """``(byte offset, H, W)`` of ``[3, H, W]`` frames packed back to back from ``start``."""
+    out, off = [], start
+    for f in frames:
+        H, W = int(f.shape[1]), int(f.shape[2])
+        out.append((off, H, W))
+        off += 3 * H * W
+    return out
+
+
+class SimCamReduce:
+    """The sim_cam reduction of a staged slab (``staging.FrameStager(reduce=...)``): one ``resized_crop_aa`` launch over
+    every frame of the slab (frames of any sizes), then one ``nan_temporal_reduce_varlen`` launch (zeros are missing,
+    :91) -> uint8 ``[V, 100, 100, 3]``.  ``add_video``'s ``meta`` is the folder's ``[(byte offset from the folder's
+    first byte, H, W)]`` and its draws."""
+    mixed_sizes = True
+
+    def __init__(self, device, avg_method: int):
+        from .pool import AATables
+        self.tables = AATables(device)
+        self.avg_method = int(avg_method)
+
+    def result_shape(self, frame_shape: tuple) -> tuple:
+        return (SIM_CAM_CROP, SIM_CAM_CROP, 3)
+
+    def __call__(self, data: torch.Tensor, slab) -> torch.Tensor:
+        frames, draws = [], []
+        for start, (layout, d) in zip(slab.starts, slab.metas):
+            frames += [(start + off, H, W) for off, H, W in layout]
+            draws += d
+        desc = crop_descriptors(frames, draws, self.tables)
+        crops = torch.ops.bgdebias.resized_crop_aa(data, desc, self.tables.tensor_for(torch.cuda.current_stream(data.device)),
+                                                   SIM_CAM_CROP, SIM_CAM_CROP)
+        return torch.ops.bgdebias.nan_temporal_reduce_varlen(crops, torch.tensor(slab.offsets, dtype=torch.int64),
+                                                             self.avg_method, True)
 
 
 def sim_cam_background(data_path: pathlib.Path, interval: int, max_frames: int, avg_method: int, device=0) -> np.ndarray:
-    """uint8 ``[100,100,3]``: the ``ave_frame`` of extract_background.py:94-98.  Zeros count as missing
-    (:91); the NaN-masked median (``avg_method`` 0) or mean (1) over the frames runs on the GPU."""
+    """uint8 ``[100,100,3]``: the ``ave_frame`` of extract_background.py:94-98.  The frames are decoded on the host;
+    the crops (one launch for the folder, draws from the torch RNG as the reference makes them) and the NaN-masked
+    median (``avg_method`` 0) or mean (1) over them, zeros counting as missing (:91), run on the GPU."""
     from . import ops as _ops  # noqa: F401  (registers torch.ops.bgdebias.*)
+    from .pool import AATables
     dev = torch.device(device if not isinstance(device, int) else f"cuda:{device}")
-    frames = sim_cam_frames(data_path, interval, max_frames).to(dev)
-    return torch.ops.bgdebias.nan_temporal_reduce(frames, int(avg_method), True).cpu().numpy()
+    frames = read_sim_cam_frames(data_path, interval, max_frames)
+    draws = crop_draws([f.shape[1:] for f in frames])
+    layout = _frame_layout(0, frames)
+    host = torch.empty(sum(3 * H * W for _, H, W in layout), dtype=torch.uint8, pin_memory=True)
+    for f, (off, H, W) in zip(frames, layout):
+        host[off:off + 3 * H * W] = f.reshape(-1)
+    tables = AATables(dev)
+    desc = crop_descriptors(layout, draws, tables)
+    with torch.cuda.device(dev):
+        crops = torch.ops.bgdebias.resized_crop_aa(host.to(dev, non_blocking=True), desc, tables.tensor, SIM_CAM_CROP,
+                                                   SIM_CAM_CROP)
+        return torch.ops.bgdebias.nan_temporal_reduce(crops, int(avg_method), True).cpu().numpy()
 
 
 def sim_cam_motion_bg_extract(data_path, dest, from_video, interval, max_frames, avg_method, device=0):
@@ -201,25 +277,38 @@ def sim_cam_motion_bg_extract(data_path, dest, from_video, interval, max_frames,
     cv2.imwrite(str(dest), cv2.cvtColor(ave_frame, cv2.COLOR_BGR2RGB))
 
 
+def in_submission_order(pool, fn, items, window: int):
+    """``fn(item)`` for every item on the executor ``pool``, at most ``window`` in flight, results yielded in the order
+    of ``items`` -- whatever order the threads finish in."""
+    pending, it = [], iter(items)
+    while True:
+        while len(pending) < window:
+            nxt = next(it, None)
+            if nxt is None:
+                break
+            pending.append(pool.submit(fn, nxt))
+        if not pending:
+            return
+        yield pending.pop(0).result()
+
+
 def bg_extract_multiple(paths: List[pathlib.Path], output_dir: pathlib.Path, from_video: bool,
                         interval: int, max_frames: int, process_id: int, method, avg_method: int,
                         device=None, decode_threads: int = 4, slab_mb: int = 512):
-    """Same role and leading arguments as the reference (extract_background.py:102-109).  For the
-    ``tmf`` method the videos of this shard are decoded by a thread pool into a pinned slab and
-    reduced many-per-launch; any other ``method`` callable is invoked video by video like the reference."""
+    """Same role and leading arguments as the reference (extract_background.py:102-109).  For the ``tmf`` and
+    ``sim_cam`` methods the videos / frame folders of this shard are decoded by a thread pool into a pinned slab and
+    reduced many-per-launch; any other ``method`` callable is invoked video by video like the reference.  Returns
+    the failures, ``[(path, reason)]``; the other videos still finish."""
     output_dir = pathlib.Path(output_dir)
-    if method is not bg_extraction_tmf:
-        extra = {}
-        if method is sim_cam_motion_bg_extract:
-            extra['device'] = _shard.device_for(process_id, torch.cuda.device_count()) if device is None else device
+    if method is not bg_extraction_tmf and method is not sim_cam_motion_bg_extract:
         for data_path in paths:
-            method(data_path, (output_dir / data_path.name).with_suffix('.jpg'), from_video, interval, max_frames,
-                   avg_method, **extra)
+            method(data_path, (output_dir / data_path.name).with_suffix('.jpg'), from_video, interval, max_frames, avg_method)
         return []
     if device is None:
         device = _shard.device_for(process_id, torch.cuda.device_count())
     dev = torch.device(f"cuda:{device}" if isinstance(device, int) else device)
     torch.cuda.set_device(dev)
+    sim_cam = method is sim_cam_motion_bg_extract
 
     os.environ.setdefault("OPENCV_FFMPEG_THREADS", "1")     # many videos in flight: one FFmpeg thread per capture, no oversubscription
     n_dec = max(1, decode_threads)
@@ -230,33 +319,35 @@ def bg_extract_multiple(paths: List[pathlib.Path], output_dir: pathlib.Path, fro
         writes = []
 
         def write(tag, bg):                                  # JPEG encoding off the staging path
-            writes.append(writers.submit(cv2.imwrite, str(tag), bg))
+            if sim_cam:                                      # the reference's channel swap before imwrite (:99)
+                writes.append(writers.submit(lambda t, b: cv2.imwrite(str(t), cv2.cvtColor(b, cv2.COLOR_BGR2RGB)), tag, bg))
+            else:
+                writes.append(writers.submit(cv2.imwrite, str(tag), bg))
 
-        stager = FrameStager(write, dev, slab_mb)
+        stager = FrameStager(write, dev, slab_mb, reduce=SimCamReduce(dev, avg_method) if sim_cam else None)
 
         def decode(p):
-            # decode into this thread's scratch frames, then pack them into the pinned slab from this thread
+            # tmf: decode into this thread's scratch frames, then pack them into the pinned slab from this thread
             try:
+                if sim_cam:
+                    return p, read_sim_cam_frames(p, interval, max_frames)
                 frames = read_frames_packed(p, from_video, interval, max_frames)
                 if not len(frames):
-                    return str(p), "no frames decoded"
+                    return p, "no frames decoded"
                 stager.add_video(frames, (output_dir / p.name).with_suffix('.jpg'))
-                return None
+                return p, None
             except Exception as e:  # keep going, report at the end
-                return str(p), repr(e)
+                return p, repr(e)
 
-        failures, window, it = [], [], iter(paths)
-        while True:
-            while len(window) < 4 * n_dec:
-                nxt = next(it, None)
-                if nxt is None:
-                    break
-                window.append(pool.submit(decode, nxt))
-            if not window:
-                break
-            r = window.pop(0).result()
-            if r is not None:
-                failures.append(r)
+        failures = []
+        for p, r in in_submission_order(pool, decode, paths, 4 * n_dec):
+            if isinstance(r, list):
+                # sim_cam: the crop draws of a folder are made here, on one thread in the order of `paths` -- the order
+                # the reference's worker draws them in, whatever order the decoder threads finish in
+                stager.add_video(r, (output_dir / p.name).with_suffix('.jpg'),
+                                 (_frame_layout(0, r), crop_draws([f.shape[1:] for f in r])))
+            elif r is not None:
+                failures.append((str(p), r))
             while writes and writes[0].done():
                 writes.pop(0).result()                       # surface write errors early, keep the list short
         stager.flush()

@@ -22,6 +22,9 @@ built library (``ImportError`` otherwise).  Ops are stream-ordered and never syn
     bgdebias::bgmix_resize_blend(Tensor src, Tensor geom, int T, int H, int W, <bgmix_blend arguments>) -> Tensor
         the pipeline's Resize((W, H), keep_ratio=False) (config ..._bgmix_plus_randAug.py:136; cv2 INTER_LINEAR, bit-exact)
         on packed uint8 crops, alone or fused with the blend.
+    bgdebias::resized_crop_aa(Tensor src, Tensor desc, Tensor tables, int out_h, int out_w) -> Tensor
+        RandomResizedCrop(100)(read_image(f).float()).permute(1, 2, 0) of many frames of any sizes, for host-made draws
+        (cil_tools/extract_background.py:81,89-90; torchvision's antialiased bilinear, bit-exact).
 """
 from __future__ import annotations
 
@@ -29,6 +32,7 @@ import ctypes
 import math
 from typing import Sequence, Tuple
 
+import numpy as np
 import torch
 
 from . import _cabi
@@ -151,6 +155,44 @@ def nan_temporal_reduce_f32(frames: torch.Tensor, avg_method: int, zero_is_missi
 @nan_temporal_reduce_f32.register_fake
 def _(frames, avg_method, zero_is_missing):
     return frames.new_empty(frames.shape[1:])
+
+
+# --------------------------------------------------------------------------- #
+# RandomResizedCrop of many frames (sim_cam extraction, extract_background.py:81,89-90)
+# --------------------------------------------------------------------------- #
+CROP_DESC_FIELDS = ("offset", "H", "W", "top", "left", "h", "w", "xtab", "ytab", "kx", "ky")
+_CROP_DESC_DTYPE = [(n, "<i8" if n == "offset" else "<i4") for n in CROP_DESC_FIELDS]     # bgd_crop_desc, 48 bytes
+
+
+@torch.library.custom_op("bgdebias::resized_crop_aa", mutates_args=(), device_types="cuda")
+def resized_crop_aa(src: torch.Tensor, desc: torch.Tensor, tables: torch.Tensor, out_h: int, out_w: int) -> torch.Tensor:
+    """Frames planar uint8 ``[3, H, W]`` at byte offsets of the flat buffer ``src`` -> float32 ``[n, out_h, out_w, 3]``:
+    frame k is ``resized_crop(frame, top, left, h, w, (out_h, out_w), antialias=True).permute(1, 2, 0)``, bit-exact.
+    ``desc``: int64 ``[n, 11]`` (host or device) with the columns of :data:`CROP_DESC_FIELDS`; ``tables``: int32 weight
+    tables on the device (``pool.AATables``; xtab / ytab = -1 where the crop size equals the output size)."""
+    _require(src.dtype == torch.uint8 and src.dim() == 1, "resized_crop_aa: src must be a flat uint8 buffer")
+    _require(desc.dim() == 2 and desc.shape[1] == len(CROP_DESC_FIELDS) and desc.dtype in (torch.int64, torch.int32),
+             f"resized_crop_aa: desc must be int64 [n, {len(CROP_DESC_FIELDS)}]")
+    _require(tables.dtype == torch.int32 and tables.dim() == 1, "resized_crop_aa: tables must be a flat int32 tensor")
+    _require(tables.device == src.device, f"resized_crop_aa: tables must be on {src.device}")
+    _require(out_h > 0 and out_w > 0, "resized_crop_aa: the output size must be positive")
+    d = desc.detach().to("cpu", torch.int64).contiguous().numpy()
+    _require(bool((d[:, 1:] >= -(1 << 31)).all() and (d[:, 1:] < (1 << 31)).all()), "resized_crop_aa: desc values out of int32 range")
+    h_desc = np.empty(d.shape[0], dtype=_CROP_DESC_DTYPE)
+    for k, name in enumerate(CROP_DESC_FIELDS):
+        h_desc[name] = d[:, k]
+    src, tables = src.contiguous(), tables.contiguous()
+    out = torch.empty((d.shape[0], out_h, out_w, 3), dtype=torch.float32, device=src.device)
+    with torch.cuda.device(src.device):
+        _cabi.check(_cabi.lib().bgd_resized_crop_aa_u8_f32(src.data_ptr(), src.numel(), h_desc.ctypes.data, d.shape[0],
+                                                           tables.data_ptr(), tables.numel(), out_h, out_w, out.data_ptr(),
+                                                           _stream_ptr(src.device)))
+    return out
+
+
+@resized_crop_aa.register_fake
+def _(src, desc, tables, out_h, out_w):
+    return src.new_empty((desc.shape[0], out_h, out_w, 3), dtype=torch.float32)
 
 
 # --------------------------------------------------------------------------- #

@@ -85,6 +85,15 @@ class AATables:
             self._dev = torch.from_numpy(host).to(self.device)
         return self._dev
 
+    def tensor_for(self, stream: torch.cuda.Stream) -> torch.Tensor:
+        """:attr:`tensor` for a launch on ``stream``.  A new key replaces the device tensor, and the caching allocator
+        would hand the old one's memory to the next allocation of the stream it was made on, while a launch on
+        ``stream`` may still read it; marking the use on ``stream`` keeps that memory out of reuse until the work
+        enqueued there so far has finished."""
+        t = self.tensor
+        t.record_stream(stream)
+        return t
+
 
 class RaggedPool:
     """Backgrounds of ANY sizes, uint8 at native size, in one device byte buffer plus a slot table -- the form

@@ -10,6 +10,9 @@ decoder is already filling the other slab.
 ``add_video`` may be called from many decoder threads at once: a thread reserves its rows under a lock and
 copies its frames into the slab outside it (numpy releases the GIL for the copy), so packing scales with the
 decoder threads instead of serialising on the caller.
+
+What a slab is reduced with is a parameter (``reduce=``): :class:`MedianReduce` (the default, tmf) or
+``extract_background.SimCamReduce`` (RandomResizedCrop + NaN-masked median / mean, whose frames may differ in size).
 """
 from __future__ import annotations
 
@@ -36,29 +39,47 @@ class _Slab:
         self.N = None
         self.offsets: List[int] = [0]
         self.tags: list = []
-        self.shapes: list = []
+        self.shapes: list = []             # result shape per video
+        self.starts: List[int] = []        # first byte of each video in the slab
+        self.metas: list = []              # per-video data for the reduction (add_video's `meta`)
         self.out_host: Optional[torch.Tensor] = None
         self.pending = False
         self.filling = 0                   # reservations whose frames are still being copied in
 
 
-class FrameStager:
-    """``add_video(frames, tag)`` queues one decoded video (list/array of equal-shaped uint8 frames);
-    ``on_result(tag, background_ndarray)`` is called for every video once its median is back on the
-    host.  Call :meth:`flush` at the end."""
+class MedianReduce:
+    """The tmf reduction: per-pixel temporal median of every video of a slab, one ``temporal_median_varlen`` launch.
+    All frames of a slab have one size."""
+    mixed_sizes = False
 
-    def __init__(self, on_result: Callable, device="cuda", slab_mb: int = 512):
+    def result_shape(self, frame_shape: tuple) -> tuple:
+        return frame_shape
+
+    def __call__(self, data: torch.Tensor, slab: "_Slab") -> torch.Tensor:
+        """``data``: the slab's bytes on the device; returns uint8 ``[V, N]`` on the current stream."""
+        return torch.ops.bgdebias.temporal_median_varlen(data.view(slab.offsets[-1], slab.N),
+                                                         torch.tensor(slab.offsets, dtype=torch.int64))
+
+
+class FrameStager:
+    """``add_video(frames, tag)`` queues one decoded video (list/array of uint8 frames);
+    ``on_result(tag, background_ndarray)`` is called for every video once its reduction (``reduce``, by default the
+    temporal median) is back on the host.  Call :meth:`flush` at the end."""
+
+    def __init__(self, on_result: Callable, device="cuda", slab_mb: int = 512, reduce=None):
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise RuntimeError("FrameStager needs a CUDA device: there is no CPU path")
         self.on_result = on_result
+        self.reduce = reduce if reduce is not None else MedianReduce()
         self.slab_bytes = int(slab_mb) << 20
         self.slabs: List[Optional[_Slab]] = [None, None]
         self.cur = 0
         self._cv = threading.Condition()
 
-    def add_video(self, frames: Sequence[np.ndarray], tag) -> None:
-        """Thread-safe.  ``frames``: a list of equal-shaped uint8 frames or one ``[T, ...]`` uint8 array."""
+    def add_video(self, frames: Sequence[np.ndarray], tag, meta=None) -> None:
+        """Thread-safe.  ``frames``: a list of uint8 frames (arrays or CPU tensors; of one shape unless the reduction
+        takes mixed sizes) or one ``[T, ...]`` uint8 array, packed back to back.  ``meta`` goes to the reduction."""
         T = len(frames)
         if T == 0:
             # reference: np.median([]) -> nan -> cv2.imwrite raises (extract_background.py:73-74)
@@ -68,28 +89,35 @@ class FrameStager:
         if stacked:
             if frames.dtype != np.uint8:
                 raise ValueError(f"{tag}: frames must be uint8")
+            sizes = None
         else:
+            frames = [np.asarray(f) for f in frames]
             for t, f in enumerate(frames):
-                if tuple(f.shape) != shape or f.dtype != np.uint8:
+                if f.dtype != np.uint8 or (tuple(f.shape) != shape and not self.reduce.mixed_sizes):
                     raise ValueError(f"{tag}: frame {t} differs in shape or dtype")
+            sizes = [f.size for f in frames]
         N = int(np.prod(shape))
-        need = T * N
+        need = T * N if sizes is None else sum(sizes)
         with self._cv:
-            slab = self._room_for(need, N)
+            slab = self._room_for(need, None if self.reduce.mixed_sizes else N)
             off = slab.used
-            slab.N = N
+            slab.N = None if self.reduce.mixed_sizes else N
             slab.used += need
             slab.offsets.append(slab.offsets[-1] + T)
             slab.tags.append(tag)
-            slab.shapes.append(shape)
+            slab.shapes.append(self.reduce.result_shape(shape))
+            slab.starts.append(off)
+            slab.metas.append(meta)
             slab.filling += 1
         try:
-            view = slab.host[off:off + need].view(T, N).numpy()
             if stacked:
-                view[:] = frames.reshape(T, N)
+                slab.host[off:off + need].view(T, N).numpy()[:] = frames.reshape(T, N)
             else:
-                for t, f in enumerate(frames):
-                    view[t] = f.reshape(-1)
+                buf = slab.host[off:off + need].numpy()
+                pos = 0
+                for f, n in zip(frames, sizes):
+                    buf[pos:pos + n] = f.reshape(-1)
+                    pos += n
         finally:
             with self._cv:
                 slab.filling -= 1
@@ -121,14 +149,11 @@ class FrameStager:
         slab = self.slabs[i]
         if slab is None or not slab.tags:
             return
-        V, N = len(slab.tags), slab.N
-        rows = slab.offsets[-1]
         # decoder threads land here too: the current device is per thread
         with torch.cuda.device(self.device), torch.cuda.stream(slab.stream):
             slab.dev[:slab.used].copy_(slab.host[:slab.used], non_blocking=True)
-            out = torch.ops.bgdebias.temporal_median_varlen(slab.dev[:slab.used].view(rows, N),
-                                                            torch.tensor(slab.offsets, dtype=torch.int64))
-            slab.out_host = torch.empty((V, N), dtype=torch.uint8, pin_memory=True)
+            out = self.reduce(slab.dev[:slab.used], slab)
+            slab.out_host = torch.empty(out.shape, dtype=torch.uint8, pin_memory=True)
             slab.out_host.copy_(out, non_blocking=True)
             slab.done.record(slab.stream)
         slab.pending = True

@@ -235,6 +235,36 @@ int bgd_bgmix_blend_ragged_normfg_f32(const float *d_fg_norm, int64_t B, int64_t
                                       const int32_t *d_left, const uint8_t *d_apply, const float *h_bg_mean,
                                       const float *h_bg_std, double alpha, int layout, float *d_out, void *stream);
 
+/* ---- RandomResizedCrop of a batch of frames (simulated-camera-motion extraction) --------------------
+ * Replaces, for every frame of many frame folders in one launch,
+ *   cil_tools/extract_background.py:81     cam_motion_pipeline = Compose([RandomResizedCrop(size=100)])
+ *   cil_tools/extract_background.py:89-90  frame = cam_motion_pipeline(read_image(f).float()).permute(1, 2, 0)
+ * The random draws (top, left, h, w) are made on the host, with the torch RNG, as RandomResizedCrop.get_params makes them;
+ * this call evaluates torchvision's resized_crop(frame, top, left, h, w, (out_h, out_w), bilinear, antialias=True) for
+ * each frame: the window [:, top:top+h, left:left+w] through ATen's antialiased bilinear resize (third-party,
+ * UpSampleKernel.cpp) with the arithmetic of bgd_aa_resize_u8_f32 -- per-axis weight tables from bgd_aa_resize_table
+ * (in = crop size, out = output size), horizontal pass then vertical, products and sums rounded as that kernel rounds them
+ * (csrc/raggedmix.cu states the order); an axis whose crop size equals the output size has no table (-1) and is skipped.
+ *
+ *   d_src       frames, planar uint8 [3][H][W] each (torchvision.io.read_image's layout), at any byte offsets
+ *   src_bytes   size of d_src; every frame must lie inside it
+ *   h_desc      HOST array of n descriptors (validated, then copied to the device on `stream`)
+ *   d_tables    int32 weight tables (device), table_words words; may be NULL when no descriptor has a table
+ *   d_out       float32 [n][out_h][out_w][3], channels last
+ * n < 2^31, and ceil(out_h / 32) * ceil(out_w / 32) <= 65535. */
+typedef struct bgd_crop_desc {
+    int64_t offset;          /* bytes from d_src to the frame's first byte */
+    int32_t H, W;            /* frame size */
+    int32_t top, left;       /* crop window: rows top .. top+h-1, columns left .. left+w-1, inside the frame */
+    int32_t h, w;
+    int32_t xtab, ytab;      /* word offsets in d_tables of the w -> out_w and h -> out_h tables; -1 = no table */
+    int32_t kx, ky;          /* taps per entry of those tables (what bgd_aa_resize_table reports for the sizes) */
+} bgd_crop_desc;
+
+int bgd_resized_crop_aa_u8_f32(const uint8_t *d_src, int64_t src_bytes, const bgd_crop_desc *h_desc, int64_t n,
+                               const int32_t *d_tables, int64_t table_words, int64_t out_h, int64_t out_w,
+                               float *d_out, void *stream);
+
 /* ---- foreground pipeline tail: Resize -> Normalize -> FormatShape (-> blend) -----------------
  * Replaces the tail of the reference's training pipeline
  *   dict(type='Resize', scale=(224, 224), keep_ratio=False), Normalize, FormatShape('NCHW')
