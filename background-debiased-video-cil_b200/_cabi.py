@@ -17,6 +17,9 @@ BGD_OK, BGD_ERR_INVALID, BGD_ERR_CUDA, BGD_ERR_UNSUPPORTED, BGD_ERR_NO_DEVICE = 
 LAYOUT_NTCHW, LAYOUT_NCTHW = 0, 1
 MEDIAN_AUTO, MEDIAN_SWAR, MEDIAN_BITSLICED, MEDIAN_COLPLANE, MEDIAN_LDSM = 0, 1, 2, 3, 4
 LAYOUTS = {"NTCHW": LAYOUT_NTCHW, "NCTHW": LAYOUT_NCTHW}
+LAYOUT_NTHWC = 2
+OUT_LAYOUTS = {**LAYOUTS, "NTHWC": LAYOUT_NTHWC}        # layouts of the *_out blend entry points
+OUT_F32, OUT_BF16, OUT_F16 = 0, 1, 2
 
 _c = ctypes
 _f32p, _i64p = _c.POINTER(_c.c_float), _c.POINTER(_c.c_int64)
@@ -61,6 +64,9 @@ SIGNATURES = {
     "bgd_actor_cut_mix_u8": (_c.c_int, [_vp, _vp, _vp, _c.c_int64, _vp, _vp, _vp]),
     "bgd_bgmix_blend_f32": (_c.c_int, _blend_common + [_vp]),
     "bgd_bgmix_blend_u8pool_f32": (_c.c_int, _blend_common + [_vp]),
+    "bgd_bgmix_blend_out": (_c.c_int, [_vp, _c.c_int64, _c.c_int64, _c.c_int64, _c.c_int64,
+                                       _vp, _c.c_int, _c.c_int64, _c.c_int64, _c.c_int64,
+                                       _vp, _vp, _vp, _vp, _vp, _f32p, _f32p, _c.c_double, _c.c_int, _c.c_int, _vp, _vp]),
     "bgd_bgmix_blend_normfg_f32": (_c.c_int, [_vp, _c.c_int64, _c.c_int64, _c.c_int64, _c.c_int64,
                                               _vp, _c.c_int, _c.c_int64, _c.c_int64, _c.c_int64,
                                               _vp, _vp, _vp, _vp, _f32p, _f32p, _c.c_double, _c.c_int, _vp, _vp]),
@@ -68,6 +74,8 @@ SIGNATURES = {
     "bgd_aa_resize_table": (_c.c_int, [_c.c_int64, _c.c_int64, _c.POINTER(_c.c_int32), _vp, _c.c_int64]),
     "bgd_aa_resize_u8_f32": (_c.c_int, [_vp, _c.POINTER(RaggedSlot), _vp, _vp, _vp]),
     "bgd_bgmix_blend_ragged_f32": (_c.c_int, [_vp] + _ragged_common + [_vp, _f32p, _f32p, _c.c_double, _c.c_int, _vp, _vp]),
+    "bgd_bgmix_blend_ragged_out": (_c.c_int, [_vp] + _ragged_common + [_vp, _f32p, _f32p, _c.c_double, _c.c_int, _c.c_int,
+                                                                       _vp, _vp]),
     "bgd_bgmix_blend_ragged_normfg_f32": (_c.c_int, [_vp] + _ragged_common + [_f32p, _f32p, _c.c_double, _c.c_int, _vp, _vp]),
     "bgd_resized_crop_aa_u8_f32": (_c.c_int, [_vp, _c.c_int64, _vp, _c.c_int64, _vp, _c.c_int64, _c.c_int64, _c.c_int64,
                                               _vp, _vp]),
@@ -78,6 +86,10 @@ SIGNATURES = {
     "bgd_bgmix_resize_blend_f32": (_c.c_int, [_vp, _c.c_int64, _i64p, _c.c_int64, _c.c_int64, _c.c_int64, _c.c_int64,
                                               _vp, _c.c_int, _c.c_int64, _c.c_int64, _c.c_int64,
                                               _vp, _vp, _vp, _vp, _vp, _f32p, _f32p, _c.c_double, _c.c_int, _vp, _vp]),
+    "bgd_bgmix_resize_blend_out": (_c.c_int, [_vp, _c.c_int64, _i64p, _c.c_int64, _c.c_int64, _c.c_int64, _c.c_int64,
+                                              _vp, _c.c_int, _c.c_int64, _c.c_int64, _c.c_int64,
+                                              _vp, _vp, _vp, _vp, _vp, _f32p, _f32p, _c.c_double, _c.c_int, _c.c_int, _vp,
+                                              _vp]),
 }
 
 _lib = None

@@ -23,6 +23,8 @@ worker processes use ``collate_fn=dataset.host_collate`` (host tensors only, saf
 ``dataset.device_finish(batch)`` in the training process: the batch crosses PCIe as uint8, a quarter of the
 reference's fp32 bytes.  The pipeline may also stop before its last ``Resize((224, 224), keep_ratio=False)``: crops of
 mixed sizes are packed by ``host_collate`` and resized (cv2 INTER_LINEAR, bit for bit) inside the blend launch.
+``device_finish(batch, dtype=torch.bfloat16, memory_format=torch.channels_last)`` hands a bf16-autocast model its input
+directly: the blend's fp32 result rounded once to bf16, stored channels-last by the same launch.
 """
 from __future__ import annotations
 
@@ -370,7 +372,8 @@ class BackgroundMixDataset(_Base):
                             img_mean: Optional[Sequence[float]] = None, img_std: Optional[Sequence[float]] = None,
                             layout: str = "NTCHW", fg_geom: Optional[torch.Tensor] = None,
                             fg_frames: Optional[int] = None, bg_imgs: Optional[Sequence[torch.Tensor]] = None,
-                            bg_slot=None) -> torch.Tensor:
+                            bg_slot=None, dtype: torch.dtype = torch.float32,
+                            memory_format: torch.memory_format = torch.contiguous_format) -> torch.Tensor:
         """uint8 ``[B,T,H,W,3]`` (host or device) + per-sample draws -> fp32 ``[B,T,3,H,W]`` on the device.
         ``img_mean``/``img_std`` are the foreground's ``Normalize`` parameters (default: the bg ones,
         as in every shipped config).
@@ -382,7 +385,20 @@ class BackgroundMixDataset(_Base):
         Clips whose size is not ``bg_crop_size`` -- a pipeline that stops before the final
         ``Resize((224, 224), keep_ratio=False)`` (config :136) -- are resized with cv2's INTER_LINEAR arithmetic, inside
         the blend launch for a dense pool: either a stacked batch of one other size, or packed crops of mixed sizes
-        (``fg_u8`` flat, ``fg_geom`` int64 ``[B,5]``, ``fg_frames`` = T; see ``ops.pack_clips``)."""
+        (``fg_u8`` flat, ``fg_geom`` int64 ``[B,5]``, ``fg_frames`` = T; see ``ops.pack_clips``).
+
+        ``dtype`` float32, bfloat16 or float16: the fp32 blend rounded once to nearest even (equal to ``.to(dtype)`` of the
+        float32 batch).  ``memory_format=torch.channels_last``: the launch writes ``[B,T,H,W,3]`` and the method returns
+        its permuted view, logical ``[B,T,3,H,W]`` (whose ``flatten(0, 1)`` is ``channels_last``) for ``layout="NTCHW"``
+        or ``[B,3,T,H,W]`` in ``channels_last_3d`` strides for ``layout="NCTHW"``."""
+        if layout not in ("NTCHW", "NCTHW"):
+            raise ValueError(f"layout must be 'NTCHW' or 'NCTHW' (got {layout!r})")
+        if dtype not in (torch.float32, torch.bfloat16, torch.float16):
+            raise ValueError(f"dtype must be torch.float32, torch.bfloat16 or torch.float16 (got {dtype})")
+        if memory_format not in (torch.contiguous_format, torch.channels_last):
+            raise ValueError(f"memory_format must be torch.contiguous_format or torch.channels_last (got {memory_format})")
+        channels_last = memory_format == torch.channels_last
+        op_layout = "NTHWC" if channels_last else layout
         dev = self.device
         mean = self.bg_mean if img_mean is None else img_mean
         std = self.bg_std if img_std is None else img_std
@@ -408,14 +424,20 @@ class BackgroundMixDataset(_Base):
             fg_frames = T
         fg_u8 = fg_u8.to(dev, non_blocking=True)
         if fg_geom is not None and dense is not None:
-            return torch.ops.bgdebias.bgmix_resize_blend(fg_u8, fg_geom, int(fg_frames), th, tw, dense, rows, top, left, app, lut,
-                                                         mean_t, std_t, float(self.alpha), layout)
-        if fg_geom is not None:
-            fg_u8 = torch.ops.bgdebias.resize_bilinear(fg_u8, fg_geom, int(fg_frames), th, tw)
-        if dense is not None:
-            return torch.ops.bgdebias.bgmix_blend(fg_u8, dense, rows, top, left, app, lut, mean_t, std_t, float(self.alpha), layout)
-        return torch.ops.bgdebias.bgmix_blend_ragged(fg_u8, ragged.data, ragged.slots_tensor, ragged.tables.tensor, rows, top, left,
-                                                     app, lut, mean_t, std_t, float(self.alpha), layout)
+            out = torch.ops.bgdebias.bgmix_resize_blend(fg_u8, fg_geom, int(fg_frames), th, tw, dense, rows, top, left, app, lut,
+                                                        mean_t, std_t, float(self.alpha), op_layout, dtype)
+        else:
+            if fg_geom is not None:
+                fg_u8 = torch.ops.bgdebias.resize_bilinear(fg_u8, fg_geom, int(fg_frames), th, tw)
+            if dense is not None:
+                out = torch.ops.bgdebias.bgmix_blend(fg_u8, dense, rows, top, left, app, lut, mean_t, std_t, float(self.alpha),
+                                                     op_layout, dtype)
+            else:
+                out = torch.ops.bgdebias.bgmix_blend_ragged(fg_u8, ragged.data, ragged.slots_tensor, ragged.tables.tensor, rows,
+                                                            top, left, app, lut, mean_t, std_t, float(self.alpha), op_layout, dtype)
+        if channels_last:                                 # [B,T,H,W,3] -> logical [B,T,3,H,W] / [B,3,T,H,W]
+            return out.permute(0, 1, 4, 2, 3) if layout == "NTCHW" else out.permute(0, 4, 1, 2, 3)
+        return out
 
     def _aa_tables(self) -> AATables:
         if "aa_tables" not in self._resized_cache:
@@ -463,28 +485,31 @@ class BackgroundMixDataset(_Base):
             out['randAug'] = torch.tensor([bool(s['randAug']) for s in samples])
         return out
 
-    def device_finish(self, batch: dict, layout: str = "NTCHW") -> dict:
+    def device_finish(self, batch: dict, layout: str = "NTCHW", dtype: torch.dtype = torch.float32,
+                      memory_format: torch.memory_format = torch.contiguous_format) -> dict:
         """The GPU half of the ``device_mix=True`` path: turns a :meth:`host_collate` batch into the dict the
         reference's default_collate would hand the model (``imgs`` fp32 ``[B,T,3,H,W]`` on the device, ``label``,
-        ``randAug``, ``bg_idx``) with one fused launch."""
+        ``randAug``, ``bg_idx``) with one fused launch.  ``dtype`` / ``memory_format``: see :meth:`mix_batch_on_device`."""
         out = {k: v for k, v in batch.items()
                if k not in ('imgs', 'bg_top', 'bg_left', 'bg_apply', 'fg_geom', 'fg_frames', 'bg_imgs', 'bg_slot')}
         if self.back_ground_from_bg_dir or 'bg_imgs' in batch:
             out['imgs'] = self.mix_batch_on_device(batch['imgs'], batch['bg_idx'], batch['bg_top'], batch['bg_left'],
                                                    batch['bg_apply'], layout=layout, fg_geom=batch.get('fg_geom'),
                                                    fg_frames=batch.get('fg_frames'), bg_imgs=batch.get('bg_imgs'),
-                                                   bg_slot=batch.get('bg_slot'))
+                                                   bg_slot=batch.get('bg_slot'), dtype=dtype, memory_format=memory_format)
         else:                                             # random-frame mode and no sample of the batch was mixed
             out['imgs'] = self.mix_batch_on_device(batch['imgs'], batch['bg_idx'], batch['bg_top'], batch['bg_left'],
                                                    batch['bg_apply'], layout=layout, fg_geom=batch.get('fg_geom'),
                                                    fg_frames=batch.get('fg_frames'),
                                                    bg_imgs=[torch.zeros((3, *self.bg_crop_size), dtype=torch.uint8)],
-                                                   bg_slot=torch.zeros(len(batch['bg_idx']), dtype=torch.int32))
+                                                   bg_slot=torch.zeros(len(batch['bg_idx']), dtype=torch.int32),
+                                                   dtype=dtype, memory_format=memory_format)
         return out
 
-    def gpu_collate(self, samples: List[dict]) -> dict:
+    def gpu_collate(self, samples: List[dict], dtype: torch.dtype = torch.float32,
+                    memory_format: torch.memory_format = torch.contiguous_format) -> dict:
         """:meth:`host_collate` + :meth:`device_finish` in one call, for ``num_workers=0`` loaders."""
-        return self.device_finish(self.host_collate(samples))
+        return self.device_finish(self.host_collate(samples), dtype=dtype, memory_format=memory_format)
 
 
 def bg_extraction_tmf(data_path, dest, from_video=False, device='cuda'):

@@ -430,6 +430,12 @@ static int median_host_pipeline(const uint8_t *const *frame_ptrs, const uint8_t 
     return BGD_OK;
 }
 
+// The *_f32 blend entry points keep their contract: fp32 out in NTCHW or NCTHW; NTHWC is for the *_out entry points.
+static int f32_layout(const char *who, int layout)
+{
+    return layout == BGD_LAYOUT_NTHWC ? fail(BGD_ERR_INVALID, "%s: unknown layout %d", who, layout) : BGD_OK;
+}
+
 }  // namespace bgd
 
 // =================================================================================================
@@ -528,8 +534,9 @@ int bgd_bgmix_blend_f32(const uint8_t *d_fg, int64_t B, int64_t T, int64_t H, in
 {
     DeviceProps dp;
     if (int rc = current_device_props(&dp)) return rc;
+    if (int rc = f32_layout("bgmix", layout)) return rc;
     return launch_bgmix(d_fg, nullptr, B, T, H, W, d_bg_pool, false, P, Hb, Wb, d_bg_idx, d_top, d_left, d_apply, d_fg_lut,
-                        h_bg_mean, h_bg_std, alpha, layout, d_out, static_cast<cudaStream_t>(stream));
+                        h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out, static_cast<cudaStream_t>(stream));
 }
 
 int bgd_bgmix_blend_u8pool_f32(const uint8_t *d_fg, int64_t B, int64_t T, int64_t H, int64_t W,
@@ -540,8 +547,21 @@ int bgd_bgmix_blend_u8pool_f32(const uint8_t *d_fg, int64_t B, int64_t T, int64_
 {
     DeviceProps dp;
     if (int rc = current_device_props(&dp)) return rc;
+    if (int rc = f32_layout("bgmix", layout)) return rc;
     return launch_bgmix(d_fg, nullptr, B, T, H, W, d_bg_pool, true, P, Hb, Wb, d_bg_idx, d_top, d_left, d_apply, d_fg_lut,
-                        h_bg_mean, h_bg_std, alpha, layout, d_out, static_cast<cudaStream_t>(stream));
+                        h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out, static_cast<cudaStream_t>(stream));
+}
+
+int bgd_bgmix_blend_out(const uint8_t *d_fg, int64_t B, int64_t T, int64_t H, int64_t W, const void *d_bg_pool, int pool_is_u8,
+                        int64_t P, int64_t Hb, int64_t Wb, const int32_t *d_bg_idx, const int32_t *d_top, const int32_t *d_left,
+                        const uint8_t *d_apply, const float *d_fg_lut, const float *h_bg_mean, const float *h_bg_std,
+                        double alpha, int layout, int out_dtype, void *d_out, void *stream)
+{
+    DeviceProps dp;
+    if (int rc = current_device_props(&dp)) return rc;
+    if (!d_fg) return fail(BGD_ERR_INVALID, "bgmix: null foreground");
+    return launch_bgmix(d_fg, nullptr, B, T, H, W, d_bg_pool, pool_is_u8 != 0, P, Hb, Wb, d_bg_idx, d_top, d_left, d_apply,
+                        d_fg_lut, h_bg_mean, h_bg_std, alpha, layout, out_dtype, d_out, static_cast<cudaStream_t>(stream));
 }
 
 int bgd_bgmix_blend_normfg_f32(const float *d_fg_norm, int64_t B, int64_t T, int64_t H, int64_t W,
@@ -553,8 +573,10 @@ int bgd_bgmix_blend_normfg_f32(const float *d_fg_norm, int64_t B, int64_t T, int
     DeviceProps dp;
     if (int rc = current_device_props(&dp)) return rc;
     if (!d_fg_norm) return fail(BGD_ERR_INVALID, "bgmix: null foreground");
+    if (int rc = f32_layout("bgmix", layout)) return rc;
     return launch_bgmix(nullptr, d_fg_norm, B, T, H, W, d_bg_pool, pool_is_u8 != 0, P, Hb, Wb, d_bg_idx, d_top, d_left,
-                        d_apply, nullptr, h_bg_mean, h_bg_std, alpha, layout, d_out, static_cast<cudaStream_t>(stream));
+                        d_apply, nullptr, h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out,
+                        static_cast<cudaStream_t>(stream));
 }
 
 int bgd_aa_resize_table(int64_t in_size, int64_t out_size, int32_t *taps, int32_t *h_words, int64_t cap_words)
@@ -577,8 +599,22 @@ int bgd_bgmix_blend_ragged_f32(const uint8_t *d_fg, int64_t B, int64_t T, int64_
     DeviceProps dp;
     if (int rc = current_device_props(&dp)) return rc;
     if (!d_fg) return fail(BGD_ERR_INVALID, "bgmix (ragged): null foreground");
+    if (int rc = f32_layout("bgmix (ragged)", layout)) return rc;
     return launch_bgmix_ragged(d_fg, nullptr, B, T, H, W, d_pool, d_slots, P, d_tables, d_bg_idx, d_top, d_left, d_apply, d_fg_lut,
-                               h_bg_mean, h_bg_std, alpha, layout, d_out, static_cast<cudaStream_t>(stream));
+                               h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out, static_cast<cudaStream_t>(stream));
+}
+
+int bgd_bgmix_blend_ragged_out(const uint8_t *d_fg, int64_t B, int64_t T, int64_t H, int64_t W, const uint8_t *d_pool,
+                               const bgd_ragged_slot *d_slots, int64_t P, const int32_t *d_tables, const int32_t *d_bg_idx,
+                               const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply, const float *d_fg_lut,
+                               const float *h_bg_mean, const float *h_bg_std, double alpha, int layout, int out_dtype,
+                               void *d_out, void *stream)
+{
+    DeviceProps dp;
+    if (int rc = current_device_props(&dp)) return rc;
+    if (!d_fg) return fail(BGD_ERR_INVALID, "bgmix (ragged): null foreground");
+    return launch_bgmix_ragged(d_fg, nullptr, B, T, H, W, d_pool, d_slots, P, d_tables, d_bg_idx, d_top, d_left, d_apply, d_fg_lut,
+                               h_bg_mean, h_bg_std, alpha, layout, out_dtype, d_out, static_cast<cudaStream_t>(stream));
 }
 
 int bgd_bgmix_blend_ragged_normfg_f32(const float *d_fg_norm, int64_t B, int64_t T, int64_t H, int64_t W, const uint8_t *d_pool,
@@ -590,8 +626,9 @@ int bgd_bgmix_blend_ragged_normfg_f32(const float *d_fg_norm, int64_t B, int64_t
     DeviceProps dp;
     if (int rc = current_device_props(&dp)) return rc;
     if (!d_fg_norm) return fail(BGD_ERR_INVALID, "bgmix (ragged): null foreground");
+    if (int rc = f32_layout("bgmix (ragged)", layout)) return rc;
     return launch_bgmix_ragged(nullptr, d_fg_norm, B, T, H, W, d_pool, d_slots, P, d_tables, d_bg_idx, d_top, d_left, d_apply,
-                               nullptr, h_bg_mean, h_bg_std, alpha, layout, d_out, static_cast<cudaStream_t>(stream));
+                               nullptr, h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out, static_cast<cudaStream_t>(stream));
 }
 
 int bgd_resized_crop_aa_u8_f32(const uint8_t *d_src, int64_t src_bytes, const bgd_crop_desc *h_desc, int64_t n,
@@ -620,8 +657,22 @@ int bgd_bgmix_resize_blend_f32(const uint8_t *d_src, int64_t src_bytes, const in
 {
     DeviceProps dp;
     if (int rc = current_device_props(&dp)) return rc;
+    if (int rc = f32_layout("bgmix_resize", layout)) return rc;
     return launch_resize_blend(d_src, src_bytes, h_geom, B, T, H, W, d_bg_pool, pool_is_u8 != 0, P, Hb, Wb, d_bg_idx, d_top,
-                               d_left, d_apply, d_fg_lut, h_bg_mean, h_bg_std, alpha, layout, d_out,
+                               d_left, d_apply, d_fg_lut, h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out,
+                               static_cast<cudaStream_t>(stream));
+}
+
+int bgd_bgmix_resize_blend_out(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t B, int64_t T, int64_t H,
+                               int64_t W, const void *d_bg_pool, int pool_is_u8, int64_t P, int64_t Hb, int64_t Wb,
+                               const int32_t *d_bg_idx, const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply,
+                               const float *d_fg_lut, const float *h_bg_mean, const float *h_bg_std, double alpha, int layout,
+                               int out_dtype, void *d_out, void *stream)
+{
+    DeviceProps dp;
+    if (int rc = current_device_props(&dp)) return rc;
+    return launch_resize_blend(d_src, src_bytes, h_geom, B, T, H, W, d_bg_pool, pool_is_u8 != 0, P, Hb, Wb, d_bg_idx, d_top,
+                               d_left, d_apply, d_fg_lut, h_bg_mean, h_bg_std, alpha, layout, out_dtype, d_out,
                                static_cast<cudaStream_t>(stream));
 }
 
@@ -632,6 +683,7 @@ int bgd_bgmix_blend_f32_host(const uint8_t *h_fg, int64_t B, int64_t T, int64_t 
                              double *h_checksum, int device)
 {
     if (B < 0 || T < 0 || H < 0 || W < 0) return fail(BGD_ERR_INVALID, "bgmix: negative size");
+    if (int rc = f32_layout("bgmix", layout)) return rc;
     if (B == 0 || T == 0 || H == 0 || W == 0) { if (h_checksum) *h_checksum = 0.0; return BGD_OK; }
     if (!h_fg || !h_bg_idx || !h_top || !h_left || !h_apply) return fail(BGD_ERR_INVALID, "bgmix: null host pointer");
     // the reference's RandomCrop raises when the crop does not fit; validate here, on host values
@@ -666,7 +718,7 @@ int bgd_bgmix_blend_f32_host(const uint8_t *h_fg, int64_t B, int64_t T, int64_t 
     }
     const int32_t *d_idx = reinterpret_cast<const int32_t *>(dp_ + o);
     if (int rc = launch_bgmix(dp_, nullptr, B, T, H, W, d_bg_pool, false, P, Hb, Wb, d_idx, d_idx + B, d_idx + 2 * B,
-                              dp_ + o + (size_t)B * 12, d_fg_lut, h_bg_mean, h_bg_std, alpha, layout, d_out, s))
+                              dp_ + o + (size_t)B * 12, d_fg_lut, h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out, s))
         return rc;
     if (h_checksum) {
         double *d_sum = reinterpret_cast<double *>(st.d_out[0]);
@@ -686,6 +738,7 @@ int bgd_bgmix_resize_blend_f32_host(const uint8_t *h_src, int64_t src_bytes, con
                                     int device)
 {
     if (B < 0 || T < 0 || H < 0 || W < 0 || src_bytes < 0) return fail(BGD_ERR_INVALID, "bgmix_resize: negative size");
+    if (int rc = f32_layout("bgmix_resize", layout)) return rc;
     if (B == 0 || T == 0 || H == 0 || W == 0) { if (h_checksum) *h_checksum = 0.0; return BGD_OK; }
     if (!h_src || !h_geom || !h_bg_idx || !h_top || !h_left || !h_apply) return fail(BGD_ERR_INVALID, "bgmix_resize: null host pointer");
     if (src_bytes % 4) return fail(BGD_ERR_INVALID, "bgmix_resize: the source buffer must be a multiple of 4 bytes long");
@@ -721,7 +774,7 @@ int bgd_bgmix_resize_blend_f32_host(const uint8_t *h_src, int64_t src_bytes, con
     const int32_t *d_idx = reinterpret_cast<const int32_t *>(dp_ + o);
     if (int rc = launch_resize_blend(dp_, src_bytes, h_geom, B, T, H, W, d_bg_pool, false, P, Hb, Wb, d_idx, d_idx + B,
                                      d_idx + 2 * B, dp_ + o + (size_t)B * 12, d_fg_lut, h_bg_mean, h_bg_std, alpha, layout,
-                                     d_out, s))
+                                     BGD_OUT_F32, d_out, s))
         return rc;
     if (h_checksum) {
         double *d_sum = reinterpret_cast<double *>(st.d_out[0]);

@@ -1,6 +1,8 @@
 // Shared helpers for libbgdebias_b200.so (sm_100a only).
 #pragma once
 
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
 #include <atomic>
@@ -8,10 +10,87 @@
 #include <cstdint>
 #include <cstdio>
 #include <string>
+#include <type_traits>
 
 #include "bgdebias.h"
 
 namespace bgd {
+
+// ---- output element types of the batch blends (BGD_OUT_*) --------------------------------
+// The blend is computed in fp32 exactly as before; a 16-bit output is that value converted once, round to nearest even
+// (what torch's .to(torch.bfloat16) / .to(torch.float16) does).  Stores stream past L2 (st.global.cs) like the fp32 ones.
+template <typename OutT> struct OutElem;
+template <> struct OutElem<__nv_bfloat16> {
+    static __device__ __forceinline__ unsigned short one(float v) { return __bfloat16_as_ushort(__float2bfloat16_rn(v)); }
+    static __device__ __forceinline__ uint32_t two(float lo, float hi)
+    {
+        const __nv_bfloat162 p = __floats2bfloat162_rn(lo, hi);
+        return (uint32_t)__bfloat16_as_ushort(p.x) | ((uint32_t)__bfloat16_as_ushort(p.y) << 16);
+    }
+};
+template <> struct OutElem<__half> {
+    static __device__ __forceinline__ unsigned short one(float v) { return __half_as_ushort(__float2half_rn(v)); }
+    static __device__ __forceinline__ uint32_t two(float lo, float hi)
+    {
+        const __half2 p = __floats2half2_rn(lo, hi);
+        return (uint32_t)__half_as_ushort(p.x) | ((uint32_t)__half_as_ushort(p.y) << 16);
+    }
+};
+
+// one value
+__device__ __forceinline__ void store_out(float *p, float v) { __stcs(p, v); }
+template <typename OutT> __device__ __forceinline__ void store_out(OutT *p, float v)
+{
+    __stcs(reinterpret_cast<unsigned short *>(p), OutElem<OutT>::one(v));
+}
+
+// 4 consecutive values of one channel plane (p 16-byte aligned for fp32, 8-byte for 16-bit)
+__device__ __forceinline__ void store_out4(float *p, const float (&r)[4])
+{
+    __stcs(reinterpret_cast<float4 *>(p), make_float4(r[0], r[1], r[2], r[3]));
+}
+template <typename OutT> __device__ __forceinline__ void store_out4(OutT *p, const float (&r)[4])
+{
+    __stcs(reinterpret_cast<uint2 *>(p), make_uint2(OutElem<OutT>::two(r[0], r[1]), OutElem<OutT>::two(r[2], r[3])));
+}
+
+// 4 pixels x 3 channels, channel innermost (BGD_LAYOUT_NTHWC): the 12 values r[c][i] go to p[3 * i + c], as three 16-byte
+// (fp32) or 8-byte (16-bit) stores; p is aligned like store_out4's when the first pixel's index is a multiple of 4
+__device__ __forceinline__ void store_out12(float *p, const float (&r)[3][4])
+{
+    __stcs(reinterpret_cast<float4 *>(p), make_float4(r[0][0], r[1][0], r[2][0], r[0][1]));
+    __stcs(reinterpret_cast<float4 *>(p + 4), make_float4(r[1][1], r[2][1], r[0][2], r[1][2]));
+    __stcs(reinterpret_cast<float4 *>(p + 8), make_float4(r[2][2], r[0][3], r[1][3], r[2][3]));
+}
+template <typename OutT> __device__ __forceinline__ void store_out12(OutT *p, const float (&r)[3][4])
+{
+    using E = OutElem<OutT>;
+    uint2 *q = reinterpret_cast<uint2 *>(p);
+    __stcs(q, make_uint2(E::two(r[0][0], r[1][0]), E::two(r[2][0], r[0][1])));
+    __stcs(q + 1, make_uint2(E::two(r[1][1], r[2][1]), E::two(r[0][2], r[1][2])));
+    __stcs(q + 2, make_uint2(E::two(r[2][2], r[0][3]), E::two(r[1][3], r[2][3])));
+}
+
+inline int out_elem_bytes(int out_dtype)           // 0 = not a BGD_OUT_* value
+{
+    return out_dtype == BGD_OUT_F32 ? 4 : (out_dtype == BGD_OUT_BF16 || out_dtype == BGD_OUT_F16) ? 2 : 0;
+}
+
+// Calls f(Tag<OutT>{}, std::integral_constant<bool, INTERLEAVED>{}) for the output type and layout of a launch, so that a
+// launcher instantiates its kernel once per (type, planar / interleaved); NTCHW and NCTHW are both planar (strides).
+// The caller has validated both arguments.
+template <typename T> struct Tag { using type = T; };
+template <typename F> void dispatch_out(int out_dtype, int layout, F &&f)
+{
+    const bool il = layout == BGD_LAYOUT_NTHWC;
+    if (out_dtype == BGD_OUT_BF16) {
+        if (il) f(Tag<__nv_bfloat16>{}, std::true_type{}); else f(Tag<__nv_bfloat16>{}, std::false_type{});
+    } else if (out_dtype == BGD_OUT_F16) {
+        if (il) f(Tag<__half>{}, std::true_type{}); else f(Tag<__half>{}, std::false_type{});
+    } else {
+        if (il) f(Tag<float>{}, std::true_type{}); else f(Tag<float>{}, std::false_type{});
+    }
+}
 
 // ---- error state (per host thread) -------------------------------------------------------
 std::string &last_error_ref();
@@ -58,20 +137,20 @@ int launch_bgmix(const uint8_t *d_fg, const float *d_fg_norm, int64_t B, int64_t
                  bool pool_is_u8, int64_t P, int64_t Hb, int64_t Wb, const int32_t *d_bg_idx,
                  const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply,
                  const float *d_lut, const float *h_mean, const float *h_std, double alpha,
-                 int layout, float *d_out, cudaStream_t stream);
+                 int layout, int out_dtype, void *d_out, cudaStream_t stream);
 int launch_resize_u8(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t B, int64_t T, int64_t H, int64_t W,
                      uint8_t *d_out, cudaStream_t stream);
 int launch_resize_blend(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t B, int64_t T, int64_t H,
                         int64_t W, const void *d_pool, bool pool_is_u8, int64_t P, int64_t Hb, int64_t Wb,
                         const int32_t *d_bg_idx, const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply,
-                        const float *d_lut, const float *h_mean, const float *h_std, double alpha, int layout, float *d_out,
-                        cudaStream_t stream);
+                        const float *d_lut, const float *h_mean, const float *h_std, double alpha, int layout, int out_dtype,
+                        void *d_out, cudaStream_t stream);
 int aa_resize_table(int64_t in_size, int64_t out_size, int32_t *K_out, int32_t *words, int64_t cap_words);
 int launch_bgmix_ragged(const uint8_t *d_fg, const float *d_fg_norm, int64_t B, int64_t T, int64_t H, int64_t W,
                         const uint8_t *d_pool, const bgd_ragged_slot *d_slots, int64_t P, const int32_t *d_tables,
                         const int32_t *d_bg_idx, const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply,
-                        const float *d_lut, const float *h_mean, const float *h_std, double alpha, int layout, float *d_out,
-                        cudaStream_t stream);
+                        const float *d_lut, const float *h_mean, const float *h_std, double alpha, int layout, int out_dtype,
+                        void *d_out, cudaStream_t stream);
 int launch_aa_resize(const uint8_t *d_img, const bgd_ragged_slot *h_slot, const int32_t *d_tables, float *d_out, cudaStream_t stream);
 int launch_resized_crop_aa(const uint8_t *d_src, int64_t src_bytes, const bgd_crop_desc *h_desc, int64_t n,
                            const int32_t *d_tables, int64_t table_words, int64_t out_h, int64_t out_w, float *d_out,

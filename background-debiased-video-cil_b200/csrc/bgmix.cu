@@ -31,17 +31,19 @@ struct MixParams {
     const int32_t *bg_idx, *top, *left;
     const uint8_t *apply;
     const float *lut;
-    float *out;
+    void *out;                            // float, or OutT of bgmix_kernel
     int64_t T, H, W, P, Hb, Wb;
     float mean[3], std[3];
     float w_fg, w_bg;
-    int64_t out_stride_t, out_stride_c;   // in elements; layout folded into strides
+    int64_t out_stride_t, out_stride_c;   // in elements; NTCHW / NCTHW folded into strides (NTHWC: 3 * H * W, 1)
 };
 
 template <typename PoolT>
 __device__ __forceinline__ float load_bg(const PoolT *p) { return (float)__ldg(p); }
 
-template <typename PoolT, int PX>
+// OutT: float, __nv_bfloat16 or __half.  IL (BGD_LAYOUT_NTHWC): a pixel's 3 channels are adjacent in the output, so the
+// 4 pixels of a thread make 12 consecutive values (store_out12) instead of three 4-value runs, one per channel plane.
+template <typename PoolT, int PX, typename OutT, bool IL>
 __global__ void __launch_bounds__(kThreads, kMixMinBlocks) bgmix_kernel(const MixParams prm)
 {
     __shared__ float s_lut[3 * 256];
@@ -73,7 +75,7 @@ __global__ void __launch_bounds__(kThreads, kMixMinBlocks) bgmix_kernel(const Mi
     }
 
     const uint8_t *fg = prm.fg + (b * prm.T * HW + p0) * 3;
-    float *out = prm.out + b * prm.T * 3 * HW + p0;
+    OutT *out = static_cast<OutT *>(prm.out) + b * prm.T * 3 * HW + (IL ? 3 * p0 : p0);
 
 #pragma unroll kMixUnroll
     for (int64_t t = 0; t < prm.T; ++t) {
@@ -91,22 +93,19 @@ __global__ void __launch_bounds__(kThreads, kMixMinBlocks) bgmix_kernel(const Mi
 #pragma unroll
             for (int k = 0; k < 3 * PX; ++k) px[k] = __ldcs(fg + t * HW * 3 + k);
         }
+        float r[3][PX];
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
-            float r[PX];
 #pragma unroll
             for (int i = 0; i < PX; ++i) {
                 const float f = s_lut[c * 256 + px[i * 3 + c]];
-                r[i] = apply ? __fadd_rn(__fmul_rn(f, prm.w_fg), g[c][i]) : f;
+                r[c][i] = apply ? __fadd_rn(__fmul_rn(f, prm.w_fg), g[c][i]) : f;
             }
-            float *dst = out + t * prm.out_stride_t + c * prm.out_stride_c;
-            if (PX == 4) {
-                __stcs(reinterpret_cast<float4 *>(dst), make_float4(r[0], r[1], r[2], r[3]));
-            } else {
-#pragma unroll
-                for (int i = 0; i < PX; ++i) __stcs(dst + i, r[i]);
-            }
+            OutT *dst = out + t * prm.out_stride_t + c * prm.out_stride_c;
+            if constexpr (PX == 4 && !IL) store_out4(dst, r[c]);
+            else if constexpr (PX == 1) store_out(dst, r[c][0]);
         }
+        if constexpr (PX == 4 && IL) store_out12(out + t * prm.out_stride_t, r);
     }
 }
 
@@ -134,7 +133,7 @@ __global__ void __launch_bounds__(kThreads) bgmix_normfg_kernel(const MixParams 
             g[i] = __fmul_rn(__fdiv_rn(__fsub_rn(load_bg(pb + i), prm.mean[c]), prm.std[c]), prm.w_bg);
     }
     const float *src = fgn + (b * prm.T * 3 + c) * HW + p0;
-    float *out = prm.out + b * prm.T * 3 * HW + c * prm.out_stride_c + p0;
+    float *out = static_cast<float *>(prm.out) + b * prm.T * 3 * HW + c * prm.out_stride_c + p0;
     for (int64_t t = 0; t < prm.T; ++t) {
         float f[VEC];
         if (VEC == 4) {
@@ -177,7 +176,7 @@ int launch_bgmix(const uint8_t *d_fg, const float *d_fg_norm, int64_t B, int64_t
                  bool pool_is_u8, int64_t P, int64_t Hb, int64_t Wb, const int32_t *d_bg_idx,
                  const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply,
                  const float *d_lut, const float *h_mean, const float *h_std, double alpha, int layout,
-                 float *d_out, cudaStream_t stream)
+                 int out_dtype, void *d_out, cudaStream_t stream)
 {
     if (B < 0 || T < 0 || H < 0 || W < 0) return fail(BGD_ERR_INVALID, "bgmix: negative size");
     if (B == 0 || T == 0 || H == 0 || W == 0) return BGD_OK;
@@ -187,7 +186,12 @@ int launch_bgmix(const uint8_t *d_fg, const float *d_fg_norm, int64_t B, int64_t
     if (P > 0 && (Hb < H || Wb < W))
         return fail(BGD_ERR_INVALID, "bgmix: crop %lldx%lld larger than pool image %lldx%lld",
                     (long long)H, (long long)W, (long long)Hb, (long long)Wb);
-    if (layout != BGD_LAYOUT_NTCHW && layout != BGD_LAYOUT_NCTHW) return fail(BGD_ERR_INVALID, "bgmix: unknown layout %d", layout);
+    if (layout != BGD_LAYOUT_NTCHW && layout != BGD_LAYOUT_NCTHW && layout != BGD_LAYOUT_NTHWC)
+        return fail(BGD_ERR_INVALID, "bgmix: unknown layout %d", layout);
+    const int out_bytes = out_elem_bytes(out_dtype);
+    if (!out_bytes) return fail(BGD_ERR_INVALID, "bgmix: unknown output type %d", out_dtype);
+    if (d_fg_norm && (layout == BGD_LAYOUT_NTHWC || out_dtype != BGD_OUT_F32))
+        return fail(BGD_ERR_INVALID, "bgmix: a normalised foreground blends to fp32 NTCHW / NCTHW only");
     if (B > 65535) return fail(BGD_ERR_INVALID, "bgmix: batch larger than 65535");
 
     MixParams prm{};
@@ -198,8 +202,9 @@ int launch_bgmix(const uint8_t *d_fg, const float *d_fg_norm, int64_t B, int64_t
     prm.w_fg = (float)(1.0 - alpha);      // python: (1 - alpha) in double, then tensor * scalar rounds to fp32
     prm.w_bg = (float)alpha;
     const int64_t HW = H * W;
-    if (layout == BGD_LAYOUT_NTCHW) { prm.out_stride_t = 3 * HW; prm.out_stride_c = HW; }
-    else                            { prm.out_stride_t = HW;     prm.out_stride_c = T * HW; }
+    if (layout == BGD_LAYOUT_NTCHW)      { prm.out_stride_t = 3 * HW; prm.out_stride_c = HW; }
+    else if (layout == BGD_LAYOUT_NCTHW) { prm.out_stride_t = HW;     prm.out_stride_c = T * HW; }
+    else                                 { prm.out_stride_t = 3 * HW; prm.out_stride_c = 1; }
 
     if (d_fg_norm) {
         const bool v4 = (W % 4 == 0) && reinterpret_cast<uintptr_t>(d_fg_norm) % 16 == 0 && reinterpret_cast<uintptr_t>(d_out) % 16 == 0;
@@ -216,17 +221,22 @@ int launch_bgmix(const uint8_t *d_fg, const float *d_fg_norm, int64_t B, int64_t
         BGD_CUDA_TRY(cudaGetLastError());
         return BGD_OK;
     }
+    // 4-pixel vectors: W % 4 == 0 keeps every thread's first pixel a multiple of 4, so its stores stay aligned
     const bool vec = (W % 4 == 0) && (reinterpret_cast<uintptr_t>(d_fg) % 4 == 0) &&
-                     (reinterpret_cast<uintptr_t>(d_out) % 16 == 0);
+                     (reinterpret_cast<uintptr_t>(d_out) % (4 * out_bytes) == 0);
     const int px = vec ? 4 : 1;
     dim3 grid((unsigned)((HW / px + kThreads - 1) / kThreads), (unsigned)B);
-    if (pool_is_u8) {
-        if (vec) bgmix_kernel<uint8_t, 4><<<grid, kThreads, 0, stream>>>(prm);
-        else     bgmix_kernel<uint8_t, 1><<<grid, kThreads, 0, stream>>>(prm);
-    } else {
-        if (vec) bgmix_kernel<float, 4><<<grid, kThreads, 0, stream>>>(prm);
-        else     bgmix_kernel<float, 1><<<grid, kThreads, 0, stream>>>(prm);
-    }
+    dispatch_out(out_dtype, layout, [&](auto o, auto il) {
+        using OutT = typename decltype(o)::type;
+        constexpr bool IL = decltype(il)::value;
+        if (pool_is_u8) {
+            if (vec) bgmix_kernel<uint8_t, 4, OutT, IL><<<grid, kThreads, 0, stream>>>(prm);
+            else     bgmix_kernel<uint8_t, 1, OutT, IL><<<grid, kThreads, 0, stream>>>(prm);
+        } else {
+            if (vec) bgmix_kernel<float, 4, OutT, IL><<<grid, kThreads, 0, stream>>>(prm);
+            else     bgmix_kernel<float, 1, OutT, IL><<<grid, kThreads, 0, stream>>>(prm);
+        }
+    });
     count_launch();
     BGD_CUDA_TRY(cudaGetLastError());
     return BGD_OK;

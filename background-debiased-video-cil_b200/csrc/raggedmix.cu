@@ -47,11 +47,11 @@ struct RaggedParams {
     const int32_t *bg_idx, *top, *left;
     const uint8_t *apply;
     const float *lut;
-    float *out;
+    void *out;                        // float, or OutT of the uint8-foreground kernels
     int64_t T, H, W, P;
     float mean[3], std[3];
     float w_fg, w_bg;
-    int64_t out_stride_t, out_stride_c;
+    int64_t out_stride_t, out_stride_c;   // in elements (NTHWC: 3 * H * W, 1)
 };
 
 __device__ __forceinline__ bgd_ragged_slot load_slot(const RaggedParams &prm, int64_t b, int &top, int &left)
@@ -64,8 +64,9 @@ __device__ __forceinline__ bgd_ragged_slot load_slot(const RaggedParams &prm, in
     return s;
 }
 
-// uint8 foreground [B][T][H][W][3]: one thread owns PX adjacent pixels of one sample for all T frames (as bgmix_kernel)
-template <int PX>
+// uint8 foreground [B][T][H][W][3]: one thread owns PX adjacent pixels of one sample for all T frames (as bgmix_kernel,
+// whose OutT / IL this kernel and the tile kernel share)
+template <int PX, typename OutT, bool IL>
 __global__ void __launch_bounds__(kThreads) bgmix_ragged_kernel(const RaggedParams prm)
 {
     __shared__ float s_lut[3 * 256];
@@ -95,7 +96,7 @@ __global__ void __launch_bounds__(kThreads) bgmix_ragged_kernel(const RaggedPara
     }
 
     const uint8_t *fg = prm.fg + (b * prm.T * HW + p0) * 3;
-    float *out = prm.out + b * prm.T * 3 * HW + p0;
+    OutT *out = static_cast<OutT *>(prm.out) + b * prm.T * 3 * HW + (IL ? 3 * p0 : p0);
 #pragma unroll 2
     for (int64_t t = 0; t < prm.T; ++t) {
         uint8_t px[3 * PX];
@@ -112,22 +113,19 @@ __global__ void __launch_bounds__(kThreads) bgmix_ragged_kernel(const RaggedPara
 #pragma unroll
             for (int k = 0; k < 3 * PX; ++k) px[k] = __ldcs(fg + t * HW * 3 + k);
         }
+        float r[3][PX];
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
-            float r[PX];
 #pragma unroll
             for (int i = 0; i < PX; ++i) {
                 const float f = s_lut[c * 256 + px[i * 3 + c]];
-                r[i] = apply ? __fadd_rn(__fmul_rn(f, prm.w_fg), g[c][i]) : f;
+                r[c][i] = apply ? __fadd_rn(__fmul_rn(f, prm.w_fg), g[c][i]) : f;
             }
-            float *dst = out + t * prm.out_stride_t + c * prm.out_stride_c;
-            if (PX == 4) {
-                __stcs(reinterpret_cast<float4 *>(dst), make_float4(r[0], r[1], r[2], r[3]));
-            } else {
-#pragma unroll
-                for (int i = 0; i < PX; ++i) __stcs(dst + i, r[i]);
-            }
+            OutT *dst = out + t * prm.out_stride_t + c * prm.out_stride_c;
+            if constexpr (PX == 4 && !IL) store_out4(dst, r[c]);
+            else if constexpr (PX == 1) store_out(dst, r[c][0]);
         }
+        if constexpr (PX == 4 && IL) store_out12(out + t * prm.out_stride_t, r);
     }
 }
 
@@ -145,6 +143,7 @@ constexpr int kMaxSrcRows = 48;           // source rows of one tile kept in sha
 #define BGD_RAGGED_MINBLOCKS 6
 #endif
 
+template <typename OutT, bool IL>
 __global__ void __launch_bounds__(kThreads, BGD_RAGGED_MINBLOCKS) bgmix_ragged_tile_kernel(const RaggedParams prm)
 {
     __shared__ float s_lut[3 * 256];
@@ -206,7 +205,7 @@ __global__ void __launch_bounds__(kThreads, BGD_RAGGED_MINBLOCKS) bgmix_ragged_t
     const int64_t HW = prm.H * prm.W;
     const int64_t p0 = (int64_t)(ty0 + ty) * W + tx0 + tx;
     const uint8_t *fg = prm.fg + (b * prm.T * HW + p0) * 3;
-    float *out = prm.out + b * prm.T * 3 * HW + p0;
+    OutT *out = static_cast<OutT *>(prm.out) + b * prm.T * 3 * HW + (IL ? 3 * p0 : p0);
 #pragma unroll 4
     for (int64_t t = 0; t < prm.T; ++t) {
         const uint32_t *src = reinterpret_cast<const uint32_t *>(fg + t * HW * 3);
@@ -218,16 +217,17 @@ __global__ void __launch_bounds__(kThreads, BGD_RAGGED_MINBLOCKS) bgmix_ragged_t
             px[4 + k] = (w1 >> (8 * k)) & 0xFF;
             px[8 + k] = (w2 >> (8 * k)) & 0xFF;
         }
+        float r[3][4];
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
-            float r[4];
 #pragma unroll
             for (int i = 0; i < 4; ++i) {
                 const float f = s_lut[c * 256 + px[i * 3 + c]];
-                r[i] = apply ? __fadd_rn(__fmul_rn(f, prm.w_fg), g[c][i]) : f;
+                r[c][i] = apply ? __fadd_rn(__fmul_rn(f, prm.w_fg), g[c][i]) : f;
             }
-            __stcs(reinterpret_cast<float4 *>(out + t * prm.out_stride_t + c * prm.out_stride_c), make_float4(r[0], r[1], r[2], r[3]));
+            if constexpr (!IL) store_out4(out + t * prm.out_stride_t + c * prm.out_stride_c, r[c]);
         }
+        if constexpr (IL) store_out12(out + t * prm.out_stride_t, r);
     }
 }
 
@@ -249,7 +249,7 @@ __global__ void __launch_bounds__(kThreads) bgmix_ragged_normfg_kernel(const Rag
         g = __fmul_rn(__fdiv_rn(__fsub_rn(raw, prm.mean[c]), prm.std[c]), prm.w_bg);
     }
     const float *src = prm.fgn + (b * prm.T * 3 + c) * HW + p;
-    float *out = prm.out + b * prm.T * 3 * HW + c * prm.out_stride_c + p;
+    float *out = static_cast<float *>(prm.out) + b * prm.T * 3 * HW + c * prm.out_stride_c + p;
     for (int64_t t = 0; t < prm.T; ++t) {
         const float f = __ldcs(src + t * 3 * HW);
         __stcs(out + t * prm.out_stride_t, apply ? __fadd_rn(__fmul_rn(f, prm.w_fg), g) : f);
@@ -322,13 +322,15 @@ int aa_resize_table(int64_t in_size, int64_t out_size, int32_t *K_out, int32_t *
 static int fill_params(RaggedParams &prm, int64_t B, int64_t T, int64_t H, int64_t W, const uint8_t *d_pool,
                        const bgd_ragged_slot *d_slots, int64_t P, const int32_t *d_tables, const int32_t *d_bg_idx,
                        const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply, const float *h_mean,
-                       const float *h_std, double alpha, int layout, float *d_out)
+                       const float *h_std, double alpha, int layout, int out_dtype, void *d_out)
 {
     if (B < 0 || T < 0 || H < 0 || W < 0 || P < 0) return fail(BGD_ERR_INVALID, "bgmix (ragged): negative size");
     if (!d_out || !d_apply) return fail(BGD_ERR_INVALID, "bgmix (ragged): null pointer");
     if (!h_mean || !h_std) return fail(BGD_ERR_INVALID, "bgmix (ragged): null mean/std");
     if (P > 0 && (!d_pool || !d_slots || !d_bg_idx || !d_top || !d_left)) return fail(BGD_ERR_INVALID, "bgmix (ragged): null pool argument");
-    if (layout != BGD_LAYOUT_NTCHW && layout != BGD_LAYOUT_NCTHW) return fail(BGD_ERR_INVALID, "bgmix (ragged): unknown layout %d", layout);
+    if (layout != BGD_LAYOUT_NTCHW && layout != BGD_LAYOUT_NCTHW && layout != BGD_LAYOUT_NTHWC)
+        return fail(BGD_ERR_INVALID, "bgmix (ragged): unknown layout %d", layout);
+    if (!out_elem_bytes(out_dtype)) return fail(BGD_ERR_INVALID, "bgmix (ragged): unknown output type %d", out_dtype);
     if (B > 65535) return fail(BGD_ERR_INVALID, "bgmix (ragged): batch larger than 65535");
     if (H >= (1 << 24) || W >= (1 << 24)) return fail(BGD_ERR_INVALID, "bgmix (ragged): crop too large");
     prm.pool = d_pool; prm.slots = d_slots; prm.tables = d_tables; prm.bg_idx = d_bg_idx; prm.top = d_top; prm.left = d_left;
@@ -338,20 +340,21 @@ static int fill_params(RaggedParams &prm, int64_t B, int64_t T, int64_t H, int64
     prm.w_fg = (float)(1.0 - alpha);
     prm.w_bg = (float)alpha;
     const int64_t HW = H * W;
-    if (layout == BGD_LAYOUT_NTCHW) { prm.out_stride_t = 3 * HW; prm.out_stride_c = HW; }
-    else                            { prm.out_stride_t = HW;     prm.out_stride_c = T * HW; }
+    if (layout == BGD_LAYOUT_NTCHW)      { prm.out_stride_t = 3 * HW; prm.out_stride_c = HW; }
+    else if (layout == BGD_LAYOUT_NCTHW) { prm.out_stride_t = HW;     prm.out_stride_c = T * HW; }
+    else                                 { prm.out_stride_t = 3 * HW; prm.out_stride_c = 1; }
     return BGD_OK;
 }
 
 int launch_bgmix_ragged(const uint8_t *d_fg, const float *d_fg_norm, int64_t B, int64_t T, int64_t H, int64_t W,
                         const uint8_t *d_pool, const bgd_ragged_slot *d_slots, int64_t P, const int32_t *d_tables,
                         const int32_t *d_bg_idx, const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply,
-                        const float *d_lut, const float *h_mean, const float *h_std, double alpha, int layout, float *d_out,
-                        cudaStream_t stream)
+                        const float *d_lut, const float *h_mean, const float *h_std, double alpha, int layout, int out_dtype,
+                        void *d_out, cudaStream_t stream)
 {
     RaggedParams prm{};
     if (int rc = fill_params(prm, B, T, H, W, d_pool, d_slots, P, d_tables, d_bg_idx, d_top, d_left, d_apply, h_mean, h_std, alpha,
-                             layout, d_out))
+                             layout, out_dtype, d_out))
         return rc;
     if (B == 0 || T == 0 || H == 0 || W == 0) return BGD_OK;
     if (!d_fg && !d_fg_norm) return fail(BGD_ERR_INVALID, "bgmix (ragged): null foreground");
@@ -359,19 +362,25 @@ int launch_bgmix_ragged(const uint8_t *d_fg, const float *d_fg_norm, int64_t B, 
     prm.fg = d_fg; prm.fgn = d_fg_norm; prm.lut = d_lut;
     const int64_t HW = H * W;
     if (d_fg_norm) {
+        if (layout == BGD_LAYOUT_NTHWC || out_dtype != BGD_OUT_F32)
+            return fail(BGD_ERR_INVALID, "bgmix (ragged): a normalised foreground blends to fp32 NTCHW / NCTHW only");
         dim3 grid((unsigned)((HW + kThreads - 1) / kThreads), 3u, (unsigned)B);
         bgmix_ragged_normfg_kernel<<<grid, kThreads, 0, stream>>>(prm);
     } else {
-        const bool vec = (W % 4 == 0) && (reinterpret_cast<uintptr_t>(d_fg) % 4 == 0) && (reinterpret_cast<uintptr_t>(d_out) % 16 == 0);
+        const bool vec = (W % 4 == 0) && (reinterpret_cast<uintptr_t>(d_fg) % 4 == 0) &&
+                         (reinterpret_cast<uintptr_t>(d_out) % (4 * out_elem_bytes(out_dtype)) == 0);
         const int px = vec ? 4 : 1;
         dim3 grid((unsigned)((HW / px + kThreads - 1) / kThreads), (unsigned)B);
         static const bool per_value = getenv("BGD_RAGGED_PER_VALUE") != nullptr;     // differential testing of the two forms
-        if (vec && !per_value) {
-            dim3 tgrid((unsigned)((W + kTile - 1) / kTile), (unsigned)((H + kTile - 1) / kTile), (unsigned)B);
-            if (tgrid.y > 65535) return fail(BGD_ERR_INVALID, "bgmix (ragged): crop too tall");
-            bgmix_ragged_tile_kernel<<<tgrid, kThreads, 0, stream>>>(prm);
-        } else if (vec) bgmix_ragged_kernel<4><<<grid, kThreads, 0, stream>>>(prm);
-        else            bgmix_ragged_kernel<1><<<grid, kThreads, 0, stream>>>(prm);
+        dim3 tgrid((unsigned)((W + kTile - 1) / kTile), (unsigned)((H + kTile - 1) / kTile), (unsigned)B);
+        if (vec && !per_value && tgrid.y > 65535) return fail(BGD_ERR_INVALID, "bgmix (ragged): crop too tall");
+        dispatch_out(out_dtype, layout, [&](auto o, auto il) {
+            using OutT = typename decltype(o)::type;
+            constexpr bool IL = decltype(il)::value;
+            if (vec && !per_value) bgmix_ragged_tile_kernel<OutT, IL><<<tgrid, kThreads, 0, stream>>>(prm);
+            else if (vec)          bgmix_ragged_kernel<4, OutT, IL><<<grid, kThreads, 0, stream>>>(prm);
+            else                   bgmix_ragged_kernel<1, OutT, IL><<<grid, kThreads, 0, stream>>>(prm);
+        });
     }
     count_launch();
     BGD_CUDA_TRY(cudaGetLastError());

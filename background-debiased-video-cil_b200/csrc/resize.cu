@@ -66,7 +66,7 @@ struct TailParams {
     const int32_t *bg_idx, *top, *left;
     const uint8_t *apply;
     const float *lut;
-    float *out;
+    void *out;                 // OutT of resize_blend_kernel
     uint8_t *out_u8;
     int64_t T, H, W, P, Hb, Wb;
     float mean[3], std[3];
@@ -162,7 +162,9 @@ __global__ void __launch_bounds__(kThreads) resize_u8_kernel(const TailParams pr
     else                           for_each_frame<false>(prm, g, t, emit);
 }
 
-template <typename PoolT>
+// OutT: float, __nv_bfloat16 or __half.  IL (BGD_LAYOUT_NTHWC): the pixel's 3 channels are adjacent in the output; a
+// lane then stores 3 consecutive values per frame and a warp still covers whole 32-byte sectors (scalar stores).
+template <typename PoolT, typename OutT, bool IL>
 __global__ void __launch_bounds__(kThreads, kBlendMinBlocks) resize_blend_kernel(const TailParams prm)
 {
     __shared__ float s_lut[3 * 256];
@@ -193,12 +195,13 @@ __global__ void __launch_bounds__(kThreads, kBlendMinBlocks) resize_blend_kernel
     }
 
     const int64_t HW = prm.H * prm.W;
-    float *out = prm.out + b * prm.T * 3 * HW + (int64_t)y * prm.W + x;
+    OutT *out = IL ? static_cast<OutT *>(prm.out) + b * prm.T * 3 * HW + 3 * ((int64_t)y * prm.W + x)
+                   : static_cast<OutT *>(prm.out) + b * prm.T * 3 * HW + (int64_t)y * prm.W + x;
     const int64_t st = prm.out_stride_t, sc = prm.out_stride_c;
     const float w_fg = prm.w_fg;
     auto emit = [&](int64_t f, int c, uint32_t v) {
         const float n = s_lut[c * 256 + v];
-        __stcs(out + f * st + c * sc, apply ? __fadd_rn(__fmul_rn(n, w_fg), bgw[c]) : n);
+        store_out(out + f * st + c * sc, apply ? __fadd_rn(__fmul_rn(n, w_fg), bgw[c]) : n);
     };
     if ((g.frame_stride & 3) == 0) for_each_frame<true>(prm, g, t, emit);
     else                           for_each_frame<false>(prm, g, t, emit);
@@ -331,8 +334,8 @@ int launch_resize_u8(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_g
 int launch_resize_blend(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t B, int64_t T, int64_t H,
                         int64_t W, const void *d_pool, bool pool_is_u8, int64_t P, int64_t Hb, int64_t Wb,
                         const int32_t *d_bg_idx, const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply,
-                        const float *d_lut, const float *h_mean, const float *h_std, double alpha, int layout, float *d_out,
-                        cudaStream_t stream)
+                        const float *d_lut, const float *h_mean, const float *h_std, double alpha, int layout, int out_dtype,
+                        void *d_out, cudaStream_t stream)
 {
     if (int rc = check_common(d_src, src_bytes, h_geom, B, T, H, W)) return rc;
     if (B == 0 || T == 0 || H == 0 || W == 0) return BGD_OK;
@@ -344,7 +347,9 @@ int launch_resize_blend(const uint8_t *d_src, int64_t src_bytes, const int64_t *
                     (long long)Hb, (long long)Wb);
     if (P > 0 && (Hb > INT32_MAX / 4 || Wb > INT32_MAX / 4 || 3 * Hb * Wb > INT32_MAX))
         return fail(BGD_ERR_INVALID, "bgmix_resize: pool images larger than 2^31 elements");
-    if (layout != BGD_LAYOUT_NTCHW && layout != BGD_LAYOUT_NCTHW) return fail(BGD_ERR_INVALID, "bgmix_resize: unknown layout %d", layout);
+    if (layout != BGD_LAYOUT_NTCHW && layout != BGD_LAYOUT_NCTHW && layout != BGD_LAYOUT_NTHWC)
+        return fail(BGD_ERR_INVALID, "bgmix_resize: unknown layout %d", layout);
+    if (!out_elem_bytes(out_dtype)) return fail(BGD_ERR_INVALID, "bgmix_resize: unknown output type %d", out_dtype);
 
     Workspace &ws = thread_workspace();
     TailParams prm{};
@@ -357,10 +362,15 @@ int launch_resize_blend(const uint8_t *d_src, int64_t src_bytes, const int64_t *
     prm.w_fg = (float)(1.0 - alpha);
     prm.w_bg = (float)alpha;
     const int64_t HW = H * W;
-    if (layout == BGD_LAYOUT_NTCHW) { prm.out_stride_t = 3 * HW; prm.out_stride_c = HW; }
-    else                            { prm.out_stride_t = HW;     prm.out_stride_c = T * HW; }
-    if (pool_is_u8) resize_blend_kernel<uint8_t><<<tile_grid(B, H, W), dim3(kTileW, kTileH), 0, stream>>>(prm);
-    else            resize_blend_kernel<float><<<tile_grid(B, H, W), dim3(kTileW, kTileH), 0, stream>>>(prm);
+    if (layout == BGD_LAYOUT_NTCHW)      { prm.out_stride_t = 3 * HW; prm.out_stride_c = HW; }
+    else if (layout == BGD_LAYOUT_NCTHW) { prm.out_stride_t = HW;     prm.out_stride_c = T * HW; }
+    else                                 { prm.out_stride_t = 3 * HW; prm.out_stride_c = 1; }
+    dispatch_out(out_dtype, layout, [&](auto o, auto il) {
+        using OutT = typename decltype(o)::type;
+        constexpr bool IL = decltype(il)::value;
+        if (pool_is_u8) resize_blend_kernel<uint8_t, OutT, IL><<<tile_grid(B, H, W), dim3(kTileW, kTileH), 0, stream>>>(prm);
+        else            resize_blend_kernel<float, OutT, IL><<<tile_grid(B, H, W), dim3(kTileW, kTileH), 0, stream>>>(prm);
+    });
     count_launch();
     cudaError_t e = cudaGetLastError();
     const int rc = e == cudaSuccess ? BGD_OK : fail(BGD_ERR_CUDA, "resize_blend_kernel launch failed: %s", cudaGetErrorString(e));

@@ -13,8 +13,11 @@ built library (``ImportError`` otherwise).  Ops are stream-ordered and never syn
         (what extract_background.py:102-109 does video by video).
     bgdebias::bgmix_blend(Tensor fg, Tensor bg_pool, Tensor bg_idx, Tensor top, Tensor left,
                           Tensor apply, Tensor fg_lut, Tensor bg_mean, Tensor bg_std,
-                          float alpha, str layout) -> Tensor
+                          float alpha, str layout, ScalarType? out_dtype=None) -> Tensor
         the batched form of BackgroundMixDataset._mix_background (libs/loader/comix_loader.py:138-145).
+        ``layout`` "NTCHW", "NCTHW" or "NTHWC" (contiguous [B, T, H, W, 3], channels-last storage of both others);
+        ``out_dtype`` float32 (None), bfloat16 or float16: the fp32 result rounded once, equal to its ``.to(out_dtype)``.
+        bgmix_blend_ragged and bgmix_resize_blend take the same two arguments.
     bgdebias::bgmix_blend_ragged(Tensor fg, Tensor pool_bytes, Tensor slots, Tensor tables, <bgmix_blend arguments>) -> Tensor
         the same blend over a ragged uint8 pool (images of any sizes, or the random frames of comix_loader.py:133-136),
         with Resize(bg_resize) (comix_loader.py:72; torchvision's antialiased bilinear, bit-exact) inside the launch.
@@ -30,7 +33,7 @@ from __future__ import annotations
 
 import ctypes
 import math
-from typing import Sequence, Tuple
+from typing import Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -227,15 +230,30 @@ def _host3(t: torch.Tensor, name: str):
     return _cabi.f32x3(t.detach().to("cpu", torch.float32).tolist())
 
 
+_OUT_DTYPES = {torch.float32: _cabi.OUT_F32, torch.bfloat16: _cabi.OUT_BF16, torch.float16: _cabi.OUT_F16}
+
+
+def _out_spec(name: str, layout: str, out_dtype: Optional[torch.dtype]) -> torch.dtype:
+    """Validates the output arguments of the uint8-foreground blends; returns the output dtype."""
+    _require(layout in _cabi.OUT_LAYOUTS, f"{name}: layout must be one of {sorted(_cabi.OUT_LAYOUTS)}")
+    dt = torch.float32 if out_dtype is None else out_dtype
+    _require(dt in _OUT_DTYPES, f"{name}: out_dtype must be float32, bfloat16 or float16 (got {dt})")
+    return dt
+
+
+def _out_shape(B: int, T: int, H: int, W: int, layout: str) -> tuple:
+    return {"NTCHW": (B, T, 3, H, W), "NCTHW": (B, 3, T, H, W), "NTHWC": (B, T, H, W, 3)}[layout]
+
+
 @torch.library.custom_op("bgdebias::bgmix_blend", mutates_args=(), device_types="cuda")
 def bgmix_blend(fg: torch.Tensor, bg_pool: torch.Tensor, bg_idx: torch.Tensor, top: torch.Tensor,
                 left: torch.Tensor, apply: torch.Tensor, fg_lut: torch.Tensor, bg_mean: torch.Tensor,
-                bg_std: torch.Tensor, alpha: float, layout: str) -> torch.Tensor:
+                bg_std: torch.Tensor, alpha: float, layout: str, out_dtype: Optional[torch.dtype] = None) -> torch.Tensor:
     _require(fg.dtype == torch.uint8 and fg.dim() == 5 and fg.shape[-1] == 3,
              "bgmix_blend: fg must be uint8 [B, T, H, W, 3]")
     _require(bg_pool.dim() == 4 and bg_pool.shape[1] == 3 and bg_pool.dtype in (torch.float32, torch.uint8),
              "bgmix_blend: bg_pool must be float32 or uint8 [P, 3, Hb, Wb]")
-    _require(layout in _cabi.LAYOUTS, f"bgmix_blend: layout must be one of {sorted(_cabi.LAYOUTS)}")
+    out_dt = _out_spec("bgmix_blend", layout, out_dtype)
     B, T, H, W, _ = fg.shape
     P, _, Hb, Wb = bg_pool.shape
     dev = fg.device
@@ -248,22 +266,20 @@ def bgmix_blend(fg: torch.Tensor, bg_pool: torch.Tensor, bg_idx: torch.Tensor, t
     _require(bg_pool.device == dev, "bgmix_blend: bg_pool must be on the same device as fg")
     fg, bg_pool = fg.contiguous(), bg_pool.contiguous()
     bg_idx, top, left, apply, fg_lut = (x.contiguous() for x in (bg_idx, top, left, apply, fg_lut))
-    shape = (B, T, 3, H, W) if layout == "NTCHW" else (B, 3, T, H, W)
-    out = torch.empty(shape, dtype=torch.float32, device=dev)
-    fn = _cabi.lib().bgd_bgmix_blend_f32 if bg_pool.dtype == torch.float32 else _cabi.lib().bgd_bgmix_blend_u8pool_f32
+    out = torch.empty(_out_shape(B, T, H, W, layout), dtype=out_dt, device=dev)
     with torch.cuda.device(dev):
-        _cabi.check(fn(fg.data_ptr(), B, T, H, W, bg_pool.data_ptr(), P, Hb, Wb, bg_idx.data_ptr(), top.data_ptr(),
-                       left.data_ptr(), apply.data_ptr(), fg_lut.data_ptr(), _host3(bg_mean, "bg_mean"),
-                       _host3(bg_std, "bg_std"), float(alpha), _cabi.LAYOUTS[layout], out.data_ptr(),
-                       _stream_ptr(dev)))
+        _cabi.check(_cabi.lib().bgd_bgmix_blend_out(
+            fg.data_ptr(), B, T, H, W, bg_pool.data_ptr(), int(bg_pool.dtype == torch.uint8), P, Hb, Wb, bg_idx.data_ptr(),
+            top.data_ptr(), left.data_ptr(), apply.data_ptr(), fg_lut.data_ptr(), _host3(bg_mean, "bg_mean"),
+            _host3(bg_std, "bg_std"), float(alpha), _cabi.OUT_LAYOUTS[layout], _OUT_DTYPES[out_dt], out.data_ptr(),
+            _stream_ptr(dev)))
     return out
 
 
 @bgmix_blend.register_fake
-def _(fg, bg_pool, bg_idx, top, left, apply, fg_lut, bg_mean, bg_std, alpha, layout):
+def _(fg, bg_pool, bg_idx, top, left, apply, fg_lut, bg_mean, bg_std, alpha, layout, out_dtype=None):
     B, T, H, W, _ = fg.shape
-    shape = (B, T, 3, H, W) if layout == "NTCHW" else (B, 3, T, H, W)
-    return fg.new_empty(shape, dtype=torch.float32)
+    return fg.new_empty(_out_shape(B, T, H, W, layout), dtype=_out_spec("bgmix_blend", layout, out_dtype))
 
 
 # --------------------------------------------------------------------------- #
@@ -285,9 +301,10 @@ def _check_ragged(name, B, dev, pool_bytes, slots, tables, bg_idx, top, left, ap
 @torch.library.custom_op("bgdebias::bgmix_blend_ragged", mutates_args=(), device_types="cuda")
 def bgmix_blend_ragged(fg: torch.Tensor, pool_bytes: torch.Tensor, slots: torch.Tensor, tables: torch.Tensor,
                        bg_idx: torch.Tensor, top: torch.Tensor, left: torch.Tensor, apply: torch.Tensor,
-                       fg_lut: torch.Tensor, bg_mean: torch.Tensor, bg_std: torch.Tensor, alpha: float, layout: str) -> torch.Tensor:
+                       fg_lut: torch.Tensor, bg_mean: torch.Tensor, bg_std: torch.Tensor, alpha: float, layout: str,
+                       out_dtype: Optional[torch.dtype] = None) -> torch.Tensor:
     _require(fg.dtype == torch.uint8 and fg.dim() == 5 and fg.shape[-1] == 3, "bgmix_blend_ragged: fg must be uint8 [B, T, H, W, 3]")
-    _require(layout in _cabi.LAYOUTS, f"bgmix_blend_ragged: layout must be one of {sorted(_cabi.LAYOUTS)}")
+    out_dt = _out_spec("bgmix_blend_ragged", layout, out_dtype)
     B, T, H, W, _ = fg.shape
     dev = fg.device
     _check_ragged("bgmix_blend_ragged", B, dev, pool_bytes, slots, tables, bg_idx, top, left, apply)
@@ -295,19 +312,19 @@ def bgmix_blend_ragged(fg: torch.Tensor, pool_bytes: torch.Tensor, slots: torch.
              "bgmix_blend_ragged: fg_lut must be float32 [3, 256] on the device")
     fg = fg.contiguous()
     bg_idx, top, left, apply, fg_lut, pool_bytes, slots, tables = (x.contiguous() for x in (bg_idx, top, left, apply, fg_lut, pool_bytes, slots, tables))
-    out = torch.empty((B, T, 3, H, W) if layout == "NTCHW" else (B, 3, T, H, W), dtype=torch.float32, device=dev)
+    out = torch.empty(_out_shape(B, T, H, W, layout), dtype=out_dt, device=dev)
     with torch.cuda.device(dev):
-        _cabi.check(_cabi.lib().bgd_bgmix_blend_ragged_f32(
+        _cabi.check(_cabi.lib().bgd_bgmix_blend_ragged_out(
             fg.data_ptr(), B, T, H, W, pool_bytes.data_ptr(), slots.data_ptr(), slots.numel() // 40, tables.data_ptr(),
             bg_idx.data_ptr(), top.data_ptr(), left.data_ptr(), apply.data_ptr(), fg_lut.data_ptr(), _host3(bg_mean, "bg_mean"),
-            _host3(bg_std, "bg_std"), float(alpha), _cabi.LAYOUTS[layout], out.data_ptr(), _stream_ptr(dev)))
+            _host3(bg_std, "bg_std"), float(alpha), _cabi.OUT_LAYOUTS[layout], _OUT_DTYPES[out_dt], out.data_ptr(), _stream_ptr(dev)))
     return out
 
 
 @bgmix_blend_ragged.register_fake
-def _(fg, pool_bytes, slots, tables, bg_idx, top, left, apply, fg_lut, bg_mean, bg_std, alpha, layout):
+def _(fg, pool_bytes, slots, tables, bg_idx, top, left, apply, fg_lut, bg_mean, bg_std, alpha, layout, out_dtype=None):
     B, T, H, W, _ = fg.shape
-    return fg.new_empty((B, T, 3, H, W) if layout == "NTCHW" else (B, 3, T, H, W), dtype=torch.float32)
+    return fg.new_empty(_out_shape(B, T, H, W, layout), dtype=_out_spec("bgmix_blend_ragged", layout, out_dtype))
 
 
 @torch.library.custom_op("bgdebias::bgmix_blend_ragged_normfg", mutates_args=(), device_types="cuda")
@@ -390,13 +407,14 @@ def _(src, geom, T, H, W):
 @torch.library.custom_op("bgdebias::bgmix_resize_blend", mutates_args=(), device_types="cuda")
 def bgmix_resize_blend(src: torch.Tensor, geom: torch.Tensor, T: int, H: int, W: int, bg_pool: torch.Tensor,
                        bg_idx: torch.Tensor, top: torch.Tensor, left: torch.Tensor, apply: torch.Tensor, fg_lut: torch.Tensor,
-                       bg_mean: torch.Tensor, bg_std: torch.Tensor, alpha: float, layout: str) -> torch.Tensor:
+                       bg_mean: torch.Tensor, bg_std: torch.Tensor, alpha: float, layout: str,
+                       out_dtype: Optional[torch.dtype] = None) -> torch.Tensor:
     """``bgmix_blend(resize_bilinear(src, geom, T, H, W), ...)`` in one launch (the resized uint8 batch never exists)."""
     src, g, gptr = _check_packed("bgmix_resize_blend", src, geom)
     B = g.shape[0]
     _require(bg_pool.dim() == 4 and bg_pool.shape[1] == 3 and bg_pool.dtype in (torch.float32, torch.uint8),
              "bgmix_resize_blend: bg_pool must be float32 or uint8 [P, 3, Hb, Wb]")
-    _require(layout in _cabi.LAYOUTS, f"bgmix_resize_blend: layout must be one of {sorted(_cabi.LAYOUTS)}")
+    out_dt = _out_spec("bgmix_resize_blend", layout, out_dtype)
     P, _, Hb, Wb = bg_pool.shape
     dev = src.device
     for name, t, dt in (("bg_idx", bg_idx, torch.int32), ("top", top, torch.int32), ("left", left, torch.int32),
@@ -408,20 +426,19 @@ def bgmix_resize_blend(src: torch.Tensor, geom: torch.Tensor, T: int, H: int, W:
     _require(bg_pool.device == dev, "bgmix_resize_blend: bg_pool must be on the same device as src")
     bg_pool = bg_pool.contiguous()
     bg_idx, top, left, apply, fg_lut = (x.contiguous() for x in (bg_idx, top, left, apply, fg_lut))
-    shape = (B, T, 3, H, W) if layout == "NTCHW" else (B, 3, T, H, W)
-    out = torch.empty(shape, dtype=torch.float32, device=dev)
+    out = torch.empty(_out_shape(B, T, H, W, layout), dtype=out_dt, device=dev)
     with torch.cuda.device(dev):
-        _cabi.check(_cabi.lib().bgd_bgmix_resize_blend_f32(
+        _cabi.check(_cabi.lib().bgd_bgmix_resize_blend_out(
             src.data_ptr(), src.numel(), gptr, B, T, H, W, bg_pool.data_ptr(), int(bg_pool.dtype == torch.uint8), P, Hb, Wb,
             bg_idx.data_ptr(), top.data_ptr(), left.data_ptr(), apply.data_ptr(), fg_lut.data_ptr(), _host3(bg_mean, "bg_mean"),
-            _host3(bg_std, "bg_std"), float(alpha), _cabi.LAYOUTS[layout], out.data_ptr(), _stream_ptr(dev)))
+            _host3(bg_std, "bg_std"), float(alpha), _cabi.OUT_LAYOUTS[layout], _OUT_DTYPES[out_dt], out.data_ptr(), _stream_ptr(dev)))
     return out
 
 
 @bgmix_resize_blend.register_fake
-def _(src, geom, T, H, W, bg_pool, bg_idx, top, left, apply, fg_lut, bg_mean, bg_std, alpha, layout):
+def _(src, geom, T, H, W, bg_pool, bg_idx, top, left, apply, fg_lut, bg_mean, bg_std, alpha, layout, out_dtype=None):
     B = geom.shape[0]
-    return src.new_empty((B, T, 3, H, W) if layout == "NTCHW" else (B, 3, T, H, W), dtype=torch.float32)
+    return src.new_empty(_out_shape(B, T, H, W, layout), dtype=_out_spec("bgmix_resize_blend", layout, out_dtype))
 
 
 # --------------------------------------------------------------------------- #

@@ -39,9 +39,21 @@ typedef enum bgd_status {
 
 /* Output layouts of the blend.  NTCHW is what the reference's DataLoader hands the model:
  * per-sample FormatShape('NCHW') gives [T,3,H,W] and default_collate stacks to [B,T,3,H,W]
- * (libs/cil/cil.py:203-210).  NCTHW is the permuted variant BASELINE.json mentions. */
+ * (libs/cil/cil.py:203-210).  NCTHW is the permuted variant BASELINE.json mentions.  NTHWC ([B][T][H][W][3], the
+ * *_out entry points only) is channels-last storage of both: its permute(0,1,4,2,3) is the logical [B,T,3,H,W] batch,
+ * whose flatten(0, 1) is torch.channels_last-contiguous, and its permute(0,4,1,2,3) is [B,3,T,H,W] in
+ * torch.channels_last_3d strides. */
 #define BGD_LAYOUT_NTCHW 0
 #define BGD_LAYOUT_NCTHW 1
+#define BGD_LAYOUT_NTHWC 2
+
+/* Output element types of the *_out blend entry points.  The blend is computed in fp32 as in the *_f32 entry points; a
+ * 16-bit output is that value rounded once to nearest even (__float2bfloat16_rn / __float2half_rn), which equals torch's
+ * .to(torch.bfloat16) / .to(torch.float16) of the fp32 result bit for bit.  Normalised values lie in about [-2.2, 2.7],
+ * far inside the fp16 range. */
+#define BGD_OUT_F32  0
+#define BGD_OUT_BF16 1
+#define BGD_OUT_F16  2
 
 /* Median kernel variants (for differential testing; AUTO is the product path). */
 #define BGD_MEDIAN_AUTO      0
@@ -166,6 +178,19 @@ int bgd_bgmix_blend_u8pool_f32(const uint8_t *d_fg, int64_t B, int64_t T, int64_
                                const float *h_bg_mean, const float *h_bg_std, double alpha,
                                int layout, float *d_out, void *stream);
 
+/* bgd_bgmix_blend_f32 / bgd_bgmix_blend_u8pool_f32 with a choice of output: replaces the same reference code
+ * (libs/loader/comix_loader.py:138-145 with :72-75, and config ..._bgmix_plus_randAug.py:137-138) and hands the model
+ * the tensor it consumes.  d_bg_pool is fp32 (pool_is_u8 == 0) or uint8 (pool_is_u8 != 0) [P][3][Hb][Wb];
+ *   layout     BGD_LAYOUT_NTCHW, BGD_LAYOUT_NCTHW or BGD_LAYOUT_NTHWC ([B][T][H][W][3])
+ *   out_dtype  BGD_OUT_F32, BGD_OUT_BF16 or BGD_OUT_F16: element type of d_out
+ * Every other argument and the arithmetic as bgd_bgmix_blend_f32. */
+int bgd_bgmix_blend_out(const uint8_t *d_fg, int64_t B, int64_t T, int64_t H, int64_t W,
+                        const void *d_bg_pool, int pool_is_u8, int64_t P, int64_t Hb, int64_t Wb,
+                        const int32_t *d_bg_idx, const int32_t *d_top, const int32_t *d_left,
+                        const uint8_t *d_apply, const float *d_fg_lut, const float *h_bg_mean,
+                        const float *h_bg_std, double alpha, int layout, int out_dtype, void *d_out,
+                        void *stream);
+
 /* Foreground already normalised: d_fg_norm fp32 [B][T][3][H][W] is the `imgs` tensor the reference's
  * pipeline hands to _mix_background (libs/loader/comix_loader.py:142); no table is involved.
  * out = fg * f32(1 - alpha) + bg_norm * f32(alpha) where apply != 0, a copy elsewhere.
@@ -227,6 +252,16 @@ int bgd_bgmix_blend_ragged_f32(const uint8_t *d_fg, int64_t B, int64_t T, int64_
                                const int32_t *d_left, const uint8_t *d_apply, const float *d_fg_lut,
                                const float *h_bg_mean, const float *h_bg_std, double alpha, int layout,
                                float *d_out, void *stream);
+
+/* bgd_bgmix_blend_ragged_f32 with a choice of output (replaces libs/loader/comix_loader.py:72-75, :126-136 and :138-145
+ * as that entry point does): layout and out_dtype as bgd_bgmix_blend_out, every other argument as
+ * bgd_bgmix_blend_ragged_f32. */
+int bgd_bgmix_blend_ragged_out(const uint8_t *d_fg, int64_t B, int64_t T, int64_t H, int64_t W,
+                               const uint8_t *d_pool, const bgd_ragged_slot *d_slots, int64_t P,
+                               const int32_t *d_tables, const int32_t *d_bg_idx, const int32_t *d_top,
+                               const int32_t *d_left, const uint8_t *d_apply, const float *d_fg_lut,
+                               const float *h_bg_mean, const float *h_bg_std, double alpha, int layout,
+                               int out_dtype, void *d_out, void *stream);
 
 /* Same for a foreground that is already normalised (fp32 [B][T][3][H][W], as bgd_bgmix_blend_normfg_f32). */
 int bgd_bgmix_blend_ragged_normfg_f32(const float *d_fg_norm, int64_t B, int64_t T, int64_t H, int64_t W,
@@ -291,6 +326,16 @@ int bgd_bgmix_resize_blend_f32(const uint8_t *d_src, int64_t src_bytes, const in
                                const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply,
                                const float *d_fg_lut, const float *h_bg_mean, const float *h_bg_std,
                                double alpha, int layout, float *d_out, void *stream);
+
+/* bgd_bgmix_resize_blend_f32 with a choice of output (replaces config ..._bgmix_plus_randAug.py:136-138 and
+ * libs/loader/comix_loader.py:138-145 as that entry point does): layout and out_dtype as bgd_bgmix_blend_out, every
+ * other argument as bgd_bgmix_resize_blend_f32. */
+int bgd_bgmix_resize_blend_out(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t B,
+                               int64_t T, int64_t H, int64_t W, const void *d_bg_pool, int pool_is_u8,
+                               int64_t P, int64_t Hb, int64_t Wb, const int32_t *d_bg_idx,
+                               const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply,
+                               const float *d_fg_lut, const float *h_bg_mean, const float *h_bg_std,
+                               double alpha, int layout, int out_dtype, void *d_out, void *stream);
 
 /* Host-buffer form of bgd_bgmix_resize_blend_f32, as bgd_bgmix_blend_f32_host is for the blend: the packed crops
  * (h_src, pinned or pageable) and the per-sample draws live in host memory -- what a DataLoader collate hands over when
