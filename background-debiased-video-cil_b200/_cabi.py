@@ -90,6 +90,7 @@ SIGNATURES = {
                                               _vp, _c.c_int, _c.c_int64, _c.c_int64, _c.c_int64,
                                               _vp, _vp, _vp, _vp, _vp, _f32p, _f32p, _c.c_double, _c.c_int, _c.c_int, _vp,
                                               _vp]),
+    "bgd_ragged_pack_u8": (_c.c_int, [_vp, _c.c_int64, _i64p, _c.c_int64, _vp, _c.c_int64, _vp]),
 }
 
 _lib = None

@@ -22,7 +22,7 @@ EXTRA_DEFINES = [d for d in os.environ.get("BGD_BUILD_DEFINES", "").split() if d
 SOURCES = ["api.cu", "median_swar.cu", "median_bitsliced.cu", "median_tma_planner.cu", "median_colplane_c1.cu",
            "median_colplane_c2.cu", "median_colplane_c4.cu", "median_ldsm_q0.cu", "median_ldsm_q1.cu",
            "median_ldsm_q2.cu", "median_ldsm_q3.cu", "median_ldsm_q4.cu", "median_ldsm_q5.cu", "bgmix.cu", "raggedmix.cu", "nanreduce.cu", "cutmix.cu", "resize.cu",
-           "resized_crop.cu"]
+           "resized_crop.cu", "shardpack.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -39,7 +39,7 @@ import numpy as np
 import torch
 
 from . import ops
-from .pool import AATables, BackgroundPool, BackgroundStore, RaggedPool, resize_like_reference, resized_hw
+from .pool import AATables, BackgroundPool, BackgroundStore, RaggedPool, ShardedPool, resize_like_reference, resized_hw
 
 try:  # mmaction is optional: register into its registries when it is importable
     from mmaction.datasets import RawframeDataset as _MMRawframeDataset
@@ -203,6 +203,9 @@ class BackgroundMixDataset(_Base):
         self._pool: Optional[BackgroundPool] = None
         self._pool_key = None
         self._store: Optional[BackgroundStore] = None
+        self._sharded: Optional[ShardedPool] = None
+        self._shard_of: dict = {}                         # name (and its realpath) -> global index of the sharded pool
+        self._shard_rows_key, self._shard_rows = None, None
         self._resized_cache = {}
 
         # pool assembly: the three modes of comix_loader.py:84-103
@@ -265,7 +268,46 @@ class BackgroundMixDataset(_Base):
         store = BackgroundStore(self.bg_resize, ragged.device)
         store.adopt([osp.realpath(p) for p in paths], ragged)
         self._store, self._pool, self._pool_key = store, None, None
+        self._sharded = None
         self.device = ragged.device
+
+    def attach_sharded_pool(self, paths: Sequence[str], sharded: ShardedPool) -> None:
+        """Mix from a pool sharded across the ranks of a process group (``pool.shard_extracted_backgrounds``): ``paths[i]`` names
+        global image ``i`` of ``sharded``.  Each rank keeps only its own images; :meth:`device_finish` fetches the images a
+        batch drew from their owners (one ``all_to_all_single``) and blends them, bit-equal to :meth:`attach_pool` with the
+        replicated pool.  ``bg_files`` may list any of these names, in any order and with repeats -- the CIL pool operations
+        stay inside the extracted set; a name outside it raises ``ValueError``, nothing is decoded on demand.  Sizes come from
+        the index, so DataLoader workers forked after this call draw crops without reading a file.
+
+        Every rank of the pool's group must call :meth:`device_finish` (or :meth:`mix_batch_on_device`) once per batch, in
+        lockstep: see :meth:`pool.ShardedPool.fetch`."""
+        if len(paths) != len(sharded):
+            raise ValueError("one path per image of the sharded pool")
+        of: dict = {}
+        for i, p in enumerate(paths):
+            of.setdefault(str(p), i)
+            of.setdefault(osp.realpath(p), i)             # bg_files are matched after realpath like bg_dir (:61-68)
+        self._sharded, self._shard_of = sharded, of
+        self._shard_rows_key, self._shard_rows = None, None
+        self._store, self._pool, self._pool_key = None, None, None
+        self.device = sharded.device
+
+    def _shard_index(self, path: str) -> int:
+        i = self._shard_of.get(path)
+        if i is None:
+            i = self._shard_of.get(osp.realpath(path))
+        if i is None:
+            raise ValueError(f"background {path!r} of bg_files is not in the sharded pool's index; a sharded pool mixes "
+                             "only the extracted backgrounds it was built from")
+        return i
+
+    def _sharded_rows(self) -> np.ndarray:
+        """Global index of every entry of the current ``bg_files`` (cached per list)."""
+        key = tuple(self.bg_files)
+        if self._shard_rows is None or key != self._shard_rows_key:
+            self._shard_rows = np.array([self._shard_index(p) for p in self.bg_files], dtype=np.int64)
+            self._shard_rows_key = key
+        return self._shard_rows
 
     # ---- per-sample API (reference contract) ---------------------------------------------------
     def prepare_train_frames(self, idx):
@@ -339,7 +381,9 @@ class BackgroundMixDataset(_Base):
     def _bg_hw(self, bg_idx: int) -> tuple:
         """Size after Resize of ``bg_files[bg_idx]``: from the resident pool / store when they know the file; else a
         process that owns the GPU decodes the image into the store (once), and a forked DataLoader worker reads the image
-        header (cached per path)."""
+        header (cached per path).  With a sharded pool the global index answers."""
+        if self._sharded is not None:
+            return self._sharded.hw(self._shard_index(self.bg_files[bg_idx]))
         if self._pool is not None and tuple(self.bg_files) == self._pool_key:
             return self._pool.hw_of(bg_idx)
         path = self.bg_files[bg_idx]
@@ -379,7 +423,8 @@ class BackgroundMixDataset(_Base):
         as in every shipped config).
 
         The background of sample b is pool image ``bg_idx[b]`` -- from the dense fp32 cache when the pool has one
-        image size and fits, else from the ragged uint8 store with ``Resize`` inside the launch -- or, in random-frame
+        image size and fits, else from the ragged uint8 store with ``Resize`` inside the launch; with a sharded pool
+        (:meth:`attach_sharded_pool`) from the images fetched from their owners, a collective -- or, in random-frame
         mode (``back_ground_from_bg_dir=False``), ``bg_imgs[bg_slot[b]]``: the uint8 frames the batch drew.
 
         Clips whose size is not ``bg_crop_size`` -- a pipeline that stops before the final
@@ -410,6 +455,14 @@ class BackgroundMixDataset(_Base):
             batch_pool = RaggedPool(self.bg_resize, dev, tables=self._aa_tables())
             batch_pool.append(bg_imgs)
             ragged, dense, rows = batch_pool, None, as_dev(bg_slot, torch.int32)
+        elif self._sharded is not None:
+            # sharded pool: fetch the drawn images from their owners (a collective), then the random-frame route
+            idx = torch.as_tensor(bg_idx).cpu().clamp(min=0, max=max(len(self.bg_files) - 1, 0))
+            gidx = torch.from_numpy(self._sharded_rows())[idx] if len(self.bg_files) else idx
+            batch_pool, slot = self._sharded.fetch(gidx, torch.as_tensor(bg_apply).cpu())
+            if not len(batch_pool):                       # nothing mixed on this rank: a placeholder the blend never reads
+                batch_pool.append([torch.zeros((3, th, tw), dtype=torch.uint8)])
+            ragged, dense, rows = batch_pool, None, as_dev(slot, torch.int32)
         else:
             pool = self.device_pool()
             ragged, dense = pool.ragged, pool.tensor

@@ -786,4 +786,12 @@ int bgd_bgmix_resize_blend_f32_host(const uint8_t *h_src, int64_t src_bytes, con
     return BGD_OK;
 }
 
+int bgd_ragged_pack_u8(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_segments, int64_t n, uint8_t *d_out,
+                       int64_t out_bytes, void *stream)
+{
+    DeviceProps dp;
+    if (int rc = current_device_props(&dp)) return rc;
+    return launch_ragged_pack(d_src, src_bytes, h_segments, n, d_out, out_bytes, static_cast<cudaStream_t>(stream));
+}
+
 }  // extern "C"

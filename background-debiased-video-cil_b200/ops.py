@@ -25,6 +25,9 @@ built library (``ImportError`` otherwise).  Ops are stream-ordered and never syn
     bgdebias::bgmix_resize_blend(Tensor src, Tensor geom, int T, int H, int W, <bgmix_blend arguments>) -> Tensor
         the pipeline's Resize((W, H), keep_ratio=False) (config ..._bgmix_plus_randAug.py:136; cv2 INTER_LINEAR, bit-exact)
         on packed uint8 crops, alone or fused with the blend.
+    bgdebias::ragged_pack(Tensor pool_bytes, Tensor segments, int out_bytes) -> Tensor
+        one launch that gathers whole images of a ragged uint8 pool into one buffer (segments int64 [n, 3] = {source
+        offset, destination offset, bytes}, 16-byte aligned): the owner side of pool.ShardedPool.fetch.
     bgdebias::resized_crop_aa(Tensor src, Tensor desc, Tensor tables, int out_h, int out_w) -> Tensor
         RandomResizedCrop(100)(read_image(f).float()).permute(1, 2, 0) of many frames of any sizes, for host-made draws
         (cil_tools/extract_background.py:81,89-90; torchvision's antialiased bilinear, bit-exact).
@@ -196,6 +199,33 @@ def resized_crop_aa(src: torch.Tensor, desc: torch.Tensor, tables: torch.Tensor,
 @resized_crop_aa.register_fake
 def _(src, desc, tables, out_h, out_w):
     return src.new_empty((desc.shape[0], out_h, out_w, 3), dtype=torch.float32)
+
+
+# --------------------------------------------------------------------------- #
+# batched ragged gather (owner side of pool.ShardedPool.fetch, replaces comix_loader.py:126-131 per owned image)
+# --------------------------------------------------------------------------- #
+@torch.library.custom_op("bgdebias::ragged_pack", mutates_args=(), device_types="cuda")
+def ragged_pack(pool_bytes: torch.Tensor, segments: torch.Tensor, out_bytes: int) -> torch.Tensor:
+    """uint8 ``[out_bytes]`` whose bytes ``[dst, dst + bytes)`` are ``pool_bytes[src:src + bytes]`` for every row
+    ``{src, dst, bytes}`` of ``segments`` (int64 ``[n, 3]``, host or device; offsets 16-byte aligned).  Bytes outside every
+    segment are left uninitialised."""
+    _require(pool_bytes.dtype == torch.uint8 and pool_bytes.dim() == 1, "ragged_pack: pool_bytes must be a flat uint8 buffer")
+    _require(segments.dim() == 2 and segments.shape[1] == 3 and segments.dtype in (torch.int64, torch.int32),
+             "ragged_pack: segments must be int64 [n, 3]")
+    _require(out_bytes >= 0, "ragged_pack: out_bytes must be >= 0")
+    seg = segments.detach().to("cpu", torch.int64).contiguous()
+    pool_bytes = pool_bytes.contiguous()
+    out = torch.empty(out_bytes, dtype=torch.uint8, device=pool_bytes.device)
+    with torch.cuda.device(pool_bytes.device):
+        _cabi.check(_cabi.lib().bgd_ragged_pack_u8(pool_bytes.data_ptr(), pool_bytes.numel(),
+                                                   ctypes.cast(seg.data_ptr(), ctypes.POINTER(ctypes.c_int64)), seg.shape[0],
+                                                   out.data_ptr(), out_bytes, _stream_ptr(pool_bytes.device)))
+    return out
+
+
+@ragged_pack.register_fake
+def _(pool_bytes, segments, out_bytes):
+    return pool_bytes.new_empty((out_bytes,))
 
 
 # --------------------------------------------------------------------------- #

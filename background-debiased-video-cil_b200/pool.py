@@ -9,7 +9,7 @@ the pool is index ``i`` of ``bg_files`` -- the reference's ``bg_idx``.
 """
 from __future__ import annotations
 
-from typing import Dict, List, Optional, Sequence, Tuple
+from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -398,6 +398,212 @@ def gather_extracted_backgrounds(output_dir, image_suffix: str = ".jpg", bg_resi
     local = RaggedPool(bg_resize, device)
     local.append(_map_in_order(lambda f: read_image(f, mode=ImageReadMode.RGB), mine))
     return all_gather_ragged(mine, local, group)
+
+
+def _pad16(n):
+    return (n + 15) & ~15
+
+
+class ShardRoute(NamedTuple):
+    """What one rank does in one exchange of :meth:`ShardedPool.fetch` (see :func:`route_requests`)."""
+    segments: np.ndarray        # int64 [n, 3] {source offset in the local pool, offset in the send buffer, bytes}
+    send_splits: List[int]      # bytes of the send buffer for each destination rank
+    recv_splits: List[int]      # bytes of the receive buffer from each source rank
+    recv_offsets: np.ndarray    # int64, offset in the receive buffer of each of this rank's requests, in request order
+
+
+def route_requests(requests: Sequence[Sequence[int]], owner: np.ndarray, slot: np.ndarray, nbytes: np.ndarray, rank: int,
+                   local_offsets: np.ndarray) -> ShardRoute:
+    """Routing of one exchange, the same pure function on every rank.  ``requests[r]``: the global pool indices rank r asks for
+    (deduplicated, in its request order); ``owner`` / ``slot`` / ``nbytes``: owning rank, slot on the owner and native size
+    ``3*h*w`` of every global index; ``local_offsets``: byte offset of every slot of THIS rank's pool.
+
+    The send buffer holds, for destination d = 0, 1, ..., the images d requested that this rank owns, in d's request order;
+    so the chunk rank r receives from source s holds r's requests owned by s in r's order, and the receiver computes its
+    offsets without asking the sender.  Every image starts on a 16-byte boundary (its size is padded), so every chunk is a
+    multiple of 16 bytes and every offset of both buffers is 16-byte aligned."""
+    world = len(requests)
+    owner, slot, nbytes = np.asarray(owner), np.asarray(slot), np.asarray(nbytes, dtype=np.int64)
+    segs, send_splits, at = [], [], 0
+    for d in range(world):
+        start = at
+        for g in requests[d]:
+            if owner[g] == rank:
+                b = int(nbytes[g])
+                segs.append((int(local_offsets[slot[g]]), at, b))
+                at += _pad16(b)
+        send_splits.append(at - start)
+    mine = [int(g) for g in requests[rank]]
+    recv_splits = [0] * world
+    for g in mine:
+        recv_splits[int(owner[g])] += _pad16(int(nbytes[g]))
+    chunk_at = np.concatenate([[0], np.cumsum(recv_splits)[:-1]]).astype(np.int64) if world else np.zeros(0, np.int64)
+    fill = list(chunk_at)
+    recv_offsets = np.empty(len(mine), dtype=np.int64)
+    for k, g in enumerate(mine):
+        r = int(owner[g])
+        recv_offsets[k] = fill[r]
+        fill[r] += _pad16(int(nbytes[g]))
+    segments = np.array(segs, dtype=np.int64).reshape(-1, 3)
+    return ShardRoute(segments, send_splits, recv_splits, recv_offsets)
+
+
+class ShardedPool:
+    """A background pool sharded across the ranks of a process group: each rank keeps only the images it owns (a
+    :class:`RaggedPool`, ~1/world of the replica: Sth-Sth-v2 67.9 GB -> ~8.5 GB per GPU on 8), plus the global index that
+    every rank holds identically -- ``names[P]``, ``owner[P]``, ``slot[P]`` and the native ``h[P]``, ``w[P]`` -- and one
+    :class:`AATables` with the resize tables of every size in the index.  Index ``i`` is what
+    ``BackgroundPool.all_gather_index`` calls ``i``: ranks in order, each rank's images in its order.
+
+    :meth:`fetch` brings the images a batch drew to the rank that mixes it, as whole native images, and returns them as a
+    per-batch :class:`RaggedPool` -- the form ``bgmix_blend_ragged`` reads, bit-equal to blending from the replica.
+
+    ``group``: the process group the index was gathered over (``None``: the default group); ``rank`` / ``world`` are this
+    process's rank in it and its size, and :meth:`fetch` runs its collectives on it, so the routing and the exchange can
+    never use different groups."""
+
+    def __init__(self, local: RaggedPool, names: Sequence[str], owner, slot, h, w, rank: int, world: int, group=None):
+        self.local = local
+        self.names: List[str] = list(names)
+        self.owner = np.asarray(owner, dtype=np.int64)
+        self.slot = np.asarray(slot, dtype=np.int64)
+        self.h = np.asarray(h, dtype=np.int64)
+        self.w = np.asarray(w, dtype=np.int64)
+        self.rank, self.world = int(rank), int(world)
+        self.group = group
+        self.bg_resize = local.bg_resize
+        self.device = local.device
+        self.tables = local.tables
+        if not (len(self.names) == len(self.owner) == len(self.slot) == len(self.h) == len(self.w)):
+            raise ValueError("one owner, slot and size per index entry")
+        if int((self.owner == self.rank).sum()) != len(local):
+            raise ValueError("the local pool must hold exactly the images the index assigns to this rank")
+        misaligned = np.flatnonzero(local.slots["offset"] % 16) if len(local) else np.zeros(0, np.int64)
+        if misaligned.size:
+            # ragged_pack reads whole images with 16-byte vectors; RaggedPool.append aligns every image, a pool adopted with
+            # from_uniform_buffer only when 3*h*w is a multiple of 16
+            raise ValueError(f"local image {int(misaligned[0])} starts at byte {int(local.slots['offset'][misaligned[0]])}, "
+                             "not a multiple of 16: a sharded pool needs 16-byte aligned images (build it with "
+                             "RaggedPool.append)")
+        self.nbytes = 3 * self.h * self.w
+        self._hw: Dict[Tuple[int, int], Tuple[int, int]] = {}      # native -> resized size; fills the tables for every size
+        for hw in set(zip(self.h.tolist(), self.w.tolist())):
+            s = local.make_slot(0, *hw)
+            self._hw[hw] = (int(s["Hb"]), int(s["Wb"]))
+
+    def __len__(self) -> int:
+        return len(self.names)
+
+    @classmethod
+    def from_local(cls, names: Sequence[str], ragged: RaggedPool, group=None) -> "ShardedPool":
+        """Collective: one ``all_gather_object`` of ``(name, h, w)`` per local image -- the index of ``all_gather_index``
+        plus the native sizes.  ``names[i]`` is image ``i`` of ``ragged``; no pixel leaves its rank."""
+        import torch.distributed as dist
+        if len(names) != len(ragged):
+            raise ValueError("one name per local background")
+        world, rank = dist.get_world_size(group), dist.get_rank(group)
+        meta = [(str(n), int(s["h"]), int(s["w"])) for n, s in zip(names, ragged.slots)]
+        metas: List[Optional[list]] = [None] * world
+        dist.all_gather_object(metas, meta, group=group)
+        rows = [(n, r, i, hh, ww) for r, per in enumerate(metas) for i, (n, hh, ww) in enumerate(per)]
+        cols = list(zip(*rows)) if rows else [[]] * 5
+        return cls(ragged, cols[0], cols[1], cols[2], cols[3], cols[4], rank, world, group)
+
+    def index(self) -> list:
+        """``[(name, owner_rank, slot_on_owner), ...]``: what ``BackgroundPool.all_gather_index`` returns."""
+        return [(n, int(r), int(i)) for n, r, i in zip(self.names, self.owner, self.slot)]
+
+    def hw(self, i: int) -> Tuple[int, int]:
+        """Size after Resize of global image ``i`` -- what RandomCrop draws its offsets from."""
+        return self._hw[(int(self.h[i]), int(self.w[i]))]
+
+    @property
+    def resident_bytes(self) -> int:
+        """Bytes of the local pool buffer on this rank's device."""
+        return int(self.local.data.numel()) if self.local.data is not None else 0
+
+    @staticmethod
+    def requests_of(bg_idx, apply) -> List[int]:
+        """The global indices a batch asks for: those of the applied samples, deduplicated, in sample order."""
+        idx = torch.as_tensor(bg_idx).tolist()
+        app = torch.as_tensor(apply).tolist()
+        return list(dict.fromkeys(int(g) for g, a in zip(idx, app) if a))
+
+    def route(self, requests: Sequence[Sequence[int]]) -> ShardRoute:
+        """:func:`route_requests` for this rank."""
+        for r, req in enumerate(requests):
+            bad = [g for g in req if not 0 <= g < len(self)]
+            if bad:
+                raise ValueError(f"rank {r} requests background {bad[0]}, outside the {len(self)}-image index")
+        return route_requests(requests, self.owner, self.slot, self.nbytes, self.rank, self.local.slots["offset"])
+
+    def pack(self, route: ShardRoute) -> torch.Tensor:
+        """The send buffer of ``route``: one ``ragged_pack`` launch over the local pool."""
+        total = int(sum(route.send_splits))
+        src = self.local.data if self.local.data is not None else torch.empty(0, dtype=torch.uint8, device=self.device)
+        return torch.ops.bgdebias.ragged_pack(src, torch.from_numpy(route.segments), total)
+
+    def assemble(self, recv: torch.Tensor, requests: Sequence[int], route: ShardRoute) -> RaggedPool:
+        """The per-batch pool over the receive buffer: image ``k`` is ``requests[k]`` (this rank's requests)."""
+        batch = RaggedPool(self.bg_resize, self.device, tables=self.tables)
+        batch.data, batch.used = recv, int(recv.numel())
+        slots = [self.local.make_slot(int(o), int(self.h[g]), int(self.w[g])) for o, g in zip(route.recv_offsets, requests)]
+        batch.slots = np.array(slots, dtype=SLOT_DTYPE) if slots else np.zeros(0, dtype=SLOT_DTYPE)
+        return batch
+
+    def fetch(self, bg_idx, apply) -> Tuple[RaggedPool, torch.Tensor]:
+        """Collective.  ``bg_idx`` / ``apply`` ([B], host or device): the global pool index and the mix flag of every sample
+        of this rank's batch.  Returns ``(batch pool, slot)``: a :class:`RaggedPool` holding the drawn images and the int32
+        ``[B]`` slot of each sample in it (0 for a sample that is not mixed; the blend ignores it).
+
+        EVERY rank of the pool's group must call ``fetch`` once per batch, in the same order -- also at world size 1 and
+        for a batch that mixes nothing -- because the call is two collectives on that group: an ``all_gather_object`` of
+        every rank's requests (after which every rank knows the whole request matrix and computes its send segments, its
+        receive splits and the receive offsets with :func:`route_requests`, no further exchange), then one ``ragged_pack``
+        launch and one ``all_to_all_single`` of bytes on the current stream.  The self-chunk carries the rank's own images,
+        so local and remote images take the same path.  A DDP training step, which mixes one batch per rank per step, meets
+        this.
+
+        The host waits here: the split sizes of ``all_to_all_single`` must be known on the host, and on an NCCL group
+        ``all_gather_object`` reads the gathered sizes back from the device, so the call returns only after the work already
+        queued on the current stream (e.g. the previous step's backward) has finished.  The replicated pool never waits."""
+        import torch.distributed as dist
+        mine = self.requests_of(bg_idx, apply)
+        requests: List[Optional[list]] = [None] * self.world
+        dist.all_gather_object(requests, mine, group=self.group)
+        route = self.route(requests)
+        recv = torch.empty(int(sum(route.recv_splits)), dtype=torch.uint8, device=self.device)
+        if any(requests):                                  # every rank sees the same matrix: all skip or none does
+            send = self.pack(route)
+            dist.all_to_all_single(recv, send, route.recv_splits, route.send_splits, group=self.group)
+        return self.assemble(recv, mine, route), self.sample_slots(bg_idx, apply, mine)
+
+    @staticmethod
+    def sample_slots(bg_idx, apply, requests: Sequence[int]) -> torch.Tensor:
+        """int32 ``[B]``: the image of the batch pool each sample blends (0 for a sample that is not mixed)."""
+        where = {g: k for k, g in enumerate(requests)}
+        app = torch.as_tensor(apply).tolist()
+        return torch.tensor([where[int(g)] if a else 0 for g, a in zip(torch.as_tensor(bg_idx).tolist(), app)],
+                            dtype=torch.int32)
+
+
+def shard_extracted_backgrounds(output_dir, image_suffix: str = ".jpg", bg_resize: Optional[int] = 256, device="cuda",
+                                group=None):
+    """The sharded twin of :func:`gather_extracted_backgrounds`: the same contiguous split of the sorted JPEGs, each rank
+    decodes its own files with ``torchvision.io.read_image(mode=RGB)`` and KEEPS them; only names and sizes are all-gathered.
+    Returns ``(paths, ShardedPool)`` with ``paths[i]`` the file of global index ``i`` (the same list, in the same order, as
+    :func:`gather_extracted_backgrounds` returns)."""
+    import pathlib
+    import torch.distributed as dist
+    from torchvision.io import ImageReadMode, read_image
+    from .shard import contiguous_splits
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    files = sorted(str(f) for f in pathlib.Path(output_dir).glob("*" + image_suffix))
+    mine = contiguous_splits(files, world)[rank] if files else []
+    local = RaggedPool(bg_resize, device)
+    local.append(_map_in_order(lambda f: read_image(f, mode=ImageReadMode.RGB), mine))
+    sharded = ShardedPool.from_local(mine, local, group)
+    return list(sharded.names), sharded
 
 
 class BackgroundStore:

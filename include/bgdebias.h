@@ -349,6 +349,20 @@ int bgd_bgmix_resize_blend_f32_host(const uint8_t *h_src, int64_t src_bytes, con
                                     const float *h_bg_mean, const float *h_bg_std, double alpha, int layout,
                                     float *d_out, double *h_checksum, int device);
 
+/* ---- batched ragged gather (owner side of the sharded background pool's exchange) --------------------
+ * Replaces, for the images of a batch that one rank owns, the per-sample background read of the reference
+ *   libs/loader/comix_loader.py:126-131   bg_idx = torch.randint(len(self.bg_files)); read_image(self.bg_files[bg_idx])
+ * when the pool is sharded across ranks: the owner copies every requested native image into one send buffer in one launch,
+ * and a single all_to_all_single delivers it (bgdebias_b200.pool.ShardedPool.fetch).
+ *
+ *   d_src        the owner's pool bytes (a RaggedPool buffer), 16-byte aligned
+ *   h_segments   HOST int64 [n][3]: {source byte offset, destination byte offset, bytes}; both offsets 16-byte aligned, every
+ *                segment inside d_src[0, src_bytes) and d_out[0, out_bytes); validated, then copied to the device on `stream`
+ *   d_out        destination buffer, 16-byte aligned; bytes outside every segment are left untouched
+ * n <= 65535; n == 0 (or only empty segments) launches nothing. */
+int bgd_ragged_pack_u8(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_segments, int64_t n, uint8_t *d_out,
+                       int64_t out_bytes, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
