@@ -39,7 +39,8 @@ import numpy as np
 import torch
 
 from . import ops
-from .pool import AATables, BackgroundPool, BackgroundStore, RaggedPool, ShardedPool, resize_like_reference, resized_hw
+from .pool import (AATables, BackgroundPool, BackgroundStore, PeerPool, RaggedPool, ShardedPool, resize_like_reference,
+                   resized_hw)
 
 try:  # mmaction is optional: register into its registries when it is importable
     from mmaction.datasets import RawframeDataset as _MMRawframeDataset
@@ -204,6 +205,7 @@ class BackgroundMixDataset(_Base):
         self._pool_key = None
         self._store: Optional[BackgroundStore] = None
         self._sharded: Optional[ShardedPool] = None
+        self._peer: Optional[PeerPool] = None             # set with _sharded: gather from peer mappings instead of fetch
         self._shard_of: dict = {}                         # name (and its realpath) -> global index of the sharded pool
         self._shard_rows_key, self._shard_rows = None, None
         self._resized_cache = {}
@@ -268,7 +270,7 @@ class BackgroundMixDataset(_Base):
         store = BackgroundStore(self.bg_resize, ragged.device)
         store.adopt([osp.realpath(p) for p in paths], ragged)
         self._store, self._pool, self._pool_key = store, None, None
-        self._sharded = None
+        self._sharded, self._peer = None, None
         self.device = ragged.device
 
     def attach_sharded_pool(self, paths: Sequence[str], sharded: ShardedPool) -> None:
@@ -287,10 +289,19 @@ class BackgroundMixDataset(_Base):
         for i, p in enumerate(paths):
             of.setdefault(str(p), i)
             of.setdefault(osp.realpath(p), i)             # bg_files are matched after realpath like bg_dir (:61-68)
-        self._sharded, self._shard_of = sharded, of
+        self._sharded, self._shard_of, self._peer = sharded, of, None
         self._shard_rows_key, self._shard_rows = None, None
         self._store, self._pool, self._pool_key = None, None, None
         self.device = sharded.device
+
+    def attach_peer_pool(self, paths: Sequence[str], peer: PeerPool) -> None:
+        """The twin of :meth:`attach_sharded_pool` for a pool whose shards are mapped into every rank of one node
+        (``pool.PeerPool.open``): the same names, the same ``ValueError`` for a name outside the index, the same draws and
+        bits; but :meth:`device_finish` reads the images a batch drew straight from their owners' memory with one local
+        launch (:meth:`pool.PeerPool.gather`) -- no collective, so ranks need not call it in lockstep, and the host does
+        not wait for the device.  Attaching a pool of any other kind detaches this one."""
+        self.attach_sharded_pool(paths, peer.sharded)
+        self._peer = peer
 
     def _shard_index(self, path: str) -> int:
         i = self._shard_of.get(path)
@@ -424,7 +435,8 @@ class BackgroundMixDataset(_Base):
 
         The background of sample b is pool image ``bg_idx[b]`` -- from the dense fp32 cache when the pool has one
         image size and fits, else from the ragged uint8 store with ``Resize`` inside the launch; with a sharded pool
-        (:meth:`attach_sharded_pool`) from the images fetched from their owners, a collective -- or, in random-frame
+        (:meth:`attach_sharded_pool`) from the images fetched from their owners, a collective, or read from their owners'
+        peer-mapped memory (:meth:`attach_peer_pool`), a local launch -- or, in random-frame
         mode (``back_ground_from_bg_dir=False``), ``bg_imgs[bg_slot[b]]``: the uint8 frames the batch drew.
 
         Clips whose size is not ``bg_crop_size`` -- a pipeline that stops before the final
@@ -456,10 +468,12 @@ class BackgroundMixDataset(_Base):
             batch_pool.append(bg_imgs)
             ragged, dense, rows = batch_pool, None, as_dev(bg_slot, torch.int32)
         elif self._sharded is not None:
-            # sharded pool: fetch the drawn images from their owners (a collective), then the random-frame route
+            # sharded pool: fetch the drawn images from their owners (a collective) or gather them from the peer mappings
+            # (a local launch), then the random-frame route
             idx = torch.as_tensor(bg_idx).cpu().clamp(min=0, max=max(len(self.bg_files) - 1, 0))
             gidx = torch.from_numpy(self._sharded_rows())[idx] if len(self.bg_files) else idx
-            batch_pool, slot = self._sharded.fetch(gidx, torch.as_tensor(bg_apply).cpu())
+            get = self._peer.gather if self._peer is not None else self._sharded.fetch
+            batch_pool, slot = get(gidx, torch.as_tensor(bg_apply).cpu())
             if not len(batch_pool):                       # nothing mixed on this rank: a placeholder the blend never reads
                 batch_pool.append([torch.zeros((3, th, tw), dtype=torch.uint8)])
             ragged, dense, rows = batch_pool, None, as_dev(slot, torch.int32)

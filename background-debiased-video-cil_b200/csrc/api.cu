@@ -7,6 +7,8 @@
 #include <thread>
 #include <vector>
 
+#include <cudaTypedefs.h>
+
 #include "bgd_common.cuh"
 
 namespace bgd {
@@ -792,6 +794,86 @@ int bgd_ragged_pack_u8(const uint8_t *d_src, int64_t src_bytes, const int64_t *h
     DeviceProps dp;
     if (int rc = current_device_props(&dp)) return rc;
     return launch_ragged_pack(d_src, src_bytes, h_segments, n, d_out, out_bytes, static_cast<cudaStream_t>(stream));
+}
+
+int bgd_ragged_gather_u8(const uint8_t *const *d_bases, const int64_t *h_base_bytes, int64_t n_bases, const int64_t *h_segments,
+                         int64_t n, uint8_t *d_out, int64_t out_bytes, void *stream)
+{
+    DeviceProps dp;
+    if (int rc = current_device_props(&dp)) return rc;
+    return launch_ragged_gather(d_bases, h_base_bytes, n_bases, h_segments, n, d_out, out_bytes,
+                                static_cast<cudaStream_t>(stream));
+}
+
+int bgd_ipc_export(const void *d_ptr, uint8_t *handle, int64_t *offset)
+{
+    if (!d_ptr || !handle || !offset) return fail(BGD_ERR_INVALID, "ipc_export: null argument");
+    DeviceProps dp;
+    if (int rc = current_device_props(&dp)) return rc;
+    cudaPointerAttributes attr;
+    BGD_CUDA_TRY(cudaPointerGetAttributes(&attr, d_ptr));
+    int dev = 0;
+    BGD_CUDA_TRY(cudaGetDevice(&dev));
+    if (attr.type != cudaMemoryTypeDevice || attr.device != dev)
+        return fail(BGD_ERR_INVALID, "ipc_export: %p is not device memory of the current device %d", d_ptr, dev);
+    // the allocation that holds d_ptr: torch's caching allocator hands out pieces of larger cudaMalloc segments, and only a
+    // segment's base can be exported.  cuMemGetAddressRange is reached through the runtime, so the library links no libcuda.
+    static const PFN_cuMemGetAddressRange_v3020 get_range = [] {
+        void *fn = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPointByVersion("cuMemGetAddressRange", &fn, 12000, cudaEnableDefault, &q) != cudaSuccess ||
+            q != cudaDriverEntryPointSuccess)
+            fn = nullptr;
+        cudaGetLastError();
+        return reinterpret_cast<PFN_cuMemGetAddressRange_v3020>(fn);
+    }();
+    if (!get_range) return fail(BGD_ERR_UNSUPPORTED, "ipc_export: the driver does not provide cuMemGetAddressRange");
+    CUdeviceptr base = 0;
+    size_t size = 0;
+    if (CUresult r = get_range(&base, &size, reinterpret_cast<CUdeviceptr>(d_ptr)))
+        return fail(BGD_ERR_UNSUPPORTED, "ipc_export: cuMemGetAddressRange failed on %p (CUresult %d)", d_ptr, (int)r);
+    cudaIpcMemHandle_t h;
+    cudaError_t e = cudaIpcGetMemHandle(&h, reinterpret_cast<void *>(base));
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(BGD_ERR_UNSUPPORTED,
+                    "ipc_export: the allocation at %p cannot be exported with cudaIpcGetMemHandle (%s); peer mapping needs "
+                    "memory from cudaMalloc -- torch's native caching allocator without expandable_segments, not the "
+                    "cudaMallocAsync backend",
+                    reinterpret_cast<void *>(base), cudaGetErrorString(e));
+    }
+    static_assert(sizeof(h) == 64, "cudaIpcMemHandle_t is 64 bytes");
+    std::memcpy(handle, &h, sizeof(h));
+    *offset = (int64_t)(reinterpret_cast<CUdeviceptr>(d_ptr) - base);
+    return BGD_OK;
+}
+
+int bgd_ipc_open(const uint8_t *handle, int device, void **d_base)
+{
+    if (!handle || !d_base) return fail(BGD_ERR_INVALID, "ipc_open: null argument");
+    DeviceProps dp;
+    if (int rc = get_device_props(device, &dp)) return rc;
+    int back = 0;
+    BGD_CUDA_TRY(cudaGetDevice(&back));
+    BGD_CUDA_TRY(cudaSetDevice(device));
+    cudaIpcMemHandle_t h;
+    std::memcpy(&h, handle, sizeof(h));
+    void *p = nullptr;
+    cudaError_t e = cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess);
+    cudaSetDevice(back);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(BGD_ERR_UNSUPPORTED, "ipc_open: cudaIpcOpenMemHandle failed on device %d: %s", device, cudaGetErrorString(e));
+    }
+    *d_base = p;
+    return BGD_OK;
+}
+
+int bgd_ipc_close(void *d_base)
+{
+    if (!d_base) return fail(BGD_ERR_INVALID, "ipc_close: null pointer");
+    BGD_CUDA_TRY(cudaIpcCloseMemHandle(d_base));
+    return BGD_OK;
 }
 
 }  // extern "C"

@@ -162,6 +162,8 @@ int launch_cutmix(const uint8_t *d_actor, const uint8_t *d_mask, const uint8_t *
                   unsigned long long *d_mask_sum, cudaStream_t stream);
 int launch_ragged_pack(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_segments, int64_t n, uint8_t *d_out,
                        int64_t out_bytes, cudaStream_t stream);
+int launch_ragged_gather(const uint8_t *const *d_bases, const int64_t *h_base_bytes, int64_t n_bases, const int64_t *h_segments,
+                         int64_t n, uint8_t *d_out, int64_t out_bytes, cudaStream_t stream);
 int launch_nan_reduce_varlen(const float *d_frames, const int64_t *h_offsets, int64_t V, int64_t N, int avg_method,
                              int zero_is_missing, uint8_t *d_out_u8, float *d_out_f32, cudaStream_t stream);
 

@@ -28,6 +28,9 @@ built library (``ImportError`` otherwise).  Ops are stream-ordered and never syn
     bgdebias::ragged_pack(Tensor pool_bytes, Tensor segments, int out_bytes) -> Tensor
         one launch that gathers whole images of a ragged uint8 pool into one buffer (segments int64 [n, 3] = {source
         offset, destination offset, bytes}, 16-byte aligned): the owner side of pool.ShardedPool.fetch.
+    bgdebias::ragged_gather(Tensor bases, Tensor base_bytes, Tensor segments, int out_bytes) -> Tensor
+        the same one-launch gather from many sources (bases: device int64 [W] of base pointers, peer mappings included;
+        segments int64 [n, 4] = {source, source offset, destination offset, bytes}): pool.PeerPool.gather.
     bgdebias::resized_crop_aa(Tensor src, Tensor desc, Tensor tables, int out_h, int out_w) -> Tensor
         RandomResizedCrop(100)(read_image(f).float()).permute(1, 2, 0) of many frames of any sizes, for host-made draws
         (cil_tools/extract_background.py:81,89-90; torchvision's antialiased bilinear, bit-exact).
@@ -226,6 +229,36 @@ def ragged_pack(pool_bytes: torch.Tensor, segments: torch.Tensor, out_bytes: int
 @ragged_pack.register_fake
 def _(pool_bytes, segments, out_bytes):
     return pool_bytes.new_empty((out_bytes,))
+
+
+@torch.library.custom_op("bgdebias::ragged_gather", mutates_args=(), device_types="cuda")
+def ragged_gather(bases: torch.Tensor, base_bytes: torch.Tensor, segments: torch.Tensor, out_bytes: int) -> torch.Tensor:
+    """uint8 ``[out_bytes]`` whose bytes ``[dst, dst + bytes)`` are the bytes ``[src, src + bytes)`` of source ``r`` for every row
+    ``{r, src, dst, bytes}`` of ``segments`` (int64 ``[n, 4]``, host or device; offsets 16-byte aligned).  ``bases``: device
+    int64 ``[W]``, the 16-byte aligned base address of every source (this process's memory or a peer mapping of
+    ``bgd_ipc_open``); ``base_bytes``: int64 ``[W]`` (host), the readable bytes from each base.  Every segment is checked
+    against these sizes before the launch.  Bytes outside every segment are left uninitialised."""
+    _require(bases.dtype == torch.int64 and bases.dim() == 1 and bases.is_cuda, "ragged_gather: bases must be device int64 [W]")
+    _require(base_bytes.dim() == 1 and base_bytes.numel() == bases.numel() and not base_bytes.is_floating_point(),
+             "ragged_gather: base_bytes must be int64 [W], one size per base")
+    _require(segments.dim() == 2 and segments.shape[1] == 4 and segments.dtype in (torch.int64, torch.int32),
+             "ragged_gather: segments must be int64 [n, 4]")
+    _require(out_bytes >= 0, "ragged_gather: out_bytes must be >= 0")
+    seg = segments.detach().to("cpu", torch.int64).contiguous()
+    sizes = base_bytes.detach().to("cpu", torch.int64).contiguous()
+    bases = bases.contiguous()
+    out = torch.empty(out_bytes, dtype=torch.uint8, device=bases.device)
+    i64p = ctypes.POINTER(ctypes.c_int64)
+    with torch.cuda.device(bases.device):
+        _cabi.check(_cabi.lib().bgd_ragged_gather_u8(bases.data_ptr(), ctypes.cast(sizes.data_ptr(), i64p), sizes.numel(),
+                                                     ctypes.cast(seg.data_ptr(), i64p), seg.shape[0], out.data_ptr(), out_bytes,
+                                                     _stream_ptr(bases.device)))
+    return out
+
+
+@ragged_gather.register_fake
+def _(bases, base_bytes, segments, out_bytes):
+    return bases.new_empty((out_bytes,), dtype=torch.uint8)
 
 
 # --------------------------------------------------------------------------- #

@@ -448,6 +448,24 @@ def route_requests(requests: Sequence[Sequence[int]], owner: np.ndarray, slot: n
     return ShardRoute(segments, send_splits, recv_splits, recv_offsets)
 
 
+def peer_segments(requests: Sequence[int], owner: np.ndarray, src_offset: np.ndarray,
+                  nbytes: np.ndarray) -> Tuple[np.ndarray, np.ndarray, int]:
+    """Host side of :meth:`PeerPool.gather`, a pure function.  ``requests``: this rank's global pool indices (deduplicated, in
+    request order, :meth:`ShardedPool.requests_of`); ``owner`` / ``src_offset`` / ``nbytes``: owning rank, byte offset in the
+    owner's pool buffer and native size ``3*h*w`` of every global index.
+
+    Returns ``(segments, dst, total)``: int64 ``[n, 4]`` rows ``{owner, source offset, destination offset, bytes}`` for
+    ``ragged_gather``, the destination offset of every request, and the size of the per-batch buffer.  Image ``k`` of the
+    batch is ``requests[k]``; every image starts on a 16-byte boundary (sizes are padded), as :meth:`RaggedPool.append` lays
+    a pool out."""
+    req = np.asarray(requests, dtype=np.int64).reshape(-1)
+    b = np.asarray(nbytes, dtype=np.int64)[req]
+    padded = (b + 15) & ~15
+    dst = np.concatenate([[0], np.cumsum(padded)[:-1]]).astype(np.int64) if req.size else np.zeros(0, np.int64)
+    segments = np.stack([np.asarray(owner, dtype=np.int64)[req], np.asarray(src_offset, dtype=np.int64)[req], dst, b], 1)
+    return segments.reshape(-1, 4), dst, int(padded.sum())
+
+
 class ShardedPool:
     """A background pool sharded across the ranks of a process group: each rank keeps only the images it owns (a
     :class:`RaggedPool`, ~1/world of the replica: Sth-Sth-v2 67.9 GB -> ~8.5 GB per GPU on 8), plus the global index that
@@ -585,6 +603,174 @@ class ShardedPool:
         app = torch.as_tensor(apply).tolist()
         return torch.tensor([where[int(g)] if a else 0 for g, a in zip(torch.as_tensor(bg_idx).tolist(), app)],
                             dtype=torch.int32)
+
+
+_USE_FETCH = ("mix from this pool with BackgroundMixDataset.attach_sharded_pool (ShardedPool.fetch, an exchange over the "
+              "process group) instead")
+
+
+def check_peer_meta(metas: Sequence[dict]) -> None:
+    """The refusals of :meth:`PeerPool.open` that every rank decides alike from the gathered metadata, a pure function.
+    ``metas[r]``: ``host`` (host id), ``uuid`` (device), ``handle`` (64 bytes, or ``None`` for an empty shard), ``offset``,
+    ``bytes`` and ``error`` (why the shard could not be exported, or ``None``) of rank ``r``.  Raises ``ValueError`` when the
+    ranks do not all run on one host, or when a rank could not export its shard."""
+    for r, m in enumerate(metas):
+        if m["host"] != metas[0]["host"]:
+            raise ValueError(f"ranks 0 and {r} run on different hosts ({metas[0]['host']!r}, {m['host']!r}): a PeerPool maps "
+                             f"GPU memory between the processes of one node; {_USE_FETCH}")
+    for r, m in enumerate(metas):
+        if m["error"] is not None:
+            raise ValueError(f"rank {r} cannot export its shard for peer mapping: {m['error']}; {_USE_FETCH}")
+        if m["handle"] is not None and (len(m["handle"]) != 64 or m["offset"] % 16):
+            raise ValueError(f"rank {r} exported a malformed handle or an unaligned buffer (offset {m['offset']}); {_USE_FETCH}")
+
+
+def _host_id() -> str:
+    """Host name plus the kernel's boot id: two machines that share a host name still differ."""
+    import socket
+    try:
+        with open("/proc/sys/kernel/random/boot_id") as f:
+            boot = f.read().strip()
+    except OSError:
+        boot = ""
+    return f"{socket.gethostname()}/{boot}"
+
+
+class PeerPool:
+    """A :class:`ShardedPool` whose shards are mapped into every rank of one node, so a rank reads the images its batch drew
+    straight from their owners' HBM (over NVLink between GPUs) instead of exchanging them.  Built by :meth:`open`, a
+    collective; after it :meth:`gather` is local: one ``ragged_gather`` launch per batch, no collective, no lockstep between
+    ranks and no host synchronisation.  The result is bit-equal to the replica, as for :meth:`ShardedPool.fetch`.
+
+    ``bases`` (device int64 ``[W]``) holds, for every rank, the address of its pool buffer in this process -- this rank's own
+    buffer, or a peer mapping -- and ``base_bytes`` (host int64 ``[W]``) the bytes in use there; ``src_offset[i]`` is the byte
+    offset of global image ``i`` in its owner's buffer.  The pool keeps ``sharded`` -- and with it the local buffer that peers
+    read -- alive.  Lifetime rule: :meth:`close` (collective) before any rank drops, grows or appends to its shard."""
+
+    def __init__(self, sharded: ShardedPool, bases: Sequence[int], base_bytes: Sequence[int], src_offset,
+                 mapped: Optional[Dict[int, int]] = None):
+        if not (len(bases) == len(base_bytes) == sharded.world):
+            raise ValueError("one base address and size per rank")
+        if any(int(b) % 16 for b in bases):
+            raise ValueError("ragged_gather reads 16-byte vectors: every base address must be 16-byte aligned")
+        self.sharded = sharded
+        self.device = sharded.device
+        self.bases: Optional[torch.Tensor] = torch.tensor([int(b) for b in bases], dtype=torch.int64, device=self.device)
+        self.base_bytes = torch.tensor([int(b) for b in base_bytes], dtype=torch.int64)
+        self.src_offset = np.asarray(src_offset, dtype=np.int64)
+        if len(self.src_offset) != len(sharded):
+            raise ValueError("one source offset per index entry")
+        self._mapped: Dict[int, int] = dict(mapped or {})          # rank -> base returned by bgd_ipc_open
+        local = sharded.local
+        self._local_state = self._state(local)
+
+    @staticmethod
+    def _state(local: RaggedPool) -> tuple:
+        return (id(local.data), local.data.data_ptr() if local.data is not None else 0, local.used, len(local))
+
+    def __len__(self) -> int:
+        return len(self.sharded)
+
+    @classmethod
+    def open(cls, sharded: ShardedPool) -> "PeerPool":
+        """Collective on ``sharded.group``: map every rank's shard into every other rank.  Each rank synchronises its device
+        (its shard is fully written), exports its buffer (``bgd_ipc_export``), and one ``all_gather_object`` shares
+        ``(host id, device UUID, handle, offset, bytes)`` and the slot offsets; each rank then opens every other rank's handle
+        (its own buffer is used directly: a handle cannot be opened in the process that exported it), and a second gather of
+        the outcomes makes every rank raise together.  ``ValueError`` -- pointing at ``attach_sharded_pool`` / ``fetch`` --
+        when the ranks are on different hosts, when a buffer cannot be exported (``expandable_segments``, the
+        ``cudaMallocAsync`` backend) or when a peer cannot be mapped."""
+        import ctypes
+        import torch.distributed as dist
+        from . import _cabi
+        local, rank, group = sharded.local, sharded.rank, sharded.group
+        dev = sharded.device if sharded.device.index is not None else torch.device("cuda", torch.cuda.current_device())
+        torch.cuda.synchronize(dev)
+        meta = dict(host=_host_id(), uuid=str(torch.cuda.get_device_properties(dev).uuid), handle=None, offset=0,
+                    bytes=int(local.used), error=None, offsets=np.asarray(local.slots["offset"], dtype=np.int64))
+        if local.used:
+            handle = ctypes.create_string_buffer(64)
+            off = ctypes.c_int64()
+            try:
+                with torch.cuda.device(dev):
+                    _cabi.check(_cabi.lib().bgd_ipc_export(local.data.data_ptr(), handle, ctypes.byref(off)))
+                meta.update(handle=handle.raw, offset=int(off.value))
+            except (ValueError, _cabi.BgdError) as e:
+                meta["error"] = str(e)
+        metas: List[Optional[dict]] = [None] * sharded.world
+        dist.all_gather_object(metas, meta, group=group)
+        check_peer_meta(metas)
+        mapped: Dict[int, int] = {}
+        error = None
+        for r, m in enumerate(metas):
+            if r == rank or m["handle"] is None:
+                continue
+            base = ctypes.c_void_p()
+            try:
+                _cabi.check(_cabi.lib().bgd_ipc_open(m["handle"], dev.index, ctypes.byref(base)))
+            except (ValueError, _cabi.BgdError) as e:
+                error = f"rank {rank} (device {meta['uuid']}) cannot map the shard of rank {r} (device {m['uuid']}): {e}"
+                break
+            mapped[r] = int(base.value)
+        errors: List[Optional[str]] = [None] * sharded.world
+        dist.all_gather_object(errors, error, group=group)
+        failed = [e for e in errors if e is not None]
+        if failed:
+            _close_mappings(mapped, dev)
+            raise ValueError(f"{failed[0]}; {_USE_FETCH}")
+        bases = [local.data.data_ptr() if r == rank and local.used else
+                 (mapped[r] + m["offset"] if r in mapped else 0) for r, m in enumerate(metas)]
+        src_offset = np.zeros(len(sharded), dtype=np.int64)
+        for r, m in enumerate(metas):
+            own = sharded.owner == r
+            src_offset[own] = m["offsets"][sharded.slot[own]]
+        return cls(sharded, bases, [m["bytes"] for m in metas], src_offset, mapped)
+
+    def gather(self, bg_idx, apply) -> Tuple[RaggedPool, torch.Tensor]:
+        """Local.  ``bg_idx`` / ``apply`` ([B], host or device): the global pool index and the mix flag of every sample of this
+        rank's batch.  Returns ``(batch pool, slot)`` as :meth:`ShardedPool.fetch` does -- the same deduplicated request order,
+        every image on a 16-byte boundary, the int32 ``[B]`` slot of each sample (0 for a sample that is not mixed) -- from one
+        ``ragged_gather`` launch on the current stream.  Ranks call it independently, as many times as they like; the host
+        never waits for the device (the slot table travels from pinned memory, and ``slot`` is returned pinned)."""
+        if self.bases is None:
+            raise RuntimeError("PeerPool.gather after close()")
+        sp = self.sharded
+        if self._state(sp.local) != self._local_state:
+            raise RuntimeError("the local shard was reallocated or appended to after PeerPool.open: peers would read a stale "
+                               "mapping; close() the PeerPool before changing a shard, then open a new one")
+        mine = sp.requests_of(bg_idx, apply)
+        bad = [g for g in mine if not 0 <= g < len(sp)]
+        if bad:
+            raise ValueError(f"background {bad[0]} is outside the {len(sp)}-image index")
+        segments, dst, total = peer_segments(mine, sp.owner, self.src_offset, sp.nbytes)
+        batch = RaggedPool(sp.bg_resize, self.device, tables=sp.tables)
+        batch.data = torch.ops.bgdebias.ragged_gather(self.bases, self.base_bytes, torch.from_numpy(segments), total)
+        batch.used = total
+        if mine:
+            batch.slots = np.array([sp.local.make_slot(int(o), int(sp.h[g]), int(sp.w[g])) for o, g in zip(dst, mine)],
+                                   dtype=SLOT_DTYPE)
+            raw = torch.from_numpy(batch.slots.view(np.uint8).reshape(-1))
+            batch._slots_dev = raw.pin_memory().to(self.device, non_blocking=True)
+        return batch, sp.sample_slots(bg_idx, apply, mine).pin_memory()     # pinned: its upload does not wait either
+
+    def close(self) -> None:
+        """Collective on the pool's group: each rank synchronises its device (its gathers have finished reading), all ranks
+        meet at a barrier, then each unmaps its peers' shards.  Call it before any rank drops or changes its shard."""
+        import torch.distributed as dist
+        if self.bases is None:
+            return
+        torch.cuda.synchronize(self.device)
+        dist.barrier(group=self.sharded.group)
+        _close_mappings(self._mapped, self.device)
+        self._mapped, self.bases = {}, None
+
+
+def _close_mappings(mapped: Dict[int, int], device) -> None:
+    from . import _cabi
+    with torch.cuda.device(device):
+        for base in mapped.values():
+            _cabi.check(_cabi.lib().bgd_ipc_close(base))
+    mapped.clear()
 
 
 def shard_extracted_backgrounds(output_dir, image_suffix: str = ".jpg", bg_resize: Optional[int] = 256, device="cuda",

@@ -363,6 +363,36 @@ int bgd_bgmix_resize_blend_f32_host(const uint8_t *h_src, int64_t src_bytes, con
 int bgd_ragged_pack_u8(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_segments, int64_t n, uint8_t *d_out,
                        int64_t out_bytes, void *stream);
 
+/* ---- multi-source ragged gather over peer-mapped shards (bgdebias_b200.pool.PeerPool.gather) ---------------------------
+ * The receiving form of the same replacement (libs/loader/comix_loader.py:126-131) on one node: every rank's shard is mapped
+ * into every other rank once (bgd_ipc_export / bgd_ipc_open), and a rank copies the images its batch drew straight from their
+ * owners' memory into one buffer, in one launch, with no collective and no host synchronisation.
+ *
+ *   d_bases       DEVICE table of n_bases source base pointers (a rank's own buffer or a peer mapping), each 16-byte aligned
+ *   h_base_bytes  HOST int64 [n_bases]: readable bytes from each base
+ *   h_segments    HOST int64 [n][4]: {source index, source byte offset, destination byte offset, bytes}; both offsets 16-byte
+ *                 aligned, every segment inside its source's [0, h_base_bytes) and inside d_out[0, out_bytes)
+ *   d_out         destination buffer, 16-byte aligned; bytes outside every segment are left untouched
+ * Every segment is validated on the host before anything is launched (BGD_ERR_INVALID names the first bad one); the table then
+ * travels through the per-thread workspace ring, so the call does not wait for the stream.  n <= 65535; n == 0 (or only
+ * empty segments) launches nothing. */
+int bgd_ragged_gather_u8(const uint8_t *const *d_bases, const int64_t *h_base_bytes, int64_t n_bases, const int64_t *h_segments,
+                         int64_t n, uint8_t *d_out, int64_t out_bytes, void *stream);
+
+/* Export the allocation that holds d_ptr (device memory of the current device) to other processes of this host: handle
+ * receives the 64-byte cudaIpcMemHandle_t of the allocation's base (found with cuMemGetAddressRange), offset the byte offset
+ * of d_ptr from that base.  BGD_ERR_UNSUPPORTED when the memory cannot be exported: it must come from cudaMalloc (torch's
+ * native caching allocator without expandable_segments; not the cudaMallocAsync backend, not cuMemCreate mappings). */
+int bgd_ipc_export(const void *d_ptr, uint8_t *handle, int64_t *offset);
+
+/* Map a handle of bgd_ipc_export from ANOTHER process into this process on `device` (cudaIpcOpenMemHandle with
+ * cudaIpcMemLazyEnablePeerAccess); *d_base receives the mapped allocation base.  A handle cannot be opened in the process
+ * that exported it.  BGD_ERR_UNSUPPORTED when the mapping fails (e.g. the two devices cannot access each other). */
+int bgd_ipc_open(const uint8_t *handle, int device, void **d_base);
+
+/* Unmap a base returned by bgd_ipc_open.  The exporter must keep its allocation alive until every mapping is closed. */
+int bgd_ipc_close(void *d_base);
+
 #ifdef __cplusplus
 }
 #endif
