@@ -130,6 +130,24 @@ class _RawframeBase:
 _Base = _MMRawframeDataset if _HAVE_MMACTION else _RawframeBase
 
 
+def _read_image(path: str, reader: Optional[Callable] = None) -> torch.Tensor:
+    """``reader(path)``, or ``torchvision.io.read_image(mode=RGB)`` as the reference decodes a background (comix_loader.py:130)."""
+    if reader is not None:
+        return torch.as_tensor(reader(path))
+    from torchvision.io import ImageReadMode, read_image
+    return read_image(path, mode=ImageReadMode.RGB)
+
+
+def _blend_clip(imgs: torch.Tensor, bg: torch.Tensor, top: int, left: int, mean, std, alpha: float, device) -> torch.Tensor:
+    """One normalised clip fp32 ``[T,3,H,W]`` blended on ``device`` with the crop at (top, left) of one resized background
+    ``[3,Hb,Wb]`` (comix_loader.py:138-145); returned on the clip's device."""
+    i32 = lambda v: torch.tensor([v], dtype=torch.int32, device=device)   # noqa: E731
+    out = torch.ops.bgdebias.bgmix_blend_normfg(
+        imgs.to(device, torch.float32).unsqueeze(0), bg.unsqueeze(0).to(device), i32(0), i32(top), i32(left),
+        torch.ones(1, dtype=torch.uint8, device=device), torch.tensor(mean), torch.tensor(std), float(alpha), "NTCHW")[0]
+    return out.to(imgs.device)
+
+
 def draw_crop(h: int, w: int, crop) -> tuple:
     """``RandomCrop.get_params`` (torchvision): nothing drawn when the image already has the crop
     size, else top then left from torch's global generator."""
@@ -201,14 +219,10 @@ class BackgroundMixDataset(_Base):
         self.device = torch.device(device)
         self.device_mix = device_mix
         self._bg_reader = bg_reader
-        self._pool: Optional[BackgroundPool] = None
-        self._pool_key = None
-        self._store: Optional[BackgroundStore] = None
-        self._sharded: Optional[ShardedPool] = None
-        self._peer: Optional[PeerPool] = None             # set with _sharded: gather from peer mappings instead of fetch
-        self._shard_of: dict = {}                         # name (and its realpath) -> global index of the sharded pool
-        self._shard_rows_key, self._shard_rows = None, None
-        self._resized_cache = {}
+        self._attach(self.device)
+        self._resized_cache = {}                          # path -> size after Resize, for forked DataLoader workers
+        self._aa: Optional[AATables] = None
+        self._luts: dict = {}                             # (mean, std) -> foreground LUT on self.device
 
         # pool assembly: the three modes of comix_loader.py:84-103
         if self.back_ground_from_bg_dir:
@@ -231,10 +245,13 @@ class BackgroundMixDataset(_Base):
 
     # ---- background access -------------------------------------------------------------------
     def _read_bg(self, path: str) -> torch.Tensor:
-        if self._bg_reader is not None:
-            return torch.as_tensor(self._bg_reader(path))
-        from torchvision.io import ImageReadMode, read_image
-        return read_image(path, mode=ImageReadMode.RGB)
+        return _read_image(path, self._bg_reader)
+
+    def _random_frame(self) -> torch.Tensor:
+        """A random frame of a random video (comix_loader.py:133-136): ``random.choice``, then ``random.randint``."""
+        video = random.choice(self.video_infos)
+        frame_index = random.randint(self.start_index, video['total_frames'] - 1 + self.start_index)
+        return self._read_bg(osp.join(video['frame_dir'], self.filename_tmpl.format(frame_index)))
 
     def _get_bg_image(self):
         """Same draws and return value as the reference (comix_loader.py:126-136): a float ``[3,h,w]``
@@ -242,10 +259,7 @@ class BackgroundMixDataset(_Base):
         if self.back_ground_from_bg_dir:
             bg_idx = torch.randint(len(self.bg_files), (1,)).item()
             return self._read_bg(self.bg_files[bg_idx]).float(), bg_idx
-        video = random.choice(self.video_infos)
-        frame_index = random.randint(self.start_index, video['total_frames'] - 1 + self.start_index)
-        path = osp.join(video['frame_dir'], self.filename_tmpl.format(frame_index))
-        return self._read_bg(path).float(), -2      # to pass sanity check
+        return self._random_frame().float(), -2      # to pass sanity check
 
     def device_pool(self) -> BackgroundPool:
         """The pool for the current ``bg_files``, index i = ``bg_files[i]``.  Every path is decoded + resized
@@ -269,9 +283,7 @@ class BackgroundMixDataset(_Base):
         them are decoded on demand as usual."""
         store = BackgroundStore(self.bg_resize, ragged.device)
         store.adopt([osp.realpath(p) for p in paths], ragged)
-        self._store, self._pool, self._pool_key = store, None, None
-        self._sharded, self._peer = None, None
-        self.device = ragged.device
+        self._attach(ragged.device, store=store)
 
     def attach_sharded_pool(self, paths: Sequence[str], sharded: ShardedPool) -> None:
         """Mix from a pool sharded across the ranks of a process group (``pool.shard_extracted_backgrounds``): ``paths[i]`` names
@@ -283,16 +295,9 @@ class BackgroundMixDataset(_Base):
 
         Every rank of the pool's group must call :meth:`device_finish` (or :meth:`mix_batch_on_device`) once per batch, in
         lockstep: see :meth:`pool.ShardedPool.fetch`."""
-        if len(paths) != len(sharded):
-            raise ValueError("one path per image of the sharded pool")
-        of: dict = {}
-        for i, p in enumerate(paths):
-            of.setdefault(str(p), i)
-            of.setdefault(osp.realpath(p), i)             # bg_files are matched after realpath like bg_dir (:61-68)
-        self._sharded, self._shard_of, self._peer = sharded, of, None
-        self._shard_rows_key, self._shard_rows = None, None
-        self._store, self._pool, self._pool_key = None, None, None
-        self.device = sharded.device
+        if [str(p) for p in paths] != sharded.names:
+            raise ValueError("paths must be the names of the sharded pool's images, in index order")
+        self._attach(sharded.device, sharded=sharded, fetch=sharded.fetch)
 
     def attach_peer_pool(self, paths: Sequence[str], peer: PeerPool) -> None:
         """The twin of :meth:`attach_sharded_pool` for a pool whose shards are mapped into every rank of one node
@@ -301,24 +306,22 @@ class BackgroundMixDataset(_Base):
         launch (:meth:`pool.PeerPool.gather`) -- no collective, so ranks need not call it in lockstep, and the host does
         not wait for the device.  Attaching a pool of any other kind detaches this one."""
         self.attach_sharded_pool(paths, peer.sharded)
-        self._peer = peer
+        self._fetch = peer.gather
 
-    def _shard_index(self, path: str) -> int:
-        i = self._shard_of.get(path)
-        if i is None:
-            i = self._shard_of.get(osp.realpath(path))
-        if i is None:
-            raise ValueError(f"background {path!r} of bg_files is not in the sharded pool's index; a sharded pool mixes "
-                             "only the extracted backgrounds it was built from")
-        return i
+    def _attach(self, device, store: Optional[BackgroundStore] = None, sharded: Optional[ShardedPool] = None,
+                fetch: Optional[Callable] = None) -> None:
+        """Mix from one pool, detaching any other: the replica ``store`` (``None``: built from ``bg_files`` on demand), or a
+        ``sharded`` pool with ``fetch(bg_idx, apply) -> (batch pool, slot)`` that brings a batch's images to this rank."""
+        self._store, self._pool, self._pool_key = store, None, None
+        self._sharded, self._fetch, self._shard_rows = sharded, fetch, None
+        self.device = device
 
     def _sharded_rows(self) -> np.ndarray:
         """Global index of every entry of the current ``bg_files`` (cached per list)."""
         key = tuple(self.bg_files)
-        if self._shard_rows is None or key != self._shard_rows_key:
-            self._shard_rows = np.array([self._shard_index(p) for p in self.bg_files], dtype=np.int64)
-            self._shard_rows_key = key
-        return self._shard_rows
+        if self._shard_rows is None or key != self._shard_rows[0]:
+            self._shard_rows = (key, self._sharded.rows_of(self.bg_files))
+        return self._shard_rows[1]
 
     # ---- per-sample API (reference contract) ---------------------------------------------------
     def prepare_train_frames(self, idx):
@@ -354,9 +357,7 @@ class BackgroundMixDataset(_Base):
                 h, w = self._bg_hw(bg_idx)                # RandomCrop sees the DRAWN image after Resize (:72-73,139-140)
             else:
                 # random frame of a random video (:133-136): same draws, the decoded uint8 frame travels with the sample
-                video = random.choice(self.video_infos)
-                frame_index = random.randint(self.start_index, video['total_frames'] - 1 + self.start_index)
-                img = self._read_bg(osp.join(video['frame_dir'], self.filename_tmpl.format(frame_index)))
+                img = self._random_frame()
                 h, w = self._resized_hw(int(img.shape[1]), int(img.shape[2]))
                 result['bg_img'] = img.to(torch.uint8)
                 bg_idx = -2                               # to pass sanity check
@@ -376,13 +377,7 @@ class BackgroundMixDataset(_Base):
         imgs = result['imgs']
         if imgs.dim() != 4 or imgs.shape[1] != 3 or tuple(imgs.shape[2:]) != (th, tw):
             raise ValueError(f"imgs must be [T, 3, {th}, {tw}] (got {tuple(imgs.shape)})")
-        dev = self.device
-        i32 = lambda v: torch.tensor([v], dtype=torch.int32, device=dev)   # noqa: E731
-        blend = torch.ops.bgdebias.bgmix_blend_normfg(
-            imgs.to(dev, torch.float32).unsqueeze(0), bg_img.unsqueeze(0).to(dev), i32(0), i32(top), i32(left),
-            torch.ones(1, dtype=torch.uint8, device=dev), torch.tensor(self.bg_mean), torch.tensor(self.bg_std),
-            float(self.alpha), "NTCHW")[0]
-        result['imgs'] = blend.to(imgs.device)
+        result['imgs'] = _blend_clip(imgs, bg_img, top, left, self.bg_mean, self.bg_std, self.alpha, self.device)
         result['bg_idx'] = bg_idx
         return result
 
@@ -394,7 +389,7 @@ class BackgroundMixDataset(_Base):
         process that owns the GPU decodes the image into the store (once), and a forked DataLoader worker reads the image
         header (cached per path).  With a sharded pool the global index answers."""
         if self._sharded is not None:
-            return self._sharded.hw(self._shard_index(self.bg_files[bg_idx]))
+            return self._sharded.hw(int(self._sharded.rows_of([self.bg_files[bg_idx]])[0]))
         if self._pool is not None and tuple(self.bg_files) == self._pool_key:
             return self._pool.hw_of(bg_idx)
         path = self.bg_files[bg_idx]
@@ -409,7 +404,7 @@ class BackgroundMixDataset(_Base):
             self._store.ensure([path], self._read_bg)
             return self._store.hw_of(self._store.slot_of[path])
         if self._bg_reader is not None:                   # DataLoader worker: size only, cached per path
-            img = torch.as_tensor(self._bg_reader(path))
+            img = self._read_bg(path)
             h, w = int(img.shape[1]), int(img.shape[2])
         else:
             from PIL import Image
@@ -472,8 +467,7 @@ class BackgroundMixDataset(_Base):
             # (a local launch), then the random-frame route
             idx = torch.as_tensor(bg_idx).cpu().clamp(min=0, max=max(len(self.bg_files) - 1, 0))
             gidx = torch.from_numpy(self._sharded_rows())[idx] if len(self.bg_files) else idx
-            get = self._peer.gather if self._peer is not None else self._sharded.fetch
-            batch_pool, slot = get(gidx, torch.as_tensor(bg_apply).cpu())
+            batch_pool, slot = self._fetch(gidx, torch.as_tensor(bg_apply).cpu())
             if not len(batch_pool):                       # nothing mixed on this rank: a placeholder the blend never reads
                 batch_pool.append([torch.zeros((3, th, tw), dtype=torch.uint8)])
             ragged, dense, rows = batch_pool, None, as_dev(slot, torch.int32)
@@ -507,15 +501,14 @@ class BackgroundMixDataset(_Base):
         return out
 
     def _aa_tables(self) -> AATables:
-        if "aa_tables" not in self._resized_cache:
-            self._resized_cache["aa_tables"] = AATables(self.device)
-        return self._resized_cache["aa_tables"]
+        if self._aa is None:
+            self._aa = AATables(self.device)
+        return self._aa
 
     def _lut(self, mean, std) -> torch.Tensor:
-        key = ("lut", mean, std)
-        if key not in self._resized_cache:
-            self._resized_cache[key] = ops.make_fg_lut(mean, std, self.device)
-        return self._resized_cache[key]
+        if (mean, std) not in self._luts:
+            self._luts[(mean, std)] = ops.make_fg_lut(mean, std, self.device)
+        return self._luts[(mean, std)]
 
     @staticmethod
     def host_collate(samples: List[dict]) -> dict:
@@ -559,18 +552,14 @@ class BackgroundMixDataset(_Base):
         ``randAug``, ``bg_idx``) with one fused launch.  ``dtype`` / ``memory_format``: see :meth:`mix_batch_on_device`."""
         out = {k: v for k, v in batch.items()
                if k not in ('imgs', 'bg_top', 'bg_left', 'bg_apply', 'fg_geom', 'fg_frames', 'bg_imgs', 'bg_slot')}
-        if self.back_ground_from_bg_dir or 'bg_imgs' in batch:
-            out['imgs'] = self.mix_batch_on_device(batch['imgs'], batch['bg_idx'], batch['bg_top'], batch['bg_left'],
-                                                   batch['bg_apply'], layout=layout, fg_geom=batch.get('fg_geom'),
-                                                   fg_frames=batch.get('fg_frames'), bg_imgs=batch.get('bg_imgs'),
-                                                   bg_slot=batch.get('bg_slot'), dtype=dtype, memory_format=memory_format)
-        else:                                             # random-frame mode and no sample of the batch was mixed
-            out['imgs'] = self.mix_batch_on_device(batch['imgs'], batch['bg_idx'], batch['bg_top'], batch['bg_left'],
-                                                   batch['bg_apply'], layout=layout, fg_geom=batch.get('fg_geom'),
-                                                   fg_frames=batch.get('fg_frames'),
-                                                   bg_imgs=[torch.zeros((3, *self.bg_crop_size), dtype=torch.uint8)],
-                                                   bg_slot=torch.zeros(len(batch['bg_idx']), dtype=torch.int32),
-                                                   dtype=dtype, memory_format=memory_format)
+        if not self.back_ground_from_bg_dir and 'bg_imgs' not in batch:
+            # random-frame mode and no sample of the batch was mixed: a placeholder frame the blend never reads
+            batch = dict(batch, bg_imgs=[torch.zeros((3, *self.bg_crop_size), dtype=torch.uint8)],
+                         bg_slot=torch.zeros(len(batch['bg_idx']), dtype=torch.int32))
+        out['imgs'] = self.mix_batch_on_device(batch['imgs'], batch['bg_idx'], batch['bg_top'], batch['bg_left'],
+                                               batch['bg_apply'], layout=layout, fg_geom=batch.get('fg_geom'),
+                                               fg_frames=batch.get('fg_frames'), bg_imgs=batch.get('bg_imgs'),
+                                               bg_slot=batch.get('bg_slot'), dtype=dtype, memory_format=memory_format)
         return out
 
     def gpu_collate(self, samples: List[dict], dtype: torch.dtype = torch.float32,
@@ -621,10 +610,7 @@ class BackgroundMix:
         self._bg_reader = bg_reader
 
     def _read(self, path):
-        if self._bg_reader is not None:
-            return torch.as_tensor(self._bg_reader(path))
-        from torchvision.io import ImageReadMode, read_image
-        return read_image(path, mode=ImageReadMode.RGB)
+        return _read_image(path, self._bg_reader)
 
     def __call__(self, results):
         results['bg_idx'] = -1
@@ -635,13 +621,7 @@ class BackgroundMix:
         bg = resize_like_reference(self._read(self.bg_files[bg_idx]).float(), self.bg_resize)
         top, left = draw_crop(bg.shape[1], bg.shape[2], self.bg_crop_size)
         imgs = torch.as_tensor(results['imgs'])
-        dev = self.device
-        i32 = lambda v: torch.tensor([v], dtype=torch.int32, device=dev)   # noqa: E731
-        out = torch.ops.bgdebias.bgmix_blend_normfg(
-            imgs.to(dev, torch.float32).unsqueeze(0), bg.unsqueeze(0).to(dev), i32(0), i32(top), i32(left),
-            torch.ones(1, dtype=torch.uint8, device=dev), torch.tensor(self.bg_mean), torch.tensor(self.bg_std),
-            float(self.alpha), "NTCHW")[0]
-        results['imgs'] = out.to(imgs.device)
+        results['imgs'] = _blend_clip(imgs, bg, top, left, self.bg_mean, self.bg_std, self.alpha, self.device)
         results['bg_idx'] = bg_idx
         return results
 

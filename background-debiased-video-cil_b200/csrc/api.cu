@@ -438,6 +438,69 @@ static int f32_layout(const char *who, int layout)
     return layout == BGD_LAYOUT_NTHWC ? fail(BGD_ERR_INVALID, "%s: unknown layout %d", who, layout) : BGD_OK;
 }
 
+// ---- the host-buffer blends: foreground and draws staged through the thread's Stager, slot 0 ----------------------------
+struct StagedBlend {
+    cudaStream_t stream;
+    const uint8_t *fg;                          // fg_bytes of foreground
+    const int32_t *bg_idx, *top, *left;         // B each
+    const uint8_t *apply;                       // B
+};
+
+// Validates the applied draws against the pool (P images of Hb x Wb, an H x W crop), then copies the foreground and the draws
+// to the device on the Stager's stream: device layout fg | bg_idx | top | left | apply.  Returns without waiting.
+static int stage_host_blend(const char *who, const uint8_t *h_fg, size_t fg_bytes, int64_t B, int64_t H, int64_t W, int64_t P,
+                            int64_t Hb, int64_t Wb, const int32_t *h_bg_idx, const int32_t *h_top, const int32_t *h_left,
+                            const uint8_t *h_apply, int device, StagedBlend *out)
+{
+    // the reference's RandomCrop raises when the crop does not fit; validate here, on host values
+    for (int64_t b = 0; b < B; ++b) {
+        if (!h_apply[b]) continue;
+        if (h_bg_idx[b] < 0 || h_bg_idx[b] >= P)
+            return fail(BGD_ERR_INVALID, "%s: bg_idx[%lld]=%d outside pool of %lld", who, (long long)b, h_bg_idx[b], (long long)P);
+        if (h_top[b] < 0 || h_top[b] + H > Hb || h_left[b] < 0 || h_left[b] + W > Wb)
+            return fail(BGD_ERR_INVALID, "%s: crop of sample %lld leaves the pool image", who, (long long)b);
+    }
+    DeviceProps dp;
+    if (int rc = get_device_props(device, &dp)) return rc;
+    BGD_CUDA_TRY(cudaSetDevice(device));
+    const size_t par_bytes = (size_t)B * 13 + 64;
+    const bool fg_pinned = is_pinned_host(h_fg);      // a page-locked foreground is copied straight from the caller's buffer
+    Stager &st = thread_stager();
+    if (int rc = st.ensure(device, fg_bytes + par_bytes + 64, 64, (fg_pinned ? 0 : fg_bytes) + par_bytes + 64, 64)) return rc;
+    cudaStream_t s = st.stream[0];
+    uint8_t *hp = st.h_in[0], *dp_ = st.d_in[0];
+    const size_t o = (fg_bytes + 15) & ~(size_t)15;
+    uint8_t *hpar = fg_pinned ? hp : hp + o;
+    if (!fg_pinned) std::memcpy(hp, h_fg, fg_bytes);
+    std::memcpy(hpar, h_bg_idx, (size_t)B * 4);
+    std::memcpy(hpar + (size_t)B * 4, h_top, (size_t)B * 4);
+    std::memcpy(hpar + (size_t)B * 8, h_left, (size_t)B * 4);
+    std::memcpy(hpar + (size_t)B * 12, h_apply, (size_t)B);
+    if (fg_pinned) {
+        BGD_CUDA_TRY(cudaMemcpyAsync(dp_, h_fg, fg_bytes, cudaMemcpyHostToDevice, s));
+        BGD_CUDA_TRY(cudaMemcpyAsync(dp_ + o, hpar, (size_t)B * 13, cudaMemcpyHostToDevice, s));
+    } else {
+        BGD_CUDA_TRY(cudaMemcpyAsync(dp_, hp, o + (size_t)B * 13, cudaMemcpyHostToDevice, s));
+    }
+    const int32_t *d_idx = reinterpret_cast<const int32_t *>(dp_ + o);
+    *out = StagedBlend{s, dp_, d_idx, d_idx + B, d_idx + 2 * B, dp_ + o + (size_t)B * 12};
+    return BGD_OK;
+}
+
+// After the launch on s: the optional checksum of the n floats of d_out, then the call's one synchronisation.
+static int finish_host_blend(const float *d_out, int64_t n, double *h_checksum, cudaStream_t s)
+{
+    Stager &st = thread_stager();
+    if (h_checksum) {
+        double *d_sum = reinterpret_cast<double *>(st.d_out[0]);
+        if (int rc = launch_sum_f32(d_out, n, d_sum, s)) return rc;
+        BGD_CUDA_TRY(cudaMemcpyAsync(st.h_out[0], d_sum, sizeof(double), cudaMemcpyDeviceToHost, s));
+    }
+    BGD_CUDA_TRY(cudaStreamSynchronize(s));
+    if (h_checksum) std::memcpy(h_checksum, st.h_out[0], sizeof(double));
+    return BGD_OK;
+}
+
 }  // namespace bgd
 
 // =================================================================================================
@@ -688,48 +751,14 @@ int bgd_bgmix_blend_f32_host(const uint8_t *h_fg, int64_t B, int64_t T, int64_t 
     if (int rc = f32_layout("bgmix", layout)) return rc;
     if (B == 0 || T == 0 || H == 0 || W == 0) { if (h_checksum) *h_checksum = 0.0; return BGD_OK; }
     if (!h_fg || !h_bg_idx || !h_top || !h_left || !h_apply) return fail(BGD_ERR_INVALID, "bgmix: null host pointer");
-    // the reference's RandomCrop raises when the crop does not fit; validate here, on host values
-    for (int64_t b = 0; b < B; ++b) {
-        if (!h_apply[b]) continue;
-        if (h_bg_idx[b] < 0 || h_bg_idx[b] >= P) return fail(BGD_ERR_INVALID, "bgmix: bg_idx[%lld]=%d outside pool of %lld", (long long)b, h_bg_idx[b], (long long)P);
-        if (h_top[b] < 0 || h_top[b] + H > Hb || h_left[b] < 0 || h_left[b] + W > Wb)
-            return fail(BGD_ERR_INVALID, "bgmix: crop of sample %lld leaves the pool image", (long long)b);
-    }
-    DeviceProps dp;
-    if (int rc = get_device_props(device, &dp)) return rc;
-    BGD_CUDA_TRY(cudaSetDevice(device));
-    const size_t fg_bytes = (size_t)B * T * H * W * 3;
-    const size_t par_bytes = (size_t)B * 13 + 64;
-    const bool fg_pinned = is_pinned_host(h_fg);      // page-locked clips are copied straight from the caller's buffer
-    Stager &st = thread_stager();
-    if (int rc = st.ensure(device, fg_bytes + par_bytes + 64, 64, (fg_pinned ? 0 : fg_bytes) + par_bytes + 64, 64)) return rc;
-    cudaStream_t s = st.stream[0];
-    uint8_t *hp = st.h_in[0], *dp_ = st.d_in[0];
-    const size_t o = (fg_bytes + 15) & ~(size_t)15;     // device layout: clips | bg_idx | top | left | apply
-    uint8_t *hpar = fg_pinned ? hp : hp + o;
-    if (!fg_pinned) std::memcpy(hp, h_fg, fg_bytes);
-    std::memcpy(hpar, h_bg_idx, (size_t)B * 4);
-    std::memcpy(hpar + (size_t)B * 4, h_top, (size_t)B * 4);
-    std::memcpy(hpar + (size_t)B * 8, h_left, (size_t)B * 4);
-    std::memcpy(hpar + (size_t)B * 12, h_apply, (size_t)B);
-    if (fg_pinned) {
-        BGD_CUDA_TRY(cudaMemcpyAsync(dp_, h_fg, fg_bytes, cudaMemcpyHostToDevice, s));
-        BGD_CUDA_TRY(cudaMemcpyAsync(dp_ + o, hpar, (size_t)B * 13, cudaMemcpyHostToDevice, s));
-    } else {
-        BGD_CUDA_TRY(cudaMemcpyAsync(dp_, hp, o + (size_t)B * 13, cudaMemcpyHostToDevice, s));
-    }
-    const int32_t *d_idx = reinterpret_cast<const int32_t *>(dp_ + o);
-    if (int rc = launch_bgmix(dp_, nullptr, B, T, H, W, d_bg_pool, false, P, Hb, Wb, d_idx, d_idx + B, d_idx + 2 * B,
-                              dp_ + o + (size_t)B * 12, d_fg_lut, h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out, s))
+    StagedBlend g;
+    if (int rc = stage_host_blend("bgmix", h_fg, (size_t)B * T * H * W * 3, B, H, W, P, Hb, Wb, h_bg_idx, h_top, h_left, h_apply,
+                                  device, &g))
         return rc;
-    if (h_checksum) {
-        double *d_sum = reinterpret_cast<double *>(st.d_out[0]);
-        if (int rc = launch_sum_f32(d_out, (int64_t)B * T * 3 * H * W, d_sum, s)) return rc;
-        BGD_CUDA_TRY(cudaMemcpyAsync(st.h_out[0], d_sum, sizeof(double), cudaMemcpyDeviceToHost, s));
-    }
-    BGD_CUDA_TRY(cudaStreamSynchronize(s));
-    if (h_checksum) std::memcpy(h_checksum, st.h_out[0], sizeof(double));
-    return BGD_OK;
+    if (int rc = launch_bgmix(g.fg, nullptr, B, T, H, W, d_bg_pool, false, P, Hb, Wb, g.bg_idx, g.top, g.left, g.apply, d_fg_lut,
+                              h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out, g.stream))
+        return rc;
+    return finish_host_blend(d_out, B * T * 3 * H * W, h_checksum, g.stream);
 }
 
 int bgd_bgmix_resize_blend_f32_host(const uint8_t *h_src, int64_t src_bytes, const int64_t *h_geom, int64_t B, int64_t T,
@@ -744,48 +773,14 @@ int bgd_bgmix_resize_blend_f32_host(const uint8_t *h_src, int64_t src_bytes, con
     if (B == 0 || T == 0 || H == 0 || W == 0) { if (h_checksum) *h_checksum = 0.0; return BGD_OK; }
     if (!h_src || !h_geom || !h_bg_idx || !h_top || !h_left || !h_apply) return fail(BGD_ERR_INVALID, "bgmix_resize: null host pointer");
     if (src_bytes % 4) return fail(BGD_ERR_INVALID, "bgmix_resize: the source buffer must be a multiple of 4 bytes long");
-    for (int64_t b = 0; b < B; ++b) {
-        if (!h_apply[b]) continue;
-        if (h_bg_idx[b] < 0 || h_bg_idx[b] >= P) return fail(BGD_ERR_INVALID, "bgmix_resize: bg_idx[%lld]=%d outside pool of %lld", (long long)b, h_bg_idx[b], (long long)P);
-        if (h_top[b] < 0 || h_top[b] + H > Hb || h_left[b] < 0 || h_left[b] + W > Wb)
-            return fail(BGD_ERR_INVALID, "bgmix_resize: crop of sample %lld leaves the pool image", (long long)b);
-    }
-    DeviceProps dp;
-    if (int rc = get_device_props(device, &dp)) return rc;
-    BGD_CUDA_TRY(cudaSetDevice(device));
-    const size_t fg_bytes = (size_t)src_bytes;
-    const size_t par_bytes = (size_t)B * 13 + 64;
-    const bool fg_pinned = is_pinned_host(h_src);     // page-locked crops are copied straight from the caller's buffer
-    Stager &st = thread_stager();
-    if (int rc = st.ensure(device, fg_bytes + par_bytes + 64, 64, (fg_pinned ? 0 : fg_bytes) + par_bytes + 64, 64)) return rc;
-    cudaStream_t s = st.stream[0];
-    uint8_t *hp = st.h_in[0], *dp_ = st.d_in[0];
-    const size_t o = (fg_bytes + 15) & ~(size_t)15;     // device layout: crops | bg_idx | top | left | apply
-    uint8_t *hpar = fg_pinned ? hp : hp + o;
-    if (!fg_pinned) std::memcpy(hp, h_src, fg_bytes);
-    std::memcpy(hpar, h_bg_idx, (size_t)B * 4);
-    std::memcpy(hpar + (size_t)B * 4, h_top, (size_t)B * 4);
-    std::memcpy(hpar + (size_t)B * 8, h_left, (size_t)B * 4);
-    std::memcpy(hpar + (size_t)B * 12, h_apply, (size_t)B);
-    if (fg_pinned) {
-        BGD_CUDA_TRY(cudaMemcpyAsync(dp_, h_src, fg_bytes, cudaMemcpyHostToDevice, s));
-        BGD_CUDA_TRY(cudaMemcpyAsync(dp_ + o, hpar, (size_t)B * 13, cudaMemcpyHostToDevice, s));
-    } else {
-        BGD_CUDA_TRY(cudaMemcpyAsync(dp_, hp, o + (size_t)B * 13, cudaMemcpyHostToDevice, s));
-    }
-    const int32_t *d_idx = reinterpret_cast<const int32_t *>(dp_ + o);
-    if (int rc = launch_resize_blend(dp_, src_bytes, h_geom, B, T, H, W, d_bg_pool, false, P, Hb, Wb, d_idx, d_idx + B,
-                                     d_idx + 2 * B, dp_ + o + (size_t)B * 12, d_fg_lut, h_bg_mean, h_bg_std, alpha, layout,
-                                     BGD_OUT_F32, d_out, s))
+    StagedBlend g;
+    if (int rc = stage_host_blend("bgmix_resize", h_src, (size_t)src_bytes, B, H, W, P, Hb, Wb, h_bg_idx, h_top, h_left, h_apply,
+                                  device, &g))
         return rc;
-    if (h_checksum) {
-        double *d_sum = reinterpret_cast<double *>(st.d_out[0]);
-        if (int rc = launch_sum_f32(d_out, (int64_t)B * T * 3 * H * W, d_sum, s)) return rc;
-        BGD_CUDA_TRY(cudaMemcpyAsync(st.h_out[0], d_sum, sizeof(double), cudaMemcpyDeviceToHost, s));
-    }
-    BGD_CUDA_TRY(cudaStreamSynchronize(s));
-    if (h_checksum) std::memcpy(h_checksum, st.h_out[0], sizeof(double));
-    return BGD_OK;
+    if (int rc = launch_resize_blend(g.fg, src_bytes, h_geom, B, T, H, W, d_bg_pool, false, P, Hb, Wb, g.bg_idx, g.top, g.left,
+                                     g.apply, d_fg_lut, h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out, g.stream))
+        return rc;
+    return finish_host_blend(d_out, B * T * 3 * H * W, h_checksum, g.stream);
 }
 
 int bgd_ragged_pack_u8(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_segments, int64_t n, uint8_t *d_out,

@@ -308,6 +308,18 @@ def _out_shape(B: int, T: int, H: int, W: int, layout: str) -> tuple:
     return {"NTCHW": (B, T, 3, H, W), "NCTHW": (B, 3, T, H, W), "NTHWC": (B, T, H, W, 3)}[layout]
 
 
+def _check_draws(name: str, B: int, dev, bg_idx, top, left, apply) -> None:
+    """The per-sample draws of a blend: int32 ``bg_idx`` / ``top`` / ``left`` and uint8 ``apply``, each ``[B]`` on ``dev``."""
+    for nm, t, dt in (("bg_idx", bg_idx, torch.int32), ("top", top, torch.int32), ("left", left, torch.int32),
+                      ("apply", apply, torch.uint8)):
+        _require(t.dtype == dt and t.dim() == 1 and t.shape[0] == B and t.device == dev, f"{name}: {nm} must be {dt} [B] on {dev}")
+
+
+def _check_lut(name: str, lut, dev) -> None:
+    _require(lut.dtype == torch.float32 and tuple(lut.shape) == (3, 256) and lut.device == dev,
+             f"{name}: fg_lut must be float32 [3, 256] on the device")
+
+
 @torch.library.custom_op("bgdebias::bgmix_blend", mutates_args=(), device_types="cuda")
 def bgmix_blend(fg: torch.Tensor, bg_pool: torch.Tensor, bg_idx: torch.Tensor, top: torch.Tensor,
                 left: torch.Tensor, apply: torch.Tensor, fg_lut: torch.Tensor, bg_mean: torch.Tensor,
@@ -320,12 +332,8 @@ def bgmix_blend(fg: torch.Tensor, bg_pool: torch.Tensor, bg_idx: torch.Tensor, t
     B, T, H, W, _ = fg.shape
     P, _, Hb, Wb = bg_pool.shape
     dev = fg.device
-    for name, t, dt in (("bg_idx", bg_idx, torch.int32), ("top", top, torch.int32), ("left", left, torch.int32),
-                        ("apply", apply, torch.uint8)):
-        _require(t.dtype == dt and t.dim() == 1 and t.shape[0] == B, f"bgmix_blend: {name} must be {dt} [B]")
-        _require(t.device == dev, f"bgmix_blend: {name} must be on {dev}")
-    _require(fg_lut.dtype == torch.float32 and tuple(fg_lut.shape) == (3, 256) and fg_lut.device == dev,
-             "bgmix_blend: fg_lut must be float32 [3, 256] on the device")
+    _check_draws("bgmix_blend", B, dev, bg_idx, top, left, apply)
+    _check_lut("bgmix_blend", fg_lut, dev)
     _require(bg_pool.device == dev, "bgmix_blend: bg_pool must be on the same device as fg")
     fg, bg_pool = fg.contiguous(), bg_pool.contiguous()
     bg_idx, top, left, apply, fg_lut = (x.contiguous() for x in (bg_idx, top, left, apply, fg_lut))
@@ -353,9 +361,7 @@ def _check_ragged(name, B, dev, pool_bytes, slots, tables, bg_idx, top, left, ap
     _require(slots.dtype == torch.uint8 and slots.dim() == 1 and slots.numel() % 40 == 0 and slots.numel() > 0,
              f"{name}: slots must be the uint8 view of a bgd_ragged_slot table (40 bytes per image)")
     _require(tables.dtype == torch.int32 and tables.dim() == 1, f"{name}: tables must be int32")
-    for nm, t, dt in (("bg_idx", bg_idx, torch.int32), ("top", top, torch.int32), ("left", left, torch.int32),
-                      ("apply", apply, torch.uint8)):
-        _require(t.dtype == dt and t.dim() == 1 and t.shape[0] == B and t.device == dev, f"{name}: {nm} must be {dt} [B] on {dev}")
+    _check_draws(name, B, dev, bg_idx, top, left, apply)
     for nm, t in (("pool_bytes", pool_bytes), ("slots", slots), ("tables", tables)):
         _require(t.device == dev, f"{name}: {nm} must be on {dev}")
     _require(slots.data_ptr() % 8 == 0, f"{name}: slots must be 8-byte aligned")
@@ -371,8 +377,7 @@ def bgmix_blend_ragged(fg: torch.Tensor, pool_bytes: torch.Tensor, slots: torch.
     B, T, H, W, _ = fg.shape
     dev = fg.device
     _check_ragged("bgmix_blend_ragged", B, dev, pool_bytes, slots, tables, bg_idx, top, left, apply)
-    _require(fg_lut.dtype == torch.float32 and tuple(fg_lut.shape) == (3, 256) and fg_lut.device == dev,
-             "bgmix_blend_ragged: fg_lut must be float32 [3, 256] on the device")
+    _check_lut("bgmix_blend_ragged", fg_lut, dev)
     fg = fg.contiguous()
     bg_idx, top, left, apply, fg_lut, pool_bytes, slots, tables = (x.contiguous() for x in (bg_idx, top, left, apply, fg_lut, pool_bytes, slots, tables))
     out = torch.empty(_out_shape(B, T, H, W, layout), dtype=out_dt, device=dev)
@@ -403,7 +408,7 @@ def bgmix_blend_ragged_normfg(fg_norm: torch.Tensor, pool_bytes: torch.Tensor, s
     _check_ragged("bgmix_blend_ragged_normfg", B, dev, pool_bytes, slots, tables, bg_idx, top, left, apply)
     fg_norm = fg_norm.contiguous()
     bg_idx, top, left, apply, pool_bytes, slots, tables = (x.contiguous() for x in (bg_idx, top, left, apply, pool_bytes, slots, tables))
-    out = torch.empty((B, T, 3, H, W) if layout == "NTCHW" else (B, 3, T, H, W), dtype=torch.float32, device=dev)
+    out = torch.empty(_out_shape(B, T, H, W, layout), dtype=torch.float32, device=dev)
     with torch.cuda.device(dev):
         _cabi.check(_cabi.lib().bgd_bgmix_blend_ragged_normfg_f32(
             fg_norm.data_ptr(), B, T, H, W, pool_bytes.data_ptr(), slots.data_ptr(), slots.numel() // 40, tables.data_ptr(),
@@ -415,7 +420,7 @@ def bgmix_blend_ragged_normfg(fg_norm: torch.Tensor, pool_bytes: torch.Tensor, s
 @bgmix_blend_ragged_normfg.register_fake
 def _(fg_norm, pool_bytes, slots, tables, bg_idx, top, left, apply, bg_mean, bg_std, alpha, layout):
     B, T, _, H, W = fg_norm.shape
-    return fg_norm.new_empty((B, T, 3, H, W) if layout == "NTCHW" else (B, 3, T, H, W))
+    return fg_norm.new_empty(_out_shape(B, T, H, W, layout))
 
 
 # --------------------------------------------------------------------------- #
@@ -480,12 +485,8 @@ def bgmix_resize_blend(src: torch.Tensor, geom: torch.Tensor, T: int, H: int, W:
     out_dt = _out_spec("bgmix_resize_blend", layout, out_dtype)
     P, _, Hb, Wb = bg_pool.shape
     dev = src.device
-    for name, t, dt in (("bg_idx", bg_idx, torch.int32), ("top", top, torch.int32), ("left", left, torch.int32),
-                        ("apply", apply, torch.uint8)):
-        _require(t.dtype == dt and t.dim() == 1 and t.shape[0] == B and t.device == dev,
-                 f"bgmix_resize_blend: {name} must be {dt} [B] on {dev}")
-    _require(fg_lut.dtype == torch.float32 and tuple(fg_lut.shape) == (3, 256) and fg_lut.device == dev,
-             "bgmix_resize_blend: fg_lut must be float32 [3, 256] on the device")
+    _check_draws("bgmix_resize_blend", B, dev, bg_idx, top, left, apply)
+    _check_lut("bgmix_resize_blend", fg_lut, dev)
     _require(bg_pool.device == dev, "bgmix_resize_blend: bg_pool must be on the same device as src")
     bg_pool = bg_pool.contiguous()
     bg_idx, top, left, apply, fg_lut = (x.contiguous() for x in (bg_idx, top, left, apply, fg_lut))
@@ -536,15 +537,11 @@ def bgmix_blend_normfg(fg_norm: torch.Tensor, bg_pool: torch.Tensor, bg_idx: tor
     B, T, _, H, W = fg_norm.shape
     P, _, Hb, Wb = bg_pool.shape
     dev = fg_norm.device
-    for name, t, dt in (("bg_idx", bg_idx, torch.int32), ("top", top, torch.int32), ("left", left, torch.int32),
-                        ("apply", apply, torch.uint8)):
-        _require(t.dtype == dt and t.dim() == 1 and t.shape[0] == B and t.device == dev,
-                 f"bgmix_blend_normfg: {name} must be {dt} [B] on {dev}")
+    _check_draws("bgmix_blend_normfg", B, dev, bg_idx, top, left, apply)
     _require(bg_pool.device == dev, "bgmix_blend_normfg: bg_pool must be on the same device as fg_norm")
     fg_norm, bg_pool = fg_norm.contiguous(), bg_pool.contiguous()
     bg_idx, top, left, apply = (x.contiguous() for x in (bg_idx, top, left, apply))
-    shape = (B, T, 3, H, W) if layout == "NTCHW" else (B, 3, T, H, W)
-    out = torch.empty(shape, dtype=torch.float32, device=dev)
+    out = torch.empty(_out_shape(B, T, H, W, layout), dtype=torch.float32, device=dev)
     with torch.cuda.device(dev):
         _cabi.check(_cabi.lib().bgd_bgmix_blend_normfg_f32(
             fg_norm.data_ptr(), B, T, H, W, bg_pool.data_ptr(), int(bg_pool.dtype == torch.uint8), P, Hb, Wb,
@@ -556,5 +553,4 @@ def bgmix_blend_normfg(fg_norm: torch.Tensor, bg_pool: torch.Tensor, bg_idx: tor
 @bgmix_blend_normfg.register_fake
 def _(fg_norm, bg_pool, bg_idx, top, left, apply, bg_mean, bg_std, alpha, layout):
     B, T, _, H, W = fg_norm.shape
-    shape = (B, T, 3, H, W) if layout == "NTCHW" else (B, 3, T, H, W)
-    return fg_norm.new_empty(shape)
+    return fg_norm.new_empty(_out_shape(B, T, H, W, layout))

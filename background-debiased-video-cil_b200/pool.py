@@ -9,6 +9,7 @@ the pool is index ``i`` of ``bg_files`` -- the reference's ``bg_idx``.
 """
 from __future__ import annotations
 
+import os
 from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple
 
 import numpy as np
@@ -35,12 +36,19 @@ def resize_like_reference(img_chw: torch.Tensor, size: Optional[int]) -> torch.T
     return Resize(size)(img)
 
 
+def _all_gather_obj(obj, world: int, group) -> list:
+    """``all_gather_object`` over ``group``: ``obj`` of every rank, in rank order."""
+    import torch.distributed as dist
+    out: list = [None] * world
+    dist.all_gather_object(out, obj, group=group)
+    return out
+
+
 def _map_in_order(fn, items, workers: Optional[int] = None) -> list:
     """``[fn(x) for x in items]`` on a small thread pool (JPEG decode and torch's resize release the GIL); a pool of
     13,320 UCF101 backgrounds takes ~50 s to decode + resize on one thread."""
     items = list(items)
     if workers is None:
-        import os
         workers = max(1, min(16, len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1)))
     if workers <= 1 or len(items) < 8:
         return [fn(x) for x in items]
@@ -304,9 +312,7 @@ class BackgroundPool:
         backgrounds): every rank learns ``[(name, owner_rank, slot_on_owner), ...]`` in rank order -- the global
         pool index -- while the pixels stay sharded where they were extracted."""
         import torch.distributed as dist
-        world = dist.get_world_size(group)
-        names_per_rank: List[Optional[list]] = [None] * world
-        dist.all_gather_object(names_per_rank, list(local_names), group=group)
+        names_per_rank = _all_gather_obj(list(local_names), dist.get_world_size(group), group)
         return [(n, r, i) for r, per in enumerate(names_per_rank) for i, n in enumerate(per)]
 
     # ---- one collective: assemble the pool from per-rank shards (SURVEY.md section 8e) ----------
@@ -323,8 +329,7 @@ class BackgroundPool:
         collective alone (the name exchange before it is host work)."""
         import torch.distributed as dist
         world = dist.get_world_size(group)
-        names_per_rank: List[Optional[list]] = [None] * world
-        dist.all_gather_object(names_per_rank, list(local_names), group=group)
+        names_per_rank = _all_gather_obj(list(local_names), world, group)
         counts = [len(n) for n in names_per_rank]
         if local_bgs.shape[0] != len(local_names):
             raise ValueError("one name per local background")
@@ -359,8 +364,7 @@ def all_gather_ragged(local_names: Sequence[str], local: "RaggedPool", group=Non
     meta = [(str(n), int(s["offset"]), int(s["h"]), int(s["w"])) for n, s in zip(local_names, local.slots)]
     if len(meta) != len(local):
         raise ValueError("one name per local background")
-    metas: List[Optional[list]] = [None] * world
-    dist.all_gather_object(metas, (int(local.used), meta), group=group)
+    metas = _all_gather_obj((int(local.used), meta), world, group)
     max_bytes = (max(u for u, _ in metas) + 15) & ~15
     out = RaggedPool(local.bg_resize, local.device)
     if max_bytes == 0:
@@ -388,6 +392,13 @@ def gather_extracted_backgrounds(output_dir, image_suffix: str = ".jpg", bg_resi
     of what the reference mixes (libs/loader/comix_loader.py:130), so the raw medians are not gathered -- and the
     pixels + names are all-gathered over NCCL / NVLink into a pool resident on every GPU.  Returns
     ``(paths, RaggedPool)``: the same index and pixels as decoding the whole directory on one rank."""
+    mine, local = _decode_my_split(output_dir, image_suffix, bg_resize, device, group)
+    return all_gather_ragged(mine, local, group)
+
+
+def _decode_my_split(output_dir, image_suffix: str, bg_resize: Optional[int], device, group) -> Tuple[List[str], RaggedPool]:
+    """This rank's contiguous split of the sorted JPEGs of ``output_dir`` (extract_background.py:128-133) and their decode
+    with ``torchvision.io.read_image(mode=RGB)`` into a :class:`RaggedPool` on ``device``."""
     import pathlib
     import torch.distributed as dist
     from torchvision.io import ImageReadMode, read_image
@@ -397,7 +408,7 @@ def gather_extracted_backgrounds(output_dir, image_suffix: str = ".jpg", bg_resi
     mine = contiguous_splits(files, world)[rank] if files else []
     local = RaggedPool(bg_resize, device)
     local.append(_map_in_order(lambda f: read_image(f, mode=ImageReadMode.RGB), mine))
-    return all_gather_ragged(mine, local, group)
+    return mine, local
 
 
 def _pad16(n):
@@ -504,6 +515,10 @@ class ShardedPool:
                              "not a multiple of 16: a sharded pool needs 16-byte aligned images (build it with "
                              "RaggedPool.append)")
         self.nbytes = 3 * self.h * self.w
+        self._row_of: Dict[str, int] = {}                           # name, and its realpath -> global index
+        for i, n in enumerate(self.names):
+            self._row_of.setdefault(n, i)
+            self._row_of.setdefault(os.path.realpath(n), i)
         self._hw: Dict[Tuple[int, int], Tuple[int, int]] = {}      # native -> resized size; fills the tables for every size
         for hw in set(zip(self.h.tolist(), self.w.tolist())):
             s = local.make_slot(0, *hw)
@@ -521,8 +536,7 @@ class ShardedPool:
             raise ValueError("one name per local background")
         world, rank = dist.get_world_size(group), dist.get_rank(group)
         meta = [(str(n), int(s["h"]), int(s["w"])) for n, s in zip(names, ragged.slots)]
-        metas: List[Optional[list]] = [None] * world
-        dist.all_gather_object(metas, meta, group=group)
+        metas = _all_gather_obj(meta, world, group)
         rows = [(n, r, i, hh, ww) for r, per in enumerate(metas) for i, (n, hh, ww) in enumerate(per)]
         cols = list(zip(*rows)) if rows else [[]] * 5
         return cls(ragged, cols[0], cols[1], cols[2], cols[3], cols[4], rank, world, group)
@@ -534,6 +548,21 @@ class ShardedPool:
     def hw(self, i: int) -> Tuple[int, int]:
         """Size after Resize of global image ``i`` -- what RandomCrop draws its offsets from."""
         return self._hw[(int(self.h[i]), int(self.w[i]))]
+
+    def rows_of(self, paths: Sequence[str]) -> np.ndarray:
+        """int64 global index of every entry of ``paths``, each matched as given or after ``realpath`` (as ``bg_dir`` is,
+        comix_loader.py:61-68).  ``ValueError`` naming the first entry that is not in the index: a sharded pool mixes only the
+        backgrounds it was built from."""
+        rows = np.empty(len(paths), dtype=np.int64)
+        for k, p in enumerate(paths):
+            i = self._row_of.get(p)
+            if i is None:
+                i = self._row_of.get(os.path.realpath(p))
+            if i is None:
+                raise ValueError(f"background {p!r} of bg_files is not in the sharded pool's index; a sharded pool mixes "
+                                 "only the extracted backgrounds it was built from")
+            rows[k] = i
+        return rows
 
     @property
     def resident_bytes(self) -> int:
@@ -547,12 +576,15 @@ class ShardedPool:
         app = torch.as_tensor(apply).tolist()
         return list(dict.fromkeys(int(g) for g, a in zip(idx, app) if a))
 
+    def _check_requests(self, requests: Sequence[int], who: str = "") -> None:
+        bad = [g for g in requests if not 0 <= g < len(self)]
+        if bad:
+            raise ValueError(f"{who}background {bad[0]} is outside the {len(self)}-image index")
+
     def route(self, requests: Sequence[Sequence[int]]) -> ShardRoute:
         """:func:`route_requests` for this rank."""
         for r, req in enumerate(requests):
-            bad = [g for g in req if not 0 <= g < len(self)]
-            if bad:
-                raise ValueError(f"rank {r} requests background {bad[0]}, outside the {len(self)}-image index")
+            self._check_requests(req, f"rank {r}: ")
         return route_requests(requests, self.owner, self.slot, self.nbytes, self.rank, self.local.slots["offset"])
 
     def pack(self, route: ShardRoute) -> torch.Tensor:
@@ -563,10 +595,18 @@ class ShardedPool:
 
     def assemble(self, recv: torch.Tensor, requests: Sequence[int], route: ShardRoute) -> RaggedPool:
         """The per-batch pool over the receive buffer: image ``k`` is ``requests[k]`` (this rank's requests)."""
+        return self._batch_pool(recv, route.recv_offsets, requests)
+
+    def _batch_pool(self, data: torch.Tensor, offsets: Sequence[int], requests: Sequence[int]) -> RaggedPool:
+        """The per-batch pool over ``data``: image ``k`` is global image ``requests[k]`` at byte ``offsets[k]``.  The slot table
+        travels from pinned memory, so building the pool never makes the host wait for the device."""
         batch = RaggedPool(self.bg_resize, self.device, tables=self.tables)
-        batch.data, batch.used = recv, int(recv.numel())
-        slots = [self.local.make_slot(int(o), int(self.h[g]), int(self.w[g])) for o, g in zip(route.recv_offsets, requests)]
-        batch.slots = np.array(slots, dtype=SLOT_DTYPE) if slots else np.zeros(0, dtype=SLOT_DTYPE)
+        batch.data, batch.used = data, int(data.numel())
+        if len(requests):
+            batch.slots = np.array([self.local.make_slot(int(o), int(self.h[g]), int(self.w[g])) for o, g in zip(offsets, requests)],
+                                   dtype=SLOT_DTYPE)
+            raw = torch.from_numpy(batch.slots.view(np.uint8).reshape(-1))
+            batch._slots_dev = raw.pin_memory().to(self.device, non_blocking=True)
         return batch
 
     def fetch(self, bg_idx, apply) -> Tuple[RaggedPool, torch.Tensor]:
@@ -587,8 +627,7 @@ class ShardedPool:
         queued on the current stream (e.g. the previous step's backward) has finished.  The replicated pool never waits."""
         import torch.distributed as dist
         mine = self.requests_of(bg_idx, apply)
-        requests: List[Optional[list]] = [None] * self.world
-        dist.all_gather_object(requests, mine, group=self.group)
+        requests = _all_gather_obj(mine, self.world, self.group)
         route = self.route(requests)
         recv = torch.empty(int(sum(route.recv_splits)), dtype=torch.uint8, device=self.device)
         if any(requests):                                  # every rank sees the same matrix: all skip or none does
@@ -681,7 +720,6 @@ class PeerPool:
         when the ranks are on different hosts, when a buffer cannot be exported (``expandable_segments``, the
         ``cudaMallocAsync`` backend) or when a peer cannot be mapped."""
         import ctypes
-        import torch.distributed as dist
         from . import _cabi
         local, rank, group = sharded.local, sharded.rank, sharded.group
         dev = sharded.device if sharded.device.index is not None else torch.device("cuda", torch.cuda.current_device())
@@ -697,8 +735,7 @@ class PeerPool:
                 meta.update(handle=handle.raw, offset=int(off.value))
             except (ValueError, _cabi.BgdError) as e:
                 meta["error"] = str(e)
-        metas: List[Optional[dict]] = [None] * sharded.world
-        dist.all_gather_object(metas, meta, group=group)
+        metas = _all_gather_obj(meta, sharded.world, group)
         check_peer_meta(metas)
         mapped: Dict[int, int] = {}
         error = None
@@ -712,9 +749,7 @@ class PeerPool:
                 error = f"rank {rank} (device {meta['uuid']}) cannot map the shard of rank {r} (device {m['uuid']}): {e}"
                 break
             mapped[r] = int(base.value)
-        errors: List[Optional[str]] = [None] * sharded.world
-        dist.all_gather_object(errors, error, group=group)
-        failed = [e for e in errors if e is not None]
+        failed = [e for e in _all_gather_obj(error, sharded.world, group) if e is not None]
         if failed:
             _close_mappings(mapped, dev)
             raise ValueError(f"{failed[0]}; {_USE_FETCH}")
@@ -739,18 +774,10 @@ class PeerPool:
             raise RuntimeError("the local shard was reallocated or appended to after PeerPool.open: peers would read a stale "
                                "mapping; close() the PeerPool before changing a shard, then open a new one")
         mine = sp.requests_of(bg_idx, apply)
-        bad = [g for g in mine if not 0 <= g < len(sp)]
-        if bad:
-            raise ValueError(f"background {bad[0]} is outside the {len(sp)}-image index")
+        sp._check_requests(mine)
         segments, dst, total = peer_segments(mine, sp.owner, self.src_offset, sp.nbytes)
-        batch = RaggedPool(sp.bg_resize, self.device, tables=sp.tables)
-        batch.data = torch.ops.bgdebias.ragged_gather(self.bases, self.base_bytes, torch.from_numpy(segments), total)
-        batch.used = total
-        if mine:
-            batch.slots = np.array([sp.local.make_slot(int(o), int(sp.h[g]), int(sp.w[g])) for o, g in zip(dst, mine)],
-                                   dtype=SLOT_DTYPE)
-            raw = torch.from_numpy(batch.slots.view(np.uint8).reshape(-1))
-            batch._slots_dev = raw.pin_memory().to(self.device, non_blocking=True)
+        data = torch.ops.bgdebias.ragged_gather(self.bases, self.base_bytes, torch.from_numpy(segments), total)
+        batch = sp._batch_pool(data, dst, mine)
         return batch, sp.sample_slots(bg_idx, apply, mine).pin_memory()     # pinned: its upload does not wait either
 
     def close(self) -> None:
@@ -779,15 +806,7 @@ def shard_extracted_backgrounds(output_dir, image_suffix: str = ".jpg", bg_resiz
     decodes its own files with ``torchvision.io.read_image(mode=RGB)`` and KEEPS them; only names and sizes are all-gathered.
     Returns ``(paths, ShardedPool)`` with ``paths[i]`` the file of global index ``i`` (the same list, in the same order, as
     :func:`gather_extracted_backgrounds` returns)."""
-    import pathlib
-    import torch.distributed as dist
-    from torchvision.io import ImageReadMode, read_image
-    from .shard import contiguous_splits
-    world, rank = dist.get_world_size(group), dist.get_rank(group)
-    files = sorted(str(f) for f in pathlib.Path(output_dir).glob("*" + image_suffix))
-    mine = contiguous_splits(files, world)[rank] if files else []
-    local = RaggedPool(bg_resize, device)
-    local.append(_map_in_order(lambda f: read_image(f, mode=ImageReadMode.RGB), mine))
+    mine, local = _decode_my_split(output_dir, image_suffix, bg_resize, device, group)
     sharded = ShardedPool.from_local(mine, local, group)
     return list(sharded.names), sharded
 

@@ -180,20 +180,43 @@ def test_device_finish_peer_equals_replicated(env, tmp_path, fg_form, prob):
             assert torch.equal(_bits(po[f]["imgs"]), _bits(ro[f]["imgs"])), (rank, f)
 
 
-def test_attaching_one_pool_detaches_the_other(env, tmp_path):
+def test_device_finish_reads_through_the_pool_attached_last(env, tmp_path):
+    """device_finish brings a batch's images through the pool attached last: PeerPool.gather, ShardedPool.fetch, or neither
+    (the replica of attach_pool)."""
     ops, _cabi, pool = env
     from bgdebias_b200 import comix_loader as cl
     imgs = _images(np.random.default_rng(1), SIZES[:2])
     peers, names = _peers(pool, imgs, [1, 1], [os.path.realpath(tmp_path / f"bg{i}.jpg") for i in range(2)])
-    ds = _dataset(cl, tmp_path, [(224, 224)], 2)
+    calls = []
+
+    def counted(what, fn):
+        def call(*args):
+            calls.append(what)
+            return fn(*args)
+        return call
+
+    for r, peer in enumerate(peers):
+        gather = peer.gather
+        peer.gather = counted(f"gather{r}", gather)
+        peer.sharded.fetch = counted(f"fetch{r}", gather)     # the real fetch is a collective; gather returns the same batch
+
+    ds = _dataset(cl, tmp_path, [(224, 224)], 2, prob=1.0)
+
+    def finish():
+        calls.clear()
+        ds.bg_files = [names[0]]
+        ds.device_finish(ds.host_collate([ds[0]]))
+        return list(calls)
+
     ds.attach_peer_pool(names, peers[0])
-    assert ds._peer is peers[0] and ds._sharded is peers[0].sharded
+    assert finish() == ["gather0"]
     ds.attach_sharded_pool(names, peers[0].sharded)
-    assert ds._peer is None
+    assert finish() == ["fetch0"]
     ds.attach_peer_pool(names, peers[0])
     ds.attach_pool(names[:1], peers[0].sharded.local)
-    assert ds._peer is None and ds._sharded is None
+    assert finish() == []
     ds.attach_peer_pool(names, peers[1])
+    assert finish() == ["gather1"]
     ds.bg_files = [names[1], str(tmp_path / "not_there.jpg")]
     assert ds._bg_hw(0) == peers[1].sharded.hw(1)
     with pytest.raises(ValueError, match="not_there.jpg"):

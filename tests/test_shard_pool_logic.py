@@ -117,12 +117,14 @@ def test_dataset_rejects_a_name_outside_the_index(tmp_path):
     ds.attach_sharded_pool(names, sp)
     ds.bg_files = [names[2], names[1], names[2], names[0]]     # a CIL union with a repeat
     assert [ds._bg_hw(i) for i in range(4)] == [(256, 256), resized_hw(240, 427, 256), (256, 256), resized_hw(240, 320, 256)]
-    assert ds._sharded_rows().tolist() == [2, 1, 2, 0]
+    assert sp.rows_of(ds.bg_files).tolist() == [2, 1, 2, 0]
     missing = str(bg / "not_extracted.jpg")
     ds.bg_files = ds.bg_files + [missing]
     with pytest.raises(ValueError, match="not_extracted.jpg"):
         ds._bg_hw(4)
     with pytest.raises(ValueError, match="not_extracted.jpg"):
-        ds._sharded_rows()
+        sp.rows_of(ds.bg_files)
+    with pytest.raises(ValueError, match="index order"):
+        ds.attach_sharded_pool(names[::-1], sp)
     with pytest.raises(ValueError):
         ShardedPool(local, names, [0, 1, 1], [0, 0, 1], [240, 240, 256], [320, 427, 256], rank=0, world=2)   # 1 != 2 local
