@@ -90,6 +90,8 @@ SIGNATURES = {
                                               _vp, _c.c_int, _c.c_int64, _c.c_int64, _c.c_int64,
                                               _vp, _vp, _vp, _vp, _vp, _f32p, _f32p, _c.c_double, _c.c_int, _c.c_int, _vp,
                                               _vp]),
+    "bgd_resize_crop_normalize_out": (_c.c_int, [_vp, _c.c_int64, _i64p, _c.c_int64, _c.c_int64, _c.c_int64, _c.c_int64,
+                                                 _vp, _c.c_int, _c.c_int, _vp, _vp]),
     "bgd_ragged_pack_u8": (_c.c_int, [_vp, _c.c_int64, _i64p, _c.c_int64, _vp, _c.c_int64, _vp]),
     "bgd_ragged_gather_u8": (_c.c_int, [_vp, _i64p, _c.c_int64, _i64p, _c.c_int64, _vp, _c.c_int64, _vp]),
     "bgd_ipc_export": (_c.c_int, [_vp, _c.c_char_p, _i64p]),

@@ -25,6 +25,11 @@ reference's fp32 bytes.  The pipeline may also stop before its last ``Resize((22
 mixed sizes are packed by ``host_collate`` and resized (cv2 INTER_LINEAR, bit for bit) inside the blend launch.
 ``device_finish(batch, dtype=torch.bfloat16, memory_format=torch.channels_last)`` hands a bf16-autocast model its input
 directly: the blend's fp32 result rounded once to bf16, stored channels-last by the same launch.
+
+Evaluation datasets (``test_mode=True``: val, test, the herding feature pass, the NME class means) never mix.  With
+``device_mix=True`` their pipeline stops after ``RawFrameDecode`` and ``device_test_pipeline`` takes the steps it no longer
+runs -- ``Resize(scale=(-1, S))``, ``CenterCrop`` or ``ThreeCrop``, ``Normalize`` and ``FormatShape('NCHW')``, see
+:class:`EvalPipeline` -- which ``device_finish`` runs on the native-size uint8 frames in one launch.
 """
 from __future__ import annotations
 
@@ -121,7 +126,8 @@ class _RawframeBase:
         return self.pipeline(results)
 
     def prepare_test_frames(self, idx):
-        return self.prepare_train_frames(idx)
+        # the pipeline alone, as mmaction's RawframeDataset.prepare_test_frames: never a subclass's training-time mix
+        return _RawframeBase.prepare_train_frames(self, idx)
 
     def __getitem__(self, idx):
         return self.prepare_test_frames(idx) if self.test_mode else self.prepare_train_frames(idx)
@@ -161,12 +167,108 @@ def draw_crop(h: int, w: int, crop) -> tuple:
     return top, left
 
 
+class EvalPipeline:
+    """The tail of an evaluation pipeline that the device runs on decoded uint8 frames (``resize_crop_normalize``):
+
+        Resize(scale=(-1, S)) -> CenterCrop(c) | ThreeCrop(c) -> Normalize(mean, std) -> FormatShape('NCHW')
+
+    ``steps`` are the mmaction step dicts of these four, in this order, moved verbatim out of ``test_pipeline``.  Any other
+    step, or another form of these (``keep_ratio=False``, another interpolation, ``to_bgr=True``, ``TenCrop``, NCTHW, ...),
+    raises ``ValueError`` naming the step; such a config keeps its CPU pipeline.
+
+    The rules restate mmaction2 0.x ``mmaction/datasets/pipelines/augmentations.py`` (``Resize``, ``CenterCrop``,
+    ``ThreeCrop``, ``Normalize``) and ``formating.py`` (``FormatShape``), and mmcv 1.x ``mmcv/image/geometric.py``
+    (``rescale_size``, ``_scale_size``, ``imresize``); neither package is a dependency:
+
+    * Resize, ``keep_ratio=True``, bilinear: ``scale=(-1, S)`` or ``(S, -1)`` becomes ``(inf, S)``, and
+      ``mmcv.rescale_size((w, h), (inf, S))`` gives ``f = S / min(h, w)``, ``(Wr, Hr) = (int(w * f + 0.5), int(h * f + 0.5))``;
+      pixels are ``cv2.resize(img, (Wr, Hr), interpolation=cv2.INTER_LINEAR)``.  240x320 -> 256x341, 320x240 -> 341x256.
+    * CenterCrop: ``left = (Wr - cw) // 2``, ``top = (Hr - ch) // 2``.
+    * ThreeCrop: needs ``ch == Hr`` or ``cw == Wr`` (mmaction asserts it).  If ``ch == Hr``: ``step = (Wr - cw) // 2`` and the
+      windows start at left 0, ``2 * step``, ``step`` in that order (so 85 pixels of slack give a right crop at 84); else the
+      same vertically.  The output is crop-major: crop k's frames follow crop k-1's.
+    * ``crop_size``: an int or ``(cw, ch)`` (mmaction's ``_pair`` order).  A crop larger than the resized frame raises.
+    * Normalize, ``to_bgr=False``: :func:`ops.make_fg_lut` of ``(mean, std)``, as the training path normalises.
+    * FormatShape('NCHW'): ``[K * T, 3, ch, cw]`` per clip.
+    """
+
+    def __init__(self, steps: Sequence[dict]):
+        steps = [dict(s) for s in steps]
+        expected = (('Resize',), ('CenterCrop', 'ThreeCrop'), ('Normalize',), ('FormatShape',))
+        for i, step in enumerate(steps):
+            if i >= len(expected) or step.get('type') not in expected[i]:
+                raise ValueError(f"device_test_pipeline: step {i}, {step.get('type')!r}, has no device form (expected "
+                                 "Resize, CenterCrop or ThreeCrop, Normalize, FormatShape, in this order)")
+        if len(steps) < len(expected):
+            raise ValueError(f"device_test_pipeline: the {' or '.join(expected[len(steps)])} step is missing")
+        resize, crop, norm, fmt = steps
+        self._only(resize, scale=None, keep_ratio=True, interpolation='bilinear', lazy=False)
+        scale = resize.get('scale')
+        if not (isinstance(scale, (tuple, list)) and len(scale) == 2 and min(scale) == -1 and max(scale) > 0
+                and all(isinstance(v, int) for v in scale)):
+            raise ValueError(f"Resize: only scale=(-1, S) or (S, -1) has a device form (got scale={scale!r})")
+        self.short_side = int(max(scale))
+        self._only(crop, crop_size=None, lazy=False)
+        cs = crop.get('crop_size')
+        cw, ch = (cs, cs) if isinstance(cs, int) else tuple(cs)
+        if not (isinstance(cw, int) and isinstance(ch, int) and cw > 0 and ch > 0):
+            raise ValueError(f"{crop['type']}: crop_size must be a positive int or (w, h) (got {cs!r})")
+        self.three, self.crop_hw = crop['type'] == 'ThreeCrop', (ch, cw)
+        self._only(norm, mean=None, std=None, to_bgr=False, adjust_magnitude=False)
+        if len(norm.get('mean', ())) != 3 or len(norm.get('std', ())) != 3:
+            raise ValueError("Normalize: mean and std must have 3 values (RGB)")
+        self.mean, self.std = tuple(float(m) for m in norm['mean']), tuple(float(v) for v in norm['std'])
+        self._only(fmt, input_format=None, collapse=False)
+        if fmt.get('input_format') != 'NCHW':
+            raise ValueError(f"FormatShape: only input_format='NCHW' has a device form (got {fmt.get('input_format')!r})")
+
+    @staticmethod
+    def _only(step: dict, **allowed) -> None:
+        """Keys other than ``type`` must be in ``allowed``; those with a non-None value there must equal it."""
+        for k, v in step.items():
+            if k == 'type':
+                continue
+            if k not in allowed or (allowed[k] is not None and v != allowed[k]):
+                raise ValueError(f"{step['type']}: {k}={v!r} has no device form")
+
+    @property
+    def n_crops(self) -> int:
+        return 3 if self.three else 1
+
+    def windows(self, h: int, w: int) -> tuple:
+        """``(Hr, Wr, [(top, left), ...])`` for a native ``h x w`` frame: the resized size and every crop's window."""
+        f = self.short_side / min(h, w)
+        Wr, Hr = int(w * f + 0.5), int(h * f + 0.5)
+        ch, cw = self.crop_hw
+        if not self.three:
+            if ch > Hr or cw > Wr:
+                raise ValueError(f"CenterCrop: crop {ch}x{cw} is larger than the resized frame {Hr}x{Wr}")
+            return Hr, Wr, [((Hr - ch) // 2, (Wr - cw) // 2)]
+        if ch == Hr and cw <= Wr:
+            step = (Wr - cw) // 2
+            return Hr, Wr, [(0, 0), (0, 2 * step), (0, step)]
+        if cw == Wr and ch <= Hr:
+            step = (Hr - ch) // 2
+            return Hr, Wr, [(0, 0), (2 * step, 0), (step, 0)]
+        raise ValueError(f"ThreeCrop: crop {ch}x{cw} must span the height or the width of the resized frame {Hr}x{Wr}")
+
+    def geometry(self, fg_geom: torch.Tensor) -> torch.Tensor:
+        """int64 ``[B * K, 9]`` for ``resize_crop_normalize`` from the ``[B, 5]`` geometry of ``ops.pack_clips``: clip-major,
+        then crop, so that the ``[B * K, T, 3, ch, cw]`` output is ``[B, K * T, 3, ch, cw]``."""
+        rows = []
+        for q in fg_geom.tolist():
+            Hr, Wr, wins = self.windows(int(q[1]), int(q[2]))
+            rows += [q[:5] + [Hr, Wr, top, left] for top, left in wins]
+        return torch.tensor(rows, dtype=torch.int64).reshape(-1, 9)
+
+
 @_register(_DATASETS)
 class BackgroundMixDataset(_Base):
-    """Same signature as the reference class (libs/loader/comix_loader.py:16-45) plus three
+    """Same signature as the reference class (libs/loader/comix_loader.py:16-45) plus four
     keyword-only extensions: ``device`` (CUDA device of the pool and the blend), ``device_mix``
-    (see module docstring) and ``bg_reader`` (callable ``path -> uint8 [3,h,w]``, defaults to
-    ``torchvision.io.read_image(mode=RGB)`` as in the reference)."""
+    (see module docstring), ``bg_reader`` (callable ``path -> uint8 [3,h,w]``, defaults to
+    ``torchvision.io.read_image(mode=RGB)`` as in the reference) and ``device_test_pipeline`` (the
+    step dicts of :class:`EvalPipeline`, required by ``device_mix=True`` with ``test_mode=True``)."""
 
     def __init__(self,
                  ann_file,
@@ -198,7 +300,14 @@ class BackgroundMixDataset(_Base):
                  device='cuda',
                  device_mix=False,
                  bg_reader: Optional[Callable] = None,
+                 device_test_pipeline: Optional[Sequence[dict]] = None,
                  **kwargs):
+        if device_test_pipeline is not None and not (device_mix and test_mode):
+            raise ValueError("device_test_pipeline is the evaluation tail of device_mix=True with test_mode=True")
+        if device_mix and test_mode and device_test_pipeline is None:
+            raise ValueError("device_mix=True with test_mode=True needs device_test_pipeline: the Resize, crop, Normalize "
+                             "and FormatShape steps moved out of test_pipeline")
+        self._eval = EvalPipeline(device_test_pipeline) if device_test_pipeline is not None else None
         super().__init__(ann_file, pipeline, data_prefix, test_mode, filename_tmpl, with_offset, multi_class,
                          num_classes, start_index, modality, sample_by_class, power, dynamic_length, **kwargs)
         bg_dir = osp.realpath(bg_dir)                 # same reason as the reference, comix_loader.py:61-68
@@ -515,9 +624,18 @@ class BackgroundMixDataset(_Base):
         """``collate_fn`` for ``device_mix=True`` that is safe in DataLoader worker processes (no CUDA): stacks
         the uint8 clips ``[B,T,H,W,3]`` and the per-sample draws into host tensors.  Pair it with
         :meth:`device_finish` in the training process; with ``pin_memory=True`` the batch travels as uint8,
-        a quarter of the bytes of the reference's fp32 batch (libs/cil/cil.py:203-210)."""
-        clips = [torch.as_tensor(s['imgs']) for s in samples]
+        a quarter of the bytes of the reference's fp32 batch (libs/cil/cil.py:203-210).
+
+        Samples without draws (``test_mode=True``) make an evaluation batch: the native-size uint8 frames packed with
+        ``ops.pack_clips`` (sizes may differ per video) and ``label``, for the eval route of :meth:`device_finish`."""
+        clips = [torch.as_tensor(np.stack(s['imgs']) if isinstance(s['imgs'], (list, tuple)) else s['imgs']) for s in samples]
         out = {}
+        if 'bg_idx' not in samples[0]:
+            out['imgs'], out['fg_geom'] = ops.pack_clips(clips)
+            out['fg_frames'] = int(clips[0].shape[0])
+            if 'label' in samples[0]:
+                out['label'] = torch.stack([torch.as_tensor(s['label']) for s in samples])
+            return out
         if all(c.shape == clips[0].shape for c in clips):
             out['imgs'] = torch.stack(clips)
         else:
@@ -549,7 +667,13 @@ class BackgroundMixDataset(_Base):
                       memory_format: torch.memory_format = torch.contiguous_format) -> dict:
         """The GPU half of the ``device_mix=True`` path: turns a :meth:`host_collate` batch into the dict the
         reference's default_collate would hand the model (``imgs`` fp32 ``[B,T,3,H,W]`` on the device, ``label``,
-        ``randAug``, ``bg_idx``) with one fused launch.  ``dtype`` / ``memory_format``: see :meth:`mix_batch_on_device`."""
+        ``randAug``, ``bg_idx``) with one fused launch.  ``dtype`` / ``memory_format``: see :meth:`mix_batch_on_device`.
+
+        An evaluation batch (no draws) runs the dataset's :class:`EvalPipeline` instead, in one launch that reads neither
+        the background pool nor any file: ``imgs`` ``[B, K*T, 3, ch, cw]`` (K crops, crop-major, as mmaction's ThreeCrop and
+        FormatShape('NCHW') yield after default_collate) and ``label``."""
+        if 'bg_idx' not in batch:
+            return self._finish_eval(batch, layout, dtype, memory_format)
         out = {k: v for k, v in batch.items()
                if k not in ('imgs', 'bg_top', 'bg_left', 'bg_apply', 'fg_geom', 'fg_frames', 'bg_imgs', 'bg_slot')}
         if not self.back_ground_from_bg_dir and 'bg_imgs' not in batch:
@@ -560,6 +684,30 @@ class BackgroundMixDataset(_Base):
                                                batch['bg_apply'], layout=layout, fg_geom=batch.get('fg_geom'),
                                                fg_frames=batch.get('fg_frames'), bg_imgs=batch.get('bg_imgs'),
                                                bg_slot=batch.get('bg_slot'), dtype=dtype, memory_format=memory_format)
+        return out
+
+    def _finish_eval(self, batch: dict, layout: str, dtype: torch.dtype, memory_format: torch.memory_format) -> dict:
+        if self._eval is None:
+            raise ValueError("an evaluation batch (no mix draws) needs a dataset built with device_test_pipeline")
+        if layout != "NTCHW":
+            raise ValueError(f"evaluation batches are FormatShape('NCHW'): layout must be 'NTCHW' (got {layout!r})")
+        if memory_format not in (torch.contiguous_format, torch.channels_last):
+            raise ValueError(f"memory_format must be torch.contiguous_format or torch.channels_last (got {memory_format})")
+        ev, dev = self._eval, self.device
+        geom = ev.geometry(batch['fg_geom'])
+        B, K, T = batch['fg_geom'].shape[0], ev.n_crops, int(batch['fg_frames'])
+        ch, cw = ev.crop_hw
+        channels_last = memory_format == torch.channels_last
+        src = batch['imgs'].to(dev, non_blocking=True)
+        imgs = torch.ops.bgdebias.resize_crop_normalize(src, geom, T, ch, cw, self._lut(ev.mean, ev.std),
+                                                        "NTHWC" if channels_last else "NTCHW", dtype)
+        if channels_last:                                 # [B*K,T,H,W,3] -> logical [B,K*T,3,H,W]
+            imgs = imgs.view(B, K * T, ch, cw, 3).permute(0, 1, 4, 2, 3)
+        else:
+            imgs = imgs.view(B, K * T, 3, ch, cw)
+        out = {'imgs': imgs}
+        if 'label' in batch:
+            out['label'] = batch['label']
         return out
 
     def gpu_collate(self, samples: List[dict], dtype: torch.dtype = torch.float32,

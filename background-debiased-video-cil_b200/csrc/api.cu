@@ -741,6 +741,16 @@ int bgd_bgmix_resize_blend_out(const uint8_t *d_src, int64_t src_bytes, const in
                                static_cast<cudaStream_t>(stream));
 }
 
+int bgd_resize_crop_normalize_out(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t n, int64_t T,
+                                  int64_t H, int64_t W, const float *d_fg_lut, int layout, int out_dtype, void *d_out,
+                                  void *stream)
+{
+    DeviceProps dp;
+    if (int rc = current_device_props(&dp)) return rc;
+    return launch_resize_normalize(d_src, src_bytes, h_geom, n, T, H, W, d_fg_lut, layout, out_dtype, d_out,
+                                   static_cast<cudaStream_t>(stream));
+}
+
 int bgd_bgmix_blend_f32_host(const uint8_t *h_fg, int64_t B, int64_t T, int64_t H, int64_t W, const float *d_bg_pool,
                              int64_t P, int64_t Hb, int64_t Wb, const int32_t *h_bg_idx, const int32_t *h_top,
                              const int32_t *h_left, const uint8_t *h_apply, const float *d_fg_lut,

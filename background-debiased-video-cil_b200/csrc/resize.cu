@@ -17,6 +17,12 @@
 // plus a per-clip table (byte offset of the crop's first pixel, crop height/width, row and frame strides), so a crop can also
 // be addressed inside a full decoded frame without a host-side copy.
 //
+// The evaluation pipelines (Resize(scale=(-1, 256)) -> CenterCrop / ThreeCrop -> Normalize -> FormatShape('NCHW')) use the
+// windowed form of the table: an entry may also name the size Hr x Wr the clip is resized to and the H x W window at
+// (top, left) of that resized image it emits.  Cropping after the resize only selects destination rows and columns, so
+// the window's coefficients are entries top.. / left.. of the Hr / Wr tables; the resized image never exists.  Those
+// entries run resize_blend_kernel with the blend compiled out (BLEND = false).
+//
 // The coefficients depend on (source size, destination size, index) only: the host evaluates them once per distinct size
 // (float/double arithmetic exactly as above) into small tables that travel with the per-clip table.  A CTA owns a 32x8 tile of
 // output pixels of one clip, one thread per pixel: it reads its column entry and its row entry, then walks the T frames of the
@@ -28,7 +34,8 @@
 
 #include <algorithm>
 #include <cmath>
-#include <unordered_map>
+#include <map>
+#include <tuple>
 #include <vector>
 
 namespace bgd {
@@ -54,7 +61,7 @@ struct Coef {                  // one per destination column / row, built on the
 struct ClipGeom {              // one per clip, built on the host
     int64_t offset;            // bytes from d_src to the crop's first pixel of frame 0
     int64_t row_stride, frame_stride;
-    int32_t xtab, ytab;        // first entry of the clip's column / row coefficients in the Coef array
+    int32_t xtab, ytab;        // coefficients of the clip's output column / row 0 in the Coef array (window offset included)
 };
 
 struct TailParams {
@@ -164,7 +171,8 @@ __global__ void __launch_bounds__(kThreads) resize_u8_kernel(const TailParams pr
 
 // OutT: float, __nv_bfloat16 or __half.  IL (BGD_LAYOUT_NTHWC): the pixel's 3 channels are adjacent in the output; a
 // lane then stores 3 consecutive values per frame and a warp still covers whole 32-byte sectors (scalar stores).
-template <typename PoolT, typename OutT, bool IL>
+// BLEND = false: Resize -> Normalize -> FormatShape only; the pool, the draws and apply are never read (PoolT unused).
+template <typename PoolT, typename OutT, bool IL, bool BLEND>
 __global__ void __launch_bounds__(kThreads, kBlendMinBlocks) resize_blend_kernel(const TailParams prm)
 {
     __shared__ float s_lut[3 * 256];
@@ -177,9 +185,9 @@ __global__ void __launch_bounds__(kThreads, kBlendMinBlocks) resize_blend_kernel
     const ClipGeom g = prm.geom[b];
     const Taps t = make_taps(prm, g, x, y);
 
-    const bool apply = prm.apply[b] != 0;
+    const bool apply = BLEND && prm.apply[b] != 0;
     float bgw[3] = {0.f, 0.f, 0.f};                  // normalised background * alpha
-    if (apply) {
+    if constexpr (BLEND) if (apply) {
         // one pool image has fewer than 2^31 elements (checked on the host): only the image index needs 64 bits
         const int Hb = (int)prm.Hb, Wb = (int)prm.Wb, plane = Hb * Wb;
         int64_t idx = prm.bg_idx[b];
@@ -241,51 +249,60 @@ void fill_coefs(int src, int dst, bool columns, Coef *out)
     }
 }
 
-struct TableKey { int64_t src; bool columns; int32_t at; };
+struct TableKey { int64_t src, dst; bool columns; int32_t at; };
 
-// Validates the host geometry table [B][5] = {offset, h, w, row stride, frame stride} against the buffer, builds the
-// coefficient tables (one per distinct source size and axis) and uploads both: [ClipGeom x B][Coef x n].
-int upload_geom(const int64_t *h_geom, int64_t B, int64_t T, int64_t H, int64_t W, int64_t src_bytes, Workspace &ws,
+// Validates the host geometry table against the buffer, builds the coefficient tables (one per distinct source size,
+// destination size and axis) and uploads both: [ClipGeom x B][Coef x n].  cols = 5: rows {offset, h, w, row stride,
+// frame stride}, each clip resized to H x W.  cols = 9: the same five plus {Hr, Wr, top, left}, the clip resized to
+// Hr x Wr and the H x W window at (top, left) emitted; 5 columns are the case Hr = H, Wr = W, top = left = 0.
+int upload_geom(const int64_t *h_geom, int cols, int64_t B, int64_t T, int64_t H, int64_t W, int64_t src_bytes, Workspace &ws,
                 TailParams *prm, cudaStream_t stream)
 {
     std::vector<TableKey> tables;
-    std::unordered_map<int64_t, int32_t> index;            // 2 * source size + axis -> first entry
+    std::map<std::tuple<int64_t, int64_t, bool>, int32_t> index;     // (source size, destination size, axis) -> first entry
     std::vector<int32_t> xt(B), yt(B);
     int64_t n_coef = 0;
-    auto table_of = [&](int64_t src, bool columns) {
-        auto it = index.find(2 * src + (columns ? 1 : 0));
+    auto table_of = [&](int64_t src, int64_t dst, bool columns) {
+        auto it = index.find({src, dst, columns});
         if (it != index.end()) return it->second;
-        tables.push_back({src, columns, (int32_t)n_coef});
-        index.emplace(2 * src + (columns ? 1 : 0), (int32_t)n_coef);
-        n_coef += columns ? W : H;
+        tables.push_back({src, dst, columns, (int32_t)n_coef});
+        index.emplace(std::make_tuple(src, dst, columns), (int32_t)n_coef);
+        n_coef += dst;
         return tables.back().at;
     };
     for (int64_t b = 0; b < B; ++b) {
-        const int64_t *q = h_geom + b * 5;
+        const int64_t *q = h_geom + b * cols;
         const int64_t off = q[0], h = q[1], w = q[2], rs = q[3], fs = q[4];
+        const int64_t Hr = cols == 9 ? q[5] : H, Wr = cols == 9 ? q[6] : W, top = cols == 9 ? q[7] : 0, left = cols == 9 ? q[8] : 0;
         if (h < 1 || w < 1 || h > INT32_MAX / 4 || w > INT32_MAX / 4)
             return fail(BGD_ERR_INVALID, "resize: clip %lld has size %lldx%lld", (long long)b, (long long)h, (long long)w);
         if (off < 0 || rs < w * 3 || fs < 0)
             return fail(BGD_ERR_INVALID, "resize: clip %lld has a negative offset or a row stride below 3*w", (long long)b);
+        if (Hr < 1 || Wr < 1 || Hr > INT32_MAX / 4 || Wr > INT32_MAX / 4)
+            return fail(BGD_ERR_INVALID, "resize: clip %lld is resized to %lldx%lld", (long long)b, (long long)Hr, (long long)Wr);
+        if (top < 0 || left < 0 || top > Hr - H || left > Wr - W)
+            return fail(BGD_ERR_INVALID, "resize: clip %lld: the %lldx%lld window at (%lld, %lld) is not inside its %lldx%lld resized "
+                        "image", (long long)b, (long long)H, (long long)W, (long long)top, (long long)left, (long long)Hr,
+                        (long long)Wr);
         // the kernel reads tap PAIRS: a one-pixel-wide crop reads 6 bytes per row as well
         const int64_t end = off + (T - 1) * fs + (h - 1) * rs + std::max<int64_t>(w, 2) * 3;
         if (end > src_bytes)
             return fail(BGD_ERR_INVALID, "resize: clip %lld ends at byte %lld of a %lld-byte buffer", (long long)b,
                         (long long)end, (long long)src_bytes);
-        if (n_coef + H + W > INT32_MAX) return fail(BGD_ERR_INVALID, "resize: too many distinct clip sizes");
-        xt[b] = table_of(w, true);
-        yt[b] = table_of(h, false);
+        if (n_coef + Hr + Wr > INT32_MAX) return fail(BGD_ERR_INVALID, "resize: too many distinct clip sizes");
+        xt[b] = table_of(w, Wr, true) + (int32_t)left;
+        yt[b] = table_of(h, Hr, false) + (int32_t)top;
     }
     const size_t geom_bytes = (size_t)B * sizeof(ClipGeom), bytes = geom_bytes + (size_t)n_coef * sizeof(Coef);
     if (int rc = ws.acquire(bytes)) return rc;
     ClipGeom *hg = static_cast<ClipGeom *>(ws.h_pinned);
     Coef *hc = reinterpret_cast<Coef *>(static_cast<char *>(ws.h_pinned) + geom_bytes);
     for (int64_t b = 0; b < B; ++b) {
-        const int64_t *q = h_geom + b * 5;
+        const int64_t *q = h_geom + b * cols;
         hg[b].offset = q[0]; hg[b].row_stride = q[3]; hg[b].frame_stride = q[4];
         hg[b].xtab = xt[b]; hg[b].ytab = yt[b];
     }
-    for (const TableKey &k : tables) fill_coefs((int)k.src, (int)(k.columns ? W : H), k.columns, hc + k.at);
+    for (const TableKey &k : tables) fill_coefs((int)k.src, (int)k.dst, k.columns, hc + k.at);
     BGD_CUDA_TRY(cudaMemcpyAsync(ws.d_ptr, ws.h_pinned, bytes, cudaMemcpyHostToDevice, stream));
     prm->geom = static_cast<const ClipGeom *>(ws.d_ptr);
     prm->coef = reinterpret_cast<const Coef *>(static_cast<const char *>(ws.d_ptr) + geom_bytes);
@@ -310,6 +327,24 @@ dim3 tile_grid(int64_t B, int64_t H, int64_t W)
     return dim3((unsigned)((W + kTileW - 1) / kTileW), (unsigned)((H + kTileH - 1) / kTileH), (unsigned)B);
 }
 
+// Output strides of the fp32 / 16-bit kernels (the layout is validated by the caller).
+void set_out_strides(int layout, int64_t T, int64_t H, int64_t W, TailParams &prm)
+{
+    const int64_t HW = H * W;
+    if (layout == BGD_LAYOUT_NTCHW)      { prm.out_stride_t = 3 * HW; prm.out_stride_c = HW; }
+    else if (layout == BGD_LAYOUT_NCTHW) { prm.out_stride_t = HW;     prm.out_stride_c = T * HW; }
+    else                                 { prm.out_stride_t = 3 * HW; prm.out_stride_c = 1; }
+}
+
+int finish_launch(const char *kernel, Workspace &ws, cudaStream_t stream)
+{
+    count_launch();
+    cudaError_t e = cudaGetLastError();
+    const int rc = e == cudaSuccess ? BGD_OK : fail(BGD_ERR_CUDA, "%s launch failed: %s", kernel, cudaGetErrorString(e));
+    const int rc2 = ws.release(stream);
+    return rc ? rc : rc2;
+}
+
 }  // namespace
 
 int launch_resize_u8(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t B, int64_t T, int64_t H, int64_t W,
@@ -320,15 +355,11 @@ int launch_resize_u8(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_g
     if (!d_out) return fail(BGD_ERR_INVALID, "resize: null output");
     Workspace &ws = thread_workspace();
     TailParams prm{};
-    if (int rc = upload_geom(h_geom, B, T, H, W, src_bytes, ws, &prm, stream)) return rc;
+    if (int rc = upload_geom(h_geom, 5, B, T, H, W, src_bytes, ws, &prm, stream)) return rc;
     prm.src = d_src; prm.out_u8 = d_out;
     prm.T = T; prm.H = H; prm.W = W;
     resize_u8_kernel<<<tile_grid(B, H, W), dim3(kTileW, kTileH), 0, stream>>>(prm);
-    count_launch();
-    cudaError_t e = cudaGetLastError();
-    const int rc = e == cudaSuccess ? BGD_OK : fail(BGD_ERR_CUDA, "resize_u8_kernel launch failed: %s", cudaGetErrorString(e));
-    const int rc2 = ws.release(stream);
-    return rc ? rc : rc2;
+    return finish_launch("resize_u8_kernel", ws, stream);
 }
 
 int launch_resize_blend(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t B, int64_t T, int64_t H,
@@ -353,7 +384,7 @@ int launch_resize_blend(const uint8_t *d_src, int64_t src_bytes, const int64_t *
 
     Workspace &ws = thread_workspace();
     TailParams prm{};
-    if (int rc = upload_geom(h_geom, B, T, H, W, src_bytes, ws, &prm, stream)) return rc;
+    if (int rc = upload_geom(h_geom, 5, B, T, H, W, src_bytes, ws, &prm, stream)) return rc;
     prm.src = d_src;
     prm.pool = d_pool; prm.bg_idx = d_bg_idx; prm.top = d_top; prm.left = d_left; prm.apply = d_apply; prm.lut = d_lut;
     prm.out = d_out;
@@ -361,21 +392,38 @@ int launch_resize_blend(const uint8_t *d_src, int64_t src_bytes, const int64_t *
     for (int c = 0; c < 3; ++c) { prm.mean[c] = h_mean[c]; prm.std[c] = h_std[c]; }
     prm.w_fg = (float)(1.0 - alpha);
     prm.w_bg = (float)alpha;
-    const int64_t HW = H * W;
-    if (layout == BGD_LAYOUT_NTCHW)      { prm.out_stride_t = 3 * HW; prm.out_stride_c = HW; }
-    else if (layout == BGD_LAYOUT_NCTHW) { prm.out_stride_t = HW;     prm.out_stride_c = T * HW; }
-    else                                 { prm.out_stride_t = 3 * HW; prm.out_stride_c = 1; }
+    set_out_strides(layout, T, H, W, prm);
     dispatch_out(out_dtype, layout, [&](auto o, auto il) {
         using OutT = typename decltype(o)::type;
         constexpr bool IL = decltype(il)::value;
-        if (pool_is_u8) resize_blend_kernel<uint8_t, OutT, IL><<<tile_grid(B, H, W), dim3(kTileW, kTileH), 0, stream>>>(prm);
-        else            resize_blend_kernel<float, OutT, IL><<<tile_grid(B, H, W), dim3(kTileW, kTileH), 0, stream>>>(prm);
+        if (pool_is_u8) resize_blend_kernel<uint8_t, OutT, IL, true><<<tile_grid(B, H, W), dim3(kTileW, kTileH), 0, stream>>>(prm);
+        else            resize_blend_kernel<float, OutT, IL, true><<<tile_grid(B, H, W), dim3(kTileW, kTileH), 0, stream>>>(prm);
     });
-    count_launch();
-    cudaError_t e = cudaGetLastError();
-    const int rc = e == cudaSuccess ? BGD_OK : fail(BGD_ERR_CUDA, "resize_blend_kernel launch failed: %s", cudaGetErrorString(e));
-    const int rc2 = ws.release(stream);
-    return rc ? rc : rc2;
+    return finish_launch("resize_blend_kernel", ws, stream);
+}
+
+int launch_resize_normalize(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t n, int64_t T, int64_t H,
+                            int64_t W, const float *d_lut, int layout, int out_dtype, void *d_out, cudaStream_t stream)
+{
+    if (int rc = check_common(d_src, src_bytes, h_geom, n, T, H, W)) return rc;
+    if (layout != BGD_LAYOUT_NTCHW && layout != BGD_LAYOUT_NTHWC)
+        return fail(BGD_ERR_INVALID, "resize_crop_normalize: layout %d is not NTCHW or NTHWC", layout);
+    if (!out_elem_bytes(out_dtype)) return fail(BGD_ERR_INVALID, "resize_crop_normalize: unknown output type %d", out_dtype);
+    if (n == 0 || T == 0 || H == 0 || W == 0) return BGD_OK;
+    if (!d_out || !d_lut) return fail(BGD_ERR_INVALID, "resize_crop_normalize: null pointer");
+
+    Workspace &ws = thread_workspace();
+    TailParams prm{};
+    if (int rc = upload_geom(h_geom, 9, n, T, H, W, src_bytes, ws, &prm, stream)) return rc;
+    prm.src = d_src; prm.lut = d_lut; prm.out = d_out;
+    prm.T = T; prm.H = H; prm.W = W;
+    set_out_strides(layout, T, H, W, prm);
+    dispatch_out(out_dtype, layout, [&](auto o, auto il) {
+        using OutT = typename decltype(o)::type;
+        constexpr bool IL = decltype(il)::value;
+        resize_blend_kernel<uint8_t, OutT, IL, false><<<tile_grid(n, H, W), dim3(kTileW, kTileH), 0, stream>>>(prm);
+    });
+    return finish_launch("resize_blend_kernel", ws, stream);
 }
 
 }  // namespace bgd

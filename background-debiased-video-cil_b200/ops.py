@@ -25,6 +25,10 @@ built library (``ImportError`` otherwise).  Ops are stream-ordered and never syn
     bgdebias::bgmix_resize_blend(Tensor src, Tensor geom, int T, int H, int W, <bgmix_blend arguments>) -> Tensor
         the pipeline's Resize((W, H), keep_ratio=False) (config ..._bgmix_plus_randAug.py:136; cv2 INTER_LINEAR, bit-exact)
         on packed uint8 crops, alone or fused with the blend.
+    bgdebias::resize_crop_normalize(Tensor src, Tensor geom, int T, int H, int W, Tensor fg_lut, str layout,
+                                    ScalarType? out_dtype=None) -> Tensor
+        the evaluation tail Resize(scale=(-1, S)) -> CenterCrop / ThreeCrop -> Normalize -> FormatShape('NCHW') on packed
+        uint8 clips (geom [n, 9]: a resized size and a window per crop), no blend.
     bgdebias::ragged_pack(Tensor pool_bytes, Tensor segments, int out_bytes) -> Tensor
         one launch that gathers whole images of a ragged uint8 pool into one buffer (segments int64 [n, 3] = {source
         offset, destination offset, bytes}, 16-byte aligned): the owner side of pool.ShardedPool.fetch.
@@ -447,9 +451,9 @@ def pack_clips(clips, pin: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
     return buf, geom
 
 
-def _check_packed(name: str, src: torch.Tensor, geom: torch.Tensor):
+def _check_packed(name: str, src: torch.Tensor, geom: torch.Tensor, cols: int = 5):
     _require(src.dtype == torch.uint8 and src.dim() == 1, f"{name}: src must be a flat uint8 buffer")
-    _require(geom.dim() == 2 and geom.shape[1] == 5, f"{name}: geom must be int64 [B, 5]")
+    _require(geom.dim() == 2 and geom.shape[1] == cols, f"{name}: geom must be int64 [B, {cols}]")
     _require(src.numel() % 4 == 0, f"{name}: src must be a multiple of 4 bytes long (ops.pack_clips pads)")
     g = geom.detach().to("cpu", torch.int64).contiguous()
     return src.contiguous(), g, ctypes.cast(g.data_ptr(), ctypes.POINTER(ctypes.c_int64))
@@ -503,6 +507,33 @@ def bgmix_resize_blend(src: torch.Tensor, geom: torch.Tensor, T: int, H: int, W:
 def _(src, geom, T, H, W, bg_pool, bg_idx, top, left, apply, fg_lut, bg_mean, bg_std, alpha, layout, out_dtype=None):
     B = geom.shape[0]
     return src.new_empty(_out_shape(B, T, H, W, layout), dtype=_out_spec("bgmix_resize_blend", layout, out_dtype))
+
+
+@torch.library.custom_op("bgdebias::resize_crop_normalize", mutates_args=(), device_types="cuda")
+def resize_crop_normalize(src: torch.Tensor, geom: torch.Tensor, T: int, H: int, W: int, fg_lut: torch.Tensor, layout: str,
+                          out_dtype: Optional[torch.dtype] = None) -> torch.Tensor:
+    """The evaluation tail Resize -> CenterCrop / ThreeCrop -> Normalize -> FormatShape('NCHW') in one launch, with no blend.
+    ``geom`` int64 ``[n, 9]``: the five columns of :func:`pack_clips`, then ``{Hr, Wr, top, left}``; entry k is
+    ``cv2.resize(frame, (Wr, Hr), interpolation=cv2.INTER_LINEAR)[top:top + H, left:left + W]`` of every frame of its clip,
+    normalised through ``fg_lut`` (:func:`make_fg_lut`).  ``layout`` "NTCHW" (``[n, T, 3, H, W]``) or "NTHWC"
+    (``[n, T, H, W, 3]``); ``out_dtype`` as :func:`bgmix_blend`.  ``comix_loader.EvalPipeline.geometry`` builds the table."""
+    src, g, gptr = _check_packed("resize_crop_normalize", src, geom, 9)
+    _require(layout in ("NTCHW", "NTHWC"), "resize_crop_normalize: layout must be 'NTCHW' or 'NTHWC'")
+    out_dt = _out_spec("resize_crop_normalize", layout, out_dtype)
+    _check_lut("resize_crop_normalize", fg_lut, src.device)
+    fg_lut = fg_lut.contiguous()
+    out = torch.empty(_out_shape(g.shape[0], T, H, W, layout), dtype=out_dt, device=src.device)
+    with torch.cuda.device(src.device):
+        _cabi.check(_cabi.lib().bgd_resize_crop_normalize_out(
+            src.data_ptr(), src.numel(), gptr, g.shape[0], T, H, W, fg_lut.data_ptr(), _cabi.OUT_LAYOUTS[layout],
+            _OUT_DTYPES[out_dt], out.data_ptr(), _stream_ptr(src.device)))
+    return out
+
+
+@resize_crop_normalize.register_fake
+def _(src, geom, T, H, W, fg_lut, layout, out_dtype=None):
+    _require(layout in ("NTCHW", "NTHWC"), "resize_crop_normalize: layout must be 'NTCHW' or 'NTHWC'")
+    return src.new_empty(_out_shape(geom.shape[0], T, H, W, layout), dtype=_out_spec("resize_crop_normalize", layout, out_dtype))
 
 
 # --------------------------------------------------------------------------- #

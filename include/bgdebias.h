@@ -337,6 +337,24 @@ int bgd_bgmix_resize_blend_out(const uint8_t *d_src, int64_t src_bytes, const in
                                const float *d_fg_lut, const float *h_bg_mean, const float *h_bg_std,
                                double alpha, int layout, int out_dtype, void *d_out, void *stream);
 
+/* The evaluation pipeline's tail, with no blend: Resize(scale=(-1, S), keep_ratio=True) -> CenterCrop / ThreeCrop ->
+ * Normalize(to_bgr=False) -> FormatShape('NCHW') of mmaction2 0.x (the val / test / feature datasets of a CIL run), so that
+ * the DataLoader can ship the decoded uint8 frames.  Each output entry resizes one source clip to Hr x Wr (cv2.resize,
+ * INTER_LINEAR, bit-exact) and emits the H x W window at (top, left) of that resized image, normalised through d_fg_lut;
+ * the resized image never exists.  The crops of one clip are entries with the same source offset.
+ *
+ *   d_src      as bgd_resize_bilinear_u8
+ *   h_geom     HOST int64 [n][9]: the five columns of bgd_resize_bilinear_u8, then {Hr, Wr, top, left}; needs
+ *              Hr, Wr >= 1, top, left >= 0, top + H <= Hr and left + W <= Wr
+ *   d_fg_lut   fp32 [3][256] normalisation table, as bgd_bgmix_blend_f32
+ *   layout     BGD_LAYOUT_NTCHW ([n][T][3][H][W]) or BGD_LAYOUT_NTHWC ([n][T][H][W][3]); BGD_LAYOUT_NCTHW is rejected
+ *   out_dtype  as bgd_bgmix_blend_out
+ * With the entries of a batch ordered clip-major, then crop, d_out [n][T][3][H][W] is [B][K*T][3][H][W]: mmaction's
+ * crop-major ThreeCrop list after FormatShape('NCHW') and default_collate. */
+int bgd_resize_crop_normalize_out(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t n,
+                                  int64_t T, int64_t H, int64_t W, const float *d_fg_lut, int layout,
+                                  int out_dtype, void *d_out, void *stream);
+
 /* Host-buffer form of bgd_bgmix_resize_blend_f32, as bgd_bgmix_blend_f32_host is for the blend: the packed crops
  * (h_src, pinned or pageable) and the per-sample draws live in host memory -- what a DataLoader collate hands over when
  * the pipeline stops after MultiScaleCrop (config :129-135) -- the fp32 pool and the table are device resident.  Copies in,
