@@ -63,7 +63,6 @@ SIGNATURES = {
     "bgd_nan_temporal_reduce_varlen_f32": (_c.c_int, [_vp, _i64p, _c.c_int64, _c.c_int64, _c.c_int, _c.c_int, _vp, _vp, _vp]),
     "bgd_actor_cut_mix_u8": (_c.c_int, [_vp, _vp, _vp, _c.c_int64, _vp, _vp, _vp]),
     "bgd_bgmix_blend_f32": (_c.c_int, _blend_common + [_vp]),
-    "bgd_bgmix_blend_u8pool_f32": (_c.c_int, _blend_common + [_vp]),
     "bgd_bgmix_blend_out": (_c.c_int, [_vp, _c.c_int64, _c.c_int64, _c.c_int64, _c.c_int64,
                                        _vp, _c.c_int, _c.c_int64, _c.c_int64, _c.c_int64,
                                        _vp, _vp, _vp, _vp, _vp, _f32p, _f32p, _c.c_double, _c.c_int, _c.c_int, _vp, _vp]),
@@ -76,7 +75,6 @@ SIGNATURES = {
     "bgd_bgmix_blend_ragged_f32": (_c.c_int, [_vp] + _ragged_common + [_vp, _f32p, _f32p, _c.c_double, _c.c_int, _vp, _vp]),
     "bgd_bgmix_blend_ragged_out": (_c.c_int, [_vp] + _ragged_common + [_vp, _f32p, _f32p, _c.c_double, _c.c_int, _c.c_int,
                                                                        _vp, _vp]),
-    "bgd_bgmix_blend_ragged_normfg_f32": (_c.c_int, [_vp] + _ragged_common + [_f32p, _f32p, _c.c_double, _c.c_int, _vp, _vp]),
     "bgd_resized_crop_aa_u8_f32": (_c.c_int, [_vp, _c.c_int64, _vp, _c.c_int64, _vp, _c.c_int64, _c.c_int64, _c.c_int64,
                                               _vp, _vp]),
     "bgd_resize_bilinear_u8": (_c.c_int, [_vp, _c.c_int64, _i64p, _c.c_int64, _c.c_int64, _c.c_int64, _c.c_int64, _vp, _vp]),

@@ -597,24 +597,9 @@ int bgd_bgmix_blend_f32(const uint8_t *d_fg, int64_t B, int64_t T, int64_t H, in
                         const int32_t *d_left, const uint8_t *d_apply, const float *d_fg_lut, const float *h_bg_mean,
                         const float *h_bg_std, double alpha, int layout, float *d_out, void *stream)
 {
-    DeviceProps dp;
-    if (int rc = current_device_props(&dp)) return rc;
     if (int rc = f32_layout("bgmix", layout)) return rc;
-    return launch_bgmix(d_fg, nullptr, B, T, H, W, d_bg_pool, false, P, Hb, Wb, d_bg_idx, d_top, d_left, d_apply, d_fg_lut,
-                        h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out, static_cast<cudaStream_t>(stream));
-}
-
-int bgd_bgmix_blend_u8pool_f32(const uint8_t *d_fg, int64_t B, int64_t T, int64_t H, int64_t W,
-                               const uint8_t *d_bg_pool, int64_t P, int64_t Hb, int64_t Wb, const int32_t *d_bg_idx,
-                               const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply,
-                               const float *d_fg_lut, const float *h_bg_mean, const float *h_bg_std, double alpha,
-                               int layout, float *d_out, void *stream)
-{
-    DeviceProps dp;
-    if (int rc = current_device_props(&dp)) return rc;
-    if (int rc = f32_layout("bgmix", layout)) return rc;
-    return launch_bgmix(d_fg, nullptr, B, T, H, W, d_bg_pool, true, P, Hb, Wb, d_bg_idx, d_top, d_left, d_apply, d_fg_lut,
-                        h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out, static_cast<cudaStream_t>(stream));
+    return bgd_bgmix_blend_out(d_fg, B, T, H, W, d_bg_pool, 0, P, Hb, Wb, d_bg_idx, d_top, d_left, d_apply, d_fg_lut, h_bg_mean,
+                               h_bg_std, alpha, layout, BGD_OUT_F32, d_out, stream);
 }
 
 int bgd_bgmix_blend_out(const uint8_t *d_fg, int64_t B, int64_t T, int64_t H, int64_t W, const void *d_bg_pool, int pool_is_u8,
@@ -624,7 +609,6 @@ int bgd_bgmix_blend_out(const uint8_t *d_fg, int64_t B, int64_t T, int64_t H, in
 {
     DeviceProps dp;
     if (int rc = current_device_props(&dp)) return rc;
-    if (!d_fg) return fail(BGD_ERR_INVALID, "bgmix: null foreground");
     return launch_bgmix(d_fg, nullptr, B, T, H, W, d_bg_pool, pool_is_u8 != 0, P, Hb, Wb, d_bg_idx, d_top, d_left, d_apply,
                         d_fg_lut, h_bg_mean, h_bg_std, alpha, layout, out_dtype, d_out, static_cast<cudaStream_t>(stream));
 }
@@ -661,12 +645,9 @@ int bgd_bgmix_blend_ragged_f32(const uint8_t *d_fg, int64_t B, int64_t T, int64_
                                const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply, const float *d_fg_lut,
                                const float *h_bg_mean, const float *h_bg_std, double alpha, int layout, float *d_out, void *stream)
 {
-    DeviceProps dp;
-    if (int rc = current_device_props(&dp)) return rc;
-    if (!d_fg) return fail(BGD_ERR_INVALID, "bgmix (ragged): null foreground");
     if (int rc = f32_layout("bgmix (ragged)", layout)) return rc;
-    return launch_bgmix_ragged(d_fg, nullptr, B, T, H, W, d_pool, d_slots, P, d_tables, d_bg_idx, d_top, d_left, d_apply, d_fg_lut,
-                               h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out, static_cast<cudaStream_t>(stream));
+    return bgd_bgmix_blend_ragged_out(d_fg, B, T, H, W, d_pool, d_slots, P, d_tables, d_bg_idx, d_top, d_left, d_apply, d_fg_lut,
+                                      h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out, stream);
 }
 
 int bgd_bgmix_blend_ragged_out(const uint8_t *d_fg, int64_t B, int64_t T, int64_t H, int64_t W, const uint8_t *d_pool,
@@ -677,23 +658,8 @@ int bgd_bgmix_blend_ragged_out(const uint8_t *d_fg, int64_t B, int64_t T, int64_
 {
     DeviceProps dp;
     if (int rc = current_device_props(&dp)) return rc;
-    if (!d_fg) return fail(BGD_ERR_INVALID, "bgmix (ragged): null foreground");
-    return launch_bgmix_ragged(d_fg, nullptr, B, T, H, W, d_pool, d_slots, P, d_tables, d_bg_idx, d_top, d_left, d_apply, d_fg_lut,
+    return launch_bgmix_ragged(d_fg, B, T, H, W, d_pool, d_slots, P, d_tables, d_bg_idx, d_top, d_left, d_apply, d_fg_lut,
                                h_bg_mean, h_bg_std, alpha, layout, out_dtype, d_out, static_cast<cudaStream_t>(stream));
-}
-
-int bgd_bgmix_blend_ragged_normfg_f32(const float *d_fg_norm, int64_t B, int64_t T, int64_t H, int64_t W, const uint8_t *d_pool,
-                                      const bgd_ragged_slot *d_slots, int64_t P, const int32_t *d_tables,
-                                      const int32_t *d_bg_idx, const int32_t *d_top, const int32_t *d_left,
-                                      const uint8_t *d_apply, const float *h_bg_mean, const float *h_bg_std, double alpha,
-                                      int layout, float *d_out, void *stream)
-{
-    DeviceProps dp;
-    if (int rc = current_device_props(&dp)) return rc;
-    if (!d_fg_norm) return fail(BGD_ERR_INVALID, "bgmix (ragged): null foreground");
-    if (int rc = f32_layout("bgmix (ragged)", layout)) return rc;
-    return launch_bgmix_ragged(nullptr, d_fg_norm, B, T, H, W, d_pool, d_slots, P, d_tables, d_bg_idx, d_top, d_left, d_apply,
-                               nullptr, h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out, static_cast<cudaStream_t>(stream));
 }
 
 int bgd_resized_crop_aa_u8_f32(const uint8_t *d_src, int64_t src_bytes, const bgd_crop_desc *h_desc, int64_t n,
@@ -720,12 +686,9 @@ int bgd_bgmix_resize_blend_f32(const uint8_t *d_src, int64_t src_bytes, const in
                                const float *d_fg_lut, const float *h_bg_mean, const float *h_bg_std, double alpha, int layout,
                                float *d_out, void *stream)
 {
-    DeviceProps dp;
-    if (int rc = current_device_props(&dp)) return rc;
     if (int rc = f32_layout("bgmix_resize", layout)) return rc;
-    return launch_resize_blend(d_src, src_bytes, h_geom, B, T, H, W, d_bg_pool, pool_is_u8 != 0, P, Hb, Wb, d_bg_idx, d_top,
-                               d_left, d_apply, d_fg_lut, h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out,
-                               static_cast<cudaStream_t>(stream));
+    return bgd_bgmix_resize_blend_out(d_src, src_bytes, h_geom, B, T, H, W, d_bg_pool, pool_is_u8, P, Hb, Wb, d_bg_idx, d_top,
+                                      d_left, d_apply, d_fg_lut, h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out, stream);
 }
 
 int bgd_bgmix_resize_blend_out(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t B, int64_t T, int64_t H,

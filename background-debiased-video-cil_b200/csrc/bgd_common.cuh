@@ -148,11 +148,11 @@ int launch_resize_blend(const uint8_t *d_src, int64_t src_bytes, const int64_t *
 int launch_resize_normalize(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t n, int64_t T, int64_t H,
                             int64_t W, const float *d_lut, int layout, int out_dtype, void *d_out, cudaStream_t stream);
 int aa_resize_table(int64_t in_size, int64_t out_size, int32_t *K_out, int32_t *words, int64_t cap_words);
-int launch_bgmix_ragged(const uint8_t *d_fg, const float *d_fg_norm, int64_t B, int64_t T, int64_t H, int64_t W,
-                        const uint8_t *d_pool, const bgd_ragged_slot *d_slots, int64_t P, const int32_t *d_tables,
-                        const int32_t *d_bg_idx, const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply,
-                        const float *d_lut, const float *h_mean, const float *h_std, double alpha, int layout, int out_dtype,
-                        void *d_out, cudaStream_t stream);
+int launch_bgmix_ragged(const uint8_t *d_fg, int64_t B, int64_t T, int64_t H, int64_t W, const uint8_t *d_pool,
+                        const bgd_ragged_slot *d_slots, int64_t P, const int32_t *d_tables, const int32_t *d_bg_idx,
+                        const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply, const float *d_lut,
+                        const float *h_mean, const float *h_std, double alpha, int layout, int out_dtype, void *d_out,
+                        cudaStream_t stream);
 int launch_aa_resize(const uint8_t *d_img, const bgd_ragged_slot *h_slot, const int32_t *d_tables, float *d_out, cudaStream_t stream);
 int launch_resized_crop_aa(const uint8_t *d_src, int64_t src_bytes, const bgd_crop_desc *h_desc, int64_t n,
                            const int32_t *d_tables, int64_t table_words, int64_t out_h, int64_t out_w, float *d_out,

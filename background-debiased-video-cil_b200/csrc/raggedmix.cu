@@ -24,10 +24,9 @@
 //   in-order vector part + scalar epilogue with contraction); an axis whose size does not change is skipped.
 // The weights depend on (in, out, i) only; bgd_aa_resize_table evaluates them on the host, once per distinct size.
 //
-// Blend arithmetic as in bgmix.cu (each operation rounded, no contraction):
-//   fg = lut[c][x];  bg = (resized - mean[c]) / std[c];  out = fg * f32(1 - alpha) + bg * f32(alpha)
+// Blend arithmetic: blend.cuh, with the resized value as the raw background.
 #include "aa_resample.cuh"
-#include "bgd_common.cuh"
+#include "blend.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -40,27 +39,20 @@ constexpr int kThreads = 256;
 
 struct RaggedParams {
     const uint8_t *fg;
-    const float *fgn;                 // normalised foreground instead of fg + lut (may be null)
     const uint8_t *pool;
     const bgd_ragged_slot *slots;
     const int32_t *tables;
-    const int32_t *bg_idx, *top, *left;
-    const uint8_t *apply;
-    const float *lut;
-    void *out;                        // float, or OutT of the uint8-foreground kernels
     int64_t T, H, W, P;
-    float mean[3], std[3];
-    float w_fg, w_bg;
-    int64_t out_stride_t, out_stride_c;   // in elements (NTHWC: 3 * H * W, 1)
+    BlendParams blend;
 };
 
 __device__ __forceinline__ bgd_ragged_slot load_slot(const RaggedParams &prm, int64_t b, int &top, int &left)
 {
-    int64_t idx = prm.bg_idx[b];
+    int64_t idx = prm.blend.bg_idx[b];
     idx = idx < 0 ? 0 : (idx >= prm.P ? prm.P - 1 : idx);                    // host validates; clamp = no OOB
     const bgd_ragged_slot s = prm.slots[idx];
-    top = min(max(prm.top[b], 0), max(s.Hb - (int)prm.H, 0));
-    left = min(max(prm.left[b], 0), max(s.Wb - (int)prm.W, 0));
+    top = min(max(prm.blend.top[b], 0), max(s.Hb - (int)prm.H, 0));
+    left = min(max(prm.blend.left[b], 0), max(s.Wb - (int)prm.W, 0));
     return s;
 }
 
@@ -69,8 +61,9 @@ __device__ __forceinline__ bgd_ragged_slot load_slot(const RaggedParams &prm, in
 template <int PX, typename OutT, bool IL>
 __global__ void __launch_bounds__(kThreads) bgmix_ragged_kernel(const RaggedParams prm)
 {
+    const BlendParams &bp = prm.blend;
     __shared__ float s_lut[3 * 256];
-    for (int i = threadIdx.x; i < 3 * 256; i += kThreads) s_lut[i] = __ldg(prm.lut + i);
+    stage_lut<kThreads>(s_lut, bp.lut, threadIdx.x);
     __syncthreads();
 
     const int64_t b = blockIdx.y;
@@ -78,7 +71,7 @@ __global__ void __launch_bounds__(kThreads) bgmix_ragged_kernel(const RaggedPara
     const int64_t p0 = ((int64_t)blockIdx.x * kThreads + threadIdx.x) * PX;
     if (p0 >= HW) return;
 
-    const bool apply = prm.apply[b] != 0;
+    const bool apply = bp.apply[b] != 0;
     float g[3][PX];
     if (apply) {
         int top, left;
@@ -91,42 +84,14 @@ __global__ void __launch_bounds__(kThreads) bgmix_ragged_kernel(const RaggedPara
             for (int i = 0; i < PX; ++i) {
                 const float raw = aa_sample(img + (int64_t)c * s.h * s.w, s.w, prm.tables, s.xtab, s.kx, s.ytab, s.ky, top + y,
                                             left + x + i);
-                g[c][i] = __fmul_rn(__fdiv_rn(__fsub_rn(raw, prm.mean[c]), prm.std[c]), prm.w_bg);
+                g[c][i] = scaled_bg(bp, c, raw);
             }
     }
 
     const uint8_t *fg = prm.fg + (b * prm.T * HW + p0) * 3;
-    OutT *out = static_cast<OutT *>(prm.out) + b * prm.T * 3 * HW + (IL ? 3 * p0 : p0);
+    OutT *out = static_cast<OutT *>(bp.out) + b * prm.T * 3 * HW + (IL ? 3 * p0 : p0);
 #pragma unroll 2
-    for (int64_t t = 0; t < prm.T; ++t) {
-        uint8_t px[3 * PX];
-        if (PX == 4) {
-            const uint32_t *src = reinterpret_cast<const uint32_t *>(fg + t * HW * 3);
-            const uint32_t w0 = __ldcs(src), w1 = __ldcs(src + 1), w2 = __ldcs(src + 2);
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                px[k] = (w0 >> (8 * k)) & 0xFF;
-                px[4 + k] = (w1 >> (8 * k)) & 0xFF;
-                px[8 + k] = (w2 >> (8 * k)) & 0xFF;
-            }
-        } else {
-#pragma unroll
-            for (int k = 0; k < 3 * PX; ++k) px[k] = __ldcs(fg + t * HW * 3 + k);
-        }
-        float r[3][PX];
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-#pragma unroll
-            for (int i = 0; i < PX; ++i) {
-                const float f = s_lut[c * 256 + px[i * 3 + c]];
-                r[c][i] = apply ? __fadd_rn(__fmul_rn(f, prm.w_fg), g[c][i]) : f;
-            }
-            OutT *dst = out + t * prm.out_stride_t + c * prm.out_stride_c;
-            if constexpr (PX == 4 && !IL) store_out4(dst, r[c]);
-            else if constexpr (PX == 1) store_out(dst, r[c][0]);
-        }
-        if constexpr (PX == 4 && IL) store_out12(out + t * prm.out_stride_t, r);
-    }
+    for (int64_t t = 0; t < prm.T; ++t) blend_frame<PX, IL>(fg + t * HW * 3, s_lut, apply, g, bp, out + t * bp.out_stride_t);
 }
 
 // ---- tiled form of the same blend (the product path when W % 4 == 0) -------------------------------------------------
@@ -146,16 +111,17 @@ constexpr int kMaxSrcRows = 48;           // source rows of one tile kept in sha
 template <typename OutT, bool IL>
 __global__ void __launch_bounds__(kThreads, BGD_RAGGED_MINBLOCKS) bgmix_ragged_tile_kernel(const RaggedParams prm)
 {
+    const BlendParams &bp = prm.blend;
     __shared__ float s_lut[3 * 256];
     __shared__ __align__(16) float s_h[3][kMaxSrcRows][kTile];
-    for (int i = threadIdx.x; i < 3 * 256; i += kThreads) s_lut[i] = __ldg(prm.lut + i);
+    stage_lut<kThreads>(s_lut, bp.lut, threadIdx.x);
 
     const int64_t b = blockIdx.z;
     const int tx0 = blockIdx.x * kTile, ty0 = blockIdx.y * kTile;
     const int ty = threadIdx.x >> 3, tx = (threadIdx.x & 7) << 2;      // this thread's row and first column inside the tile
     const int W = (int)prm.W, H = (int)prm.H;
     const bool inside = ty0 + ty < H && tx0 + tx < W;                  // W % 4 == 0: a group of 4 is inside or outside as a whole
-    const bool apply = prm.apply[b] != 0;                              // uniform over the CTA
+    const bool apply = bp.apply[b] != 0;                                // uniform over the CTA
 
     float g[3][4];
     if (apply) {
@@ -195,7 +161,7 @@ __global__ void __launch_bounds__(kThreads, BGD_RAGGED_MINBLOCKS) bgmix_ragged_t
             for (int c = 0; c < 3; ++c)
 #pragma unroll
                 for (int i = 0; i < 4; ++i)
-                    g[c][i] = __fmul_rn(__fdiv_rn(__fsub_rn(g[c][i], prm.mean[c]), prm.std[c]), prm.w_bg);
+                    g[c][i] = scaled_bg(bp, c, g[c][i]);
         }
     } else {
         __syncthreads();                                               // the table load above
@@ -205,55 +171,9 @@ __global__ void __launch_bounds__(kThreads, BGD_RAGGED_MINBLOCKS) bgmix_ragged_t
     const int64_t HW = prm.H * prm.W;
     const int64_t p0 = (int64_t)(ty0 + ty) * W + tx0 + tx;
     const uint8_t *fg = prm.fg + (b * prm.T * HW + p0) * 3;
-    OutT *out = static_cast<OutT *>(prm.out) + b * prm.T * 3 * HW + (IL ? 3 * p0 : p0);
+    OutT *out = static_cast<OutT *>(bp.out) + b * prm.T * 3 * HW + (IL ? 3 * p0 : p0);
 #pragma unroll 4
-    for (int64_t t = 0; t < prm.T; ++t) {
-        const uint32_t *src = reinterpret_cast<const uint32_t *>(fg + t * HW * 3);
-        const uint32_t w0 = __ldcs(src), w1 = __ldcs(src + 1), w2 = __ldcs(src + 2);
-        uint8_t px[12];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            px[k] = (w0 >> (8 * k)) & 0xFF;
-            px[4 + k] = (w1 >> (8 * k)) & 0xFF;
-            px[8 + k] = (w2 >> (8 * k)) & 0xFF;
-        }
-        float r[3][4];
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const float f = s_lut[c * 256 + px[i * 3 + c]];
-                r[c][i] = apply ? __fadd_rn(__fmul_rn(f, prm.w_fg), g[c][i]) : f;
-            }
-            if constexpr (!IL) store_out4(out + t * prm.out_stride_t + c * prm.out_stride_c, r[c]);
-        }
-        if constexpr (IL) store_out12(out + t * prm.out_stride_t, r);
-    }
-}
-
-// normalised fp32 foreground [B][T][3][H][W] (the reference's `imgs`): one thread = one pixel of one (sample, channel)
-__global__ void __launch_bounds__(kThreads) bgmix_ragged_normfg_kernel(const RaggedParams prm)
-{
-    const int64_t b = blockIdx.z, c = blockIdx.y;
-    const int64_t HW = prm.H * prm.W;
-    const int64_t p = (int64_t)blockIdx.x * kThreads + threadIdx.x;
-    if (p >= HW) return;
-    const bool apply = prm.apply[b] != 0;
-    float g = 0.f;
-    if (apply) {
-        int top, left;
-        const bgd_ragged_slot s = load_slot(prm, b, top, left);
-        const int y = (int)(p / prm.W), x = (int)(p - (int64_t)y * prm.W);
-        const float raw = aa_sample(prm.pool + s.offset + c * (int64_t)s.h * s.w, s.w, prm.tables, s.xtab, s.kx, s.ytab, s.ky,
-                                    top + y, left + x);
-        g = __fmul_rn(__fdiv_rn(__fsub_rn(raw, prm.mean[c]), prm.std[c]), prm.w_bg);
-    }
-    const float *src = prm.fgn + (b * prm.T * 3 + c) * HW + p;
-    float *out = static_cast<float *>(prm.out) + b * prm.T * 3 * HW + c * prm.out_stride_c + p;
-    for (int64_t t = 0; t < prm.T; ++t) {
-        const float f = __ldcs(src + t * 3 * HW);
-        __stcs(out + t * prm.out_stride_t, apply ? __fadd_rn(__fmul_rn(f, prm.w_fg), g) : f);
-    }
+    for (int64_t t = 0; t < prm.T; ++t) blend_frame<4, IL>(fg + t * HW * 3, s_lut, apply, g, bp, out + t * bp.out_stride_t);
 }
 
 // Resize alone: planar uint8 [3][h][w] -> fp32 [3][Hb][Wb]
@@ -319,69 +239,38 @@ int aa_resize_table(int64_t in_size, int64_t out_size, int32_t *K_out, int32_t *
     return BGD_OK;
 }
 
-static int fill_params(RaggedParams &prm, int64_t B, int64_t T, int64_t H, int64_t W, const uint8_t *d_pool,
-                       const bgd_ragged_slot *d_slots, int64_t P, const int32_t *d_tables, const int32_t *d_bg_idx,
-                       const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply, const float *h_mean,
-                       const float *h_std, double alpha, int layout, int out_dtype, void *d_out)
-{
-    if (B < 0 || T < 0 || H < 0 || W < 0 || P < 0) return fail(BGD_ERR_INVALID, "bgmix (ragged): negative size");
-    if (!d_out || !d_apply) return fail(BGD_ERR_INVALID, "bgmix (ragged): null pointer");
-    if (!h_mean || !h_std) return fail(BGD_ERR_INVALID, "bgmix (ragged): null mean/std");
-    if (P > 0 && (!d_pool || !d_slots || !d_bg_idx || !d_top || !d_left)) return fail(BGD_ERR_INVALID, "bgmix (ragged): null pool argument");
-    if (layout != BGD_LAYOUT_NTCHW && layout != BGD_LAYOUT_NCTHW && layout != BGD_LAYOUT_NTHWC)
-        return fail(BGD_ERR_INVALID, "bgmix (ragged): unknown layout %d", layout);
-    if (!out_elem_bytes(out_dtype)) return fail(BGD_ERR_INVALID, "bgmix (ragged): unknown output type %d", out_dtype);
-    if (B > 65535) return fail(BGD_ERR_INVALID, "bgmix (ragged): batch larger than 65535");
-    if (H >= (1 << 24) || W >= (1 << 24)) return fail(BGD_ERR_INVALID, "bgmix (ragged): crop too large");
-    prm.pool = d_pool; prm.slots = d_slots; prm.tables = d_tables; prm.bg_idx = d_bg_idx; prm.top = d_top; prm.left = d_left;
-    prm.apply = d_apply; prm.out = d_out;
-    prm.T = T; prm.H = H; prm.W = W; prm.P = P > 0 ? P : 1;
-    for (int c = 0; c < 3; ++c) { prm.mean[c] = h_mean[c]; prm.std[c] = h_std[c]; }
-    prm.w_fg = (float)(1.0 - alpha);
-    prm.w_bg = (float)alpha;
-    const int64_t HW = H * W;
-    if (layout == BGD_LAYOUT_NTCHW)      { prm.out_stride_t = 3 * HW; prm.out_stride_c = HW; }
-    else if (layout == BGD_LAYOUT_NCTHW) { prm.out_stride_t = HW;     prm.out_stride_c = T * HW; }
-    else                                 { prm.out_stride_t = 3 * HW; prm.out_stride_c = 1; }
-    return BGD_OK;
-}
-
-int launch_bgmix_ragged(const uint8_t *d_fg, const float *d_fg_norm, int64_t B, int64_t T, int64_t H, int64_t W,
-                        const uint8_t *d_pool, const bgd_ragged_slot *d_slots, int64_t P, const int32_t *d_tables,
-                        const int32_t *d_bg_idx, const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply,
-                        const float *d_lut, const float *h_mean, const float *h_std, double alpha, int layout, int out_dtype,
-                        void *d_out, cudaStream_t stream)
+int launch_bgmix_ragged(const uint8_t *d_fg, int64_t B, int64_t T, int64_t H, int64_t W, const uint8_t *d_pool,
+                        const bgd_ragged_slot *d_slots, int64_t P, const int32_t *d_tables, const int32_t *d_bg_idx,
+                        const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply, const float *d_lut,
+                        const float *h_mean, const float *h_std, double alpha, int layout, int out_dtype, void *d_out,
+                        cudaStream_t stream)
 {
     RaggedParams prm{};
-    if (int rc = fill_params(prm, B, T, H, W, d_pool, d_slots, P, d_tables, d_bg_idx, d_top, d_left, d_apply, h_mean, h_std, alpha,
-                             layout, out_dtype, d_out))
+    if (int rc = fill_blend("bgmix (ragged)", B, T, H, W, P, d_bg_idx, d_top, d_left, d_apply, d_lut, h_mean, h_std, alpha,
+                            layout, out_dtype, d_out, &prm.blend))
         return rc;
+    if (H >= (1 << 24) || W >= (1 << 24)) return fail(BGD_ERR_INVALID, "bgmix (ragged): crop too large");
     if (B == 0 || T == 0 || H == 0 || W == 0) return BGD_OK;
-    if (!d_fg && !d_fg_norm) return fail(BGD_ERR_INVALID, "bgmix (ragged): null foreground");
-    if (d_fg && !d_lut) return fail(BGD_ERR_INVALID, "bgmix (ragged): null table");
-    prm.fg = d_fg; prm.fgn = d_fg_norm; prm.lut = d_lut;
+    if (P > 0 && (!d_pool || !d_slots)) return fail(BGD_ERR_INVALID, "bgmix (ragged): null pool argument");
+    if (!d_fg) return fail(BGD_ERR_INVALID, "bgmix (ragged): null foreground");
+    if (!d_lut) return fail(BGD_ERR_INVALID, "bgmix (ragged): null table");
+    prm.fg = d_fg; prm.pool = d_pool; prm.slots = d_slots; prm.tables = d_tables;
+    prm.T = T; prm.H = H; prm.W = W; prm.P = P > 0 ? P : 1;
     const int64_t HW = H * W;
-    if (d_fg_norm) {
-        if (layout == BGD_LAYOUT_NTHWC || out_dtype != BGD_OUT_F32)
-            return fail(BGD_ERR_INVALID, "bgmix (ragged): a normalised foreground blends to fp32 NTCHW / NCTHW only");
-        dim3 grid((unsigned)((HW + kThreads - 1) / kThreads), 3u, (unsigned)B);
-        bgmix_ragged_normfg_kernel<<<grid, kThreads, 0, stream>>>(prm);
-    } else {
-        const bool vec = (W % 4 == 0) && (reinterpret_cast<uintptr_t>(d_fg) % 4 == 0) &&
-                         (reinterpret_cast<uintptr_t>(d_out) % (4 * out_elem_bytes(out_dtype)) == 0);
-        const int px = vec ? 4 : 1;
-        dim3 grid((unsigned)((HW / px + kThreads - 1) / kThreads), (unsigned)B);
-        static const bool per_value = getenv("BGD_RAGGED_PER_VALUE") != nullptr;     // differential testing of the two forms
-        dim3 tgrid((unsigned)((W + kTile - 1) / kTile), (unsigned)((H + kTile - 1) / kTile), (unsigned)B);
-        if (vec && !per_value && tgrid.y > 65535) return fail(BGD_ERR_INVALID, "bgmix (ragged): crop too tall");
-        dispatch_out(out_dtype, layout, [&](auto o, auto il) {
-            using OutT = typename decltype(o)::type;
-            constexpr bool IL = decltype(il)::value;
-            if (vec && !per_value) bgmix_ragged_tile_kernel<OutT, IL><<<tgrid, kThreads, 0, stream>>>(prm);
-            else if (vec)          bgmix_ragged_kernel<4, OutT, IL><<<grid, kThreads, 0, stream>>>(prm);
-            else                   bgmix_ragged_kernel<1, OutT, IL><<<grid, kThreads, 0, stream>>>(prm);
-        });
-    }
+    const bool vec = (W % 4 == 0) && (reinterpret_cast<uintptr_t>(d_fg) % 4 == 0) &&
+                     (reinterpret_cast<uintptr_t>(d_out) % (4 * out_elem_bytes(out_dtype)) == 0);
+    const int px = vec ? 4 : 1;
+    dim3 grid((unsigned)((HW / px + kThreads - 1) / kThreads), (unsigned)B);
+    static const bool per_value = getenv("BGD_RAGGED_PER_VALUE") != nullptr;     // differential testing of the two forms
+    dim3 tgrid((unsigned)((W + kTile - 1) / kTile), (unsigned)((H + kTile - 1) / kTile), (unsigned)B);
+    if (vec && !per_value && tgrid.y > 65535) return fail(BGD_ERR_INVALID, "bgmix (ragged): crop too tall");
+    dispatch_out(out_dtype, layout, [&](auto o, auto il) {
+        using OutT = typename decltype(o)::type;
+        constexpr bool IL = decltype(il)::value;
+        if (vec && !per_value) bgmix_ragged_tile_kernel<OutT, IL><<<tgrid, kThreads, 0, stream>>>(prm);
+        else if (vec)          bgmix_ragged_kernel<4, OutT, IL><<<grid, kThreads, 0, stream>>>(prm);
+        else                   bgmix_ragged_kernel<1, OutT, IL><<<grid, kThreads, 0, stream>>>(prm);
+    });
     count_launch();
     BGD_CUDA_TRY(cudaGetLastError());
     return BGD_OK;

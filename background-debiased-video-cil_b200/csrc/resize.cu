@@ -28,9 +28,9 @@
 // output pixels of one clip, one thread per pixel: it reads its column entry and its row entry, then walks the T frames of the
 // clip.  Per frame it reads the two 6-byte tap pairs (RGB of two adjacent source pixels) with aligned 32-bit loads and a
 // funnel shift, so neighbouring lanes share cache lines, pairs left/right bytes with byte permutes and multiplies with dp2a;
-// the 3 results go through the normalisation table and the blend of bgmix.cu and are stored as one coalesced 128-byte row
+// the 3 results go through the normalisation table and the blend of blend.cuh and are stored as one coalesced 128-byte row
 // per warp and channel plane.
-#include "bgd_common.cuh"
+#include "blend.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -68,17 +68,10 @@ struct TailParams {
     const uint8_t *src;
     const ClipGeom *geom;
     const Coef *coef;
-    // blend half (unused by the uint8 resize kernel)
     const void *pool;
-    const int32_t *bg_idx, *top, *left;
-    const uint8_t *apply;
-    const float *lut;
-    void *out;                 // OutT of resize_blend_kernel
     uint8_t *out_u8;
     int64_t T, H, W, P, Hb, Wb;
-    float mean[3], std[3];
-    float w_fg, w_bg;
-    int64_t out_stride_t, out_stride_c;
+    BlendParams blend;         // unused by the uint8 resize kernel
 };
 
 struct Taps {
@@ -175,8 +168,9 @@ __global__ void __launch_bounds__(kThreads) resize_u8_kernel(const TailParams pr
 template <typename PoolT, typename OutT, bool IL, bool BLEND>
 __global__ void __launch_bounds__(kThreads, kBlendMinBlocks) resize_blend_kernel(const TailParams prm)
 {
+    const BlendParams &bp = prm.blend;
     __shared__ float s_lut[3 * 256];
-    for (int i = threadIdx.y * kTileW + threadIdx.x; i < 3 * 256; i += kThreads) s_lut[i] = __ldg(prm.lut + i);
+    stage_lut<kThreads>(s_lut, bp.lut, threadIdx.y * kTileW + threadIdx.x);
     __syncthreads();
 
     const int64_t b = blockIdx.z;
@@ -185,31 +179,27 @@ __global__ void __launch_bounds__(kThreads, kBlendMinBlocks) resize_blend_kernel
     const ClipGeom g = prm.geom[b];
     const Taps t = make_taps(prm, g, x, y);
 
-    const bool apply = BLEND && prm.apply[b] != 0;
+    const bool apply = BLEND && bp.apply[b] != 0;
     float bgw[3] = {0.f, 0.f, 0.f};                  // normalised background * alpha
     if constexpr (BLEND) if (apply) {
         // one pool image has fewer than 2^31 elements (checked on the host): only the image index needs 64 bits
         const int Hb = (int)prm.Hb, Wb = (int)prm.Wb, plane = Hb * Wb;
-        int64_t idx = prm.bg_idx[b];
+        int64_t idx = bp.bg_idx[b];
         idx = idx < 0 ? 0 : (idx >= prm.P ? prm.P - 1 : idx);               // host validates; clamp = no OOB
-        const int top = min(max(prm.top[b], 0), Hb - (int)prm.H);
-        const int left = min(max(prm.left[b], 0), Wb - (int)prm.W);
+        const int top = min(max(bp.top[b], 0), Hb - (int)prm.H);
+        const int left = min(max(bp.left[b], 0), Wb - (int)prm.W);
         const PoolT *pb = static_cast<const PoolT *>(prm.pool) + idx * (3 * plane) + ((top + y) * Wb + left + x);
 #pragma unroll
-        for (int c = 0; c < 3; ++c) {
-            const float raw = (float)__ldg(pb + c * plane);
-            bgw[c] = __fmul_rn(__fdiv_rn(__fsub_rn(raw, prm.mean[c]), prm.std[c]), prm.w_bg);
-        }
+        for (int c = 0; c < 3; ++c) bgw[c] = scaled_bg(bp, c, (float)__ldg(pb + c * plane));
     }
 
     const int64_t HW = prm.H * prm.W;
-    OutT *out = IL ? static_cast<OutT *>(prm.out) + b * prm.T * 3 * HW + 3 * ((int64_t)y * prm.W + x)
-                   : static_cast<OutT *>(prm.out) + b * prm.T * 3 * HW + (int64_t)y * prm.W + x;
-    const int64_t st = prm.out_stride_t, sc = prm.out_stride_c;
-    const float w_fg = prm.w_fg;
+    OutT *out = IL ? static_cast<OutT *>(bp.out) + b * prm.T * 3 * HW + 3 * ((int64_t)y * prm.W + x)
+                   : static_cast<OutT *>(bp.out) + b * prm.T * 3 * HW + (int64_t)y * prm.W + x;
+    const int64_t st = bp.out_stride_t, sc = bp.out_stride_c;
+    const float w_fg = bp.w_fg;
     auto emit = [&](int64_t f, int c, uint32_t v) {
-        const float n = s_lut[c * 256 + v];
-        store_out(out + f * st + c * sc, apply ? __fadd_rn(__fmul_rn(n, w_fg), bgw[c]) : n);
+        store_out(out + f * st + c * sc, mix(s_lut[c * 256 + v], bgw[c], apply, w_fg));
     };
     if ((g.frame_stride & 3) == 0) for_each_frame<true>(prm, g, t, emit);
     else                           for_each_frame<false>(prm, g, t, emit);
@@ -327,15 +317,6 @@ dim3 tile_grid(int64_t B, int64_t H, int64_t W)
     return dim3((unsigned)((W + kTileW - 1) / kTileW), (unsigned)((H + kTileH - 1) / kTileH), (unsigned)B);
 }
 
-// Output strides of the fp32 / 16-bit kernels (the layout is validated by the caller).
-void set_out_strides(int layout, int64_t T, int64_t H, int64_t W, TailParams &prm)
-{
-    const int64_t HW = H * W;
-    if (layout == BGD_LAYOUT_NTCHW)      { prm.out_stride_t = 3 * HW; prm.out_stride_c = HW; }
-    else if (layout == BGD_LAYOUT_NCTHW) { prm.out_stride_t = HW;     prm.out_stride_c = T * HW; }
-    else                                 { prm.out_stride_t = 3 * HW; prm.out_stride_c = 1; }
-}
-
 int finish_launch(const char *kernel, Workspace &ws, cudaStream_t stream)
 {
     count_launch();
@@ -368,31 +349,24 @@ int launch_resize_blend(const uint8_t *d_src, int64_t src_bytes, const int64_t *
                         const float *d_lut, const float *h_mean, const float *h_std, double alpha, int layout, int out_dtype,
                         void *d_out, cudaStream_t stream)
 {
+    TailParams prm{};
     if (int rc = check_common(d_src, src_bytes, h_geom, B, T, H, W)) return rc;
+    if (int rc = fill_blend("bgmix_resize", B, T, H, W, P, d_bg_idx, d_top, d_left, d_apply, d_lut, h_mean, h_std, alpha, layout,
+                            out_dtype, d_out, &prm.blend))
+        return rc;
     if (B == 0 || T == 0 || H == 0 || W == 0) return BGD_OK;
-    if (!d_out || !d_lut || !d_apply) return fail(BGD_ERR_INVALID, "bgmix_resize: null pointer");
-    if (!h_mean || !h_std) return fail(BGD_ERR_INVALID, "bgmix_resize: null mean/std");
-    if (P > 0 && (!d_pool || !d_bg_idx || !d_top || !d_left)) return fail(BGD_ERR_INVALID, "bgmix_resize: null pool argument");
+    if (!d_lut) return fail(BGD_ERR_INVALID, "bgmix_resize: null pointer");
+    if (P > 0 && !d_pool) return fail(BGD_ERR_INVALID, "bgmix_resize: null pool argument");
     if (P > 0 && (Hb < H || Wb < W))
         return fail(BGD_ERR_INVALID, "bgmix_resize: crop %lldx%lld larger than pool image %lldx%lld", (long long)H, (long long)W,
                     (long long)Hb, (long long)Wb);
     if (P > 0 && (Hb > INT32_MAX / 4 || Wb > INT32_MAX / 4 || 3 * Hb * Wb > INT32_MAX))
         return fail(BGD_ERR_INVALID, "bgmix_resize: pool images larger than 2^31 elements");
-    if (layout != BGD_LAYOUT_NTCHW && layout != BGD_LAYOUT_NCTHW && layout != BGD_LAYOUT_NTHWC)
-        return fail(BGD_ERR_INVALID, "bgmix_resize: unknown layout %d", layout);
-    if (!out_elem_bytes(out_dtype)) return fail(BGD_ERR_INVALID, "bgmix_resize: unknown output type %d", out_dtype);
 
     Workspace &ws = thread_workspace();
-    TailParams prm{};
     if (int rc = upload_geom(h_geom, 5, B, T, H, W, src_bytes, ws, &prm, stream)) return rc;
-    prm.src = d_src;
-    prm.pool = d_pool; prm.bg_idx = d_bg_idx; prm.top = d_top; prm.left = d_left; prm.apply = d_apply; prm.lut = d_lut;
-    prm.out = d_out;
+    prm.src = d_src; prm.pool = d_pool;
     prm.T = T; prm.H = H; prm.W = W; prm.P = P > 0 ? P : 1; prm.Hb = Hb; prm.Wb = Wb;
-    for (int c = 0; c < 3; ++c) { prm.mean[c] = h_mean[c]; prm.std[c] = h_std[c]; }
-    prm.w_fg = (float)(1.0 - alpha);
-    prm.w_bg = (float)alpha;
-    set_out_strides(layout, T, H, W, prm);
     dispatch_out(out_dtype, layout, [&](auto o, auto il) {
         using OutT = typename decltype(o)::type;
         constexpr bool IL = decltype(il)::value;
@@ -405,19 +379,18 @@ int launch_resize_blend(const uint8_t *d_src, int64_t src_bytes, const int64_t *
 int launch_resize_normalize(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t n, int64_t T, int64_t H,
                             int64_t W, const float *d_lut, int layout, int out_dtype, void *d_out, cudaStream_t stream)
 {
+    TailParams prm{};
     if (int rc = check_common(d_src, src_bytes, h_geom, n, T, H, W)) return rc;
     if (layout != BGD_LAYOUT_NTCHW && layout != BGD_LAYOUT_NTHWC)
         return fail(BGD_ERR_INVALID, "resize_crop_normalize: layout %d is not NTCHW or NTHWC", layout);
-    if (!out_elem_bytes(out_dtype)) return fail(BGD_ERR_INVALID, "resize_crop_normalize: unknown output type %d", out_dtype);
+    if (int rc = fill_blend_out("resize_crop_normalize", n, T, H, W, d_lut, layout, out_dtype, d_out, &prm.blend)) return rc;
     if (n == 0 || T == 0 || H == 0 || W == 0) return BGD_OK;
-    if (!d_out || !d_lut) return fail(BGD_ERR_INVALID, "resize_crop_normalize: null pointer");
+    if (!d_lut) return fail(BGD_ERR_INVALID, "resize_crop_normalize: null pointer");
 
     Workspace &ws = thread_workspace();
-    TailParams prm{};
     if (int rc = upload_geom(h_geom, 9, n, T, H, W, src_bytes, ws, &prm, stream)) return rc;
-    prm.src = d_src; prm.lut = d_lut; prm.out = d_out;
+    prm.src = d_src;
     prm.T = T; prm.H = H; prm.W = W;
-    set_out_strides(layout, T, H, W, prm);
     dispatch_out(out_dtype, layout, [&](auto o, auto il) {
         using OutT = typename decltype(o)::type;
         constexpr bool IL = decltype(il)::value;

@@ -324,6 +324,21 @@ def _check_lut(name: str, lut, dev) -> None:
              f"{name}: fg_lut must be float32 [3, 256] on the device")
 
 
+def _blend_tail(name: str, B: int, T: int, H: int, W: int, dev, bg_idx, top, left, apply, fg_lut, bg_mean, bg_std,
+                alpha: float, layout: str, out_dtype: Optional[torch.dtype]):
+    """Validates the arguments the uint8-foreground blends share and allocates the output.  Returns ``(out, keep, tail)``:
+    ``tail`` is the C ABI's argument run from ``d_bg_idx`` to ``d_out`` (the stream follows it), ``keep`` the tensors
+    its pointers point into, to hold until the call returns."""
+    out_dt = _out_spec(name, layout, out_dtype)
+    _check_draws(name, B, dev, bg_idx, top, left, apply)
+    _check_lut(name, fg_lut, dev)
+    keep = [x.contiguous() for x in (bg_idx, top, left, apply, fg_lut)]
+    out = torch.empty(_out_shape(B, T, H, W, layout), dtype=out_dt, device=dev)
+    tail = [x.data_ptr() for x in keep] + [_host3(bg_mean, "bg_mean"), _host3(bg_std, "bg_std"), float(alpha),
+                                           _cabi.OUT_LAYOUTS[layout], _OUT_DTYPES[out_dt], out.data_ptr()]
+    return out, keep, tail
+
+
 @torch.library.custom_op("bgdebias::bgmix_blend", mutates_args=(), device_types="cuda")
 def bgmix_blend(fg: torch.Tensor, bg_pool: torch.Tensor, bg_idx: torch.Tensor, top: torch.Tensor,
                 left: torch.Tensor, apply: torch.Tensor, fg_lut: torch.Tensor, bg_mean: torch.Tensor,
@@ -332,22 +347,16 @@ def bgmix_blend(fg: torch.Tensor, bg_pool: torch.Tensor, bg_idx: torch.Tensor, t
              "bgmix_blend: fg must be uint8 [B, T, H, W, 3]")
     _require(bg_pool.dim() == 4 and bg_pool.shape[1] == 3 and bg_pool.dtype in (torch.float32, torch.uint8),
              "bgmix_blend: bg_pool must be float32 or uint8 [P, 3, Hb, Wb]")
-    out_dt = _out_spec("bgmix_blend", layout, out_dtype)
     B, T, H, W, _ = fg.shape
     P, _, Hb, Wb = bg_pool.shape
     dev = fg.device
-    _check_draws("bgmix_blend", B, dev, bg_idx, top, left, apply)
-    _check_lut("bgmix_blend", fg_lut, dev)
+    out, _keep, tail = _blend_tail("bgmix_blend", B, T, H, W, dev, bg_idx, top, left, apply, fg_lut, bg_mean, bg_std, alpha,
+                                   layout, out_dtype)
     _require(bg_pool.device == dev, "bgmix_blend: bg_pool must be on the same device as fg")
     fg, bg_pool = fg.contiguous(), bg_pool.contiguous()
-    bg_idx, top, left, apply, fg_lut = (x.contiguous() for x in (bg_idx, top, left, apply, fg_lut))
-    out = torch.empty(_out_shape(B, T, H, W, layout), dtype=out_dt, device=dev)
     with torch.cuda.device(dev):
-        _cabi.check(_cabi.lib().bgd_bgmix_blend_out(
-            fg.data_ptr(), B, T, H, W, bg_pool.data_ptr(), int(bg_pool.dtype == torch.uint8), P, Hb, Wb, bg_idx.data_ptr(),
-            top.data_ptr(), left.data_ptr(), apply.data_ptr(), fg_lut.data_ptr(), _host3(bg_mean, "bg_mean"),
-            _host3(bg_std, "bg_std"), float(alpha), _cabi.OUT_LAYOUTS[layout], _OUT_DTYPES[out_dt], out.data_ptr(),
-            _stream_ptr(dev)))
+        _cabi.check(_cabi.lib().bgd_bgmix_blend_out(fg.data_ptr(), B, T, H, W, bg_pool.data_ptr(),
+                                                    int(bg_pool.dtype == torch.uint8), P, Hb, Wb, *tail, _stream_ptr(dev)))
     return out
 
 
@@ -360,12 +369,11 @@ def _(fg, bg_pool, bg_idx, top, left, apply, fg_lut, bg_mean, bg_std, alpha, lay
 # --------------------------------------------------------------------------- #
 # BG-mix over a ragged uint8 pool (pool.RaggedPool): Resize + RandomCrop + Normalize + blend in one launch
 # --------------------------------------------------------------------------- #
-def _check_ragged(name, B, dev, pool_bytes, slots, tables, bg_idx, top, left, apply):
+def _check_ragged(name, dev, pool_bytes, slots, tables):
     _require(pool_bytes.dtype == torch.uint8 and pool_bytes.dim() == 1, f"{name}: pool_bytes must be a flat uint8 buffer")
     _require(slots.dtype == torch.uint8 and slots.dim() == 1 and slots.numel() % 40 == 0 and slots.numel() > 0,
              f"{name}: slots must be the uint8 view of a bgd_ragged_slot table (40 bytes per image)")
     _require(tables.dtype == torch.int32 and tables.dim() == 1, f"{name}: tables must be int32")
-    _check_draws(name, B, dev, bg_idx, top, left, apply)
     for nm, t in (("pool_bytes", pool_bytes), ("slots", slots), ("tables", tables)):
         _require(t.device == dev, f"{name}: {nm} must be on {dev}")
     _require(slots.data_ptr() % 8 == 0, f"{name}: slots must be 8-byte aligned")
@@ -377,19 +385,15 @@ def bgmix_blend_ragged(fg: torch.Tensor, pool_bytes: torch.Tensor, slots: torch.
                        fg_lut: torch.Tensor, bg_mean: torch.Tensor, bg_std: torch.Tensor, alpha: float, layout: str,
                        out_dtype: Optional[torch.dtype] = None) -> torch.Tensor:
     _require(fg.dtype == torch.uint8 and fg.dim() == 5 and fg.shape[-1] == 3, "bgmix_blend_ragged: fg must be uint8 [B, T, H, W, 3]")
-    out_dt = _out_spec("bgmix_blend_ragged", layout, out_dtype)
     B, T, H, W, _ = fg.shape
     dev = fg.device
-    _check_ragged("bgmix_blend_ragged", B, dev, pool_bytes, slots, tables, bg_idx, top, left, apply)
-    _check_lut("bgmix_blend_ragged", fg_lut, dev)
-    fg = fg.contiguous()
-    bg_idx, top, left, apply, fg_lut, pool_bytes, slots, tables = (x.contiguous() for x in (bg_idx, top, left, apply, fg_lut, pool_bytes, slots, tables))
-    out = torch.empty(_out_shape(B, T, H, W, layout), dtype=out_dt, device=dev)
+    _check_ragged("bgmix_blend_ragged", dev, pool_bytes, slots, tables)
+    out, _keep, tail = _blend_tail("bgmix_blend_ragged", B, T, H, W, dev, bg_idx, top, left, apply, fg_lut, bg_mean, bg_std,
+                                   alpha, layout, out_dtype)
+    fg, pool_bytes, slots, tables = (x.contiguous() for x in (fg, pool_bytes, slots, tables))
     with torch.cuda.device(dev):
-        _cabi.check(_cabi.lib().bgd_bgmix_blend_ragged_out(
-            fg.data_ptr(), B, T, H, W, pool_bytes.data_ptr(), slots.data_ptr(), slots.numel() // 40, tables.data_ptr(),
-            bg_idx.data_ptr(), top.data_ptr(), left.data_ptr(), apply.data_ptr(), fg_lut.data_ptr(), _host3(bg_mean, "bg_mean"),
-            _host3(bg_std, "bg_std"), float(alpha), _cabi.OUT_LAYOUTS[layout], _OUT_DTYPES[out_dt], out.data_ptr(), _stream_ptr(dev)))
+        _cabi.check(_cabi.lib().bgd_bgmix_blend_ragged_out(fg.data_ptr(), B, T, H, W, pool_bytes.data_ptr(), slots.data_ptr(),
+                                                           slots.numel() // 40, tables.data_ptr(), *tail, _stream_ptr(dev)))
     return out
 
 
@@ -397,34 +401,6 @@ def bgmix_blend_ragged(fg: torch.Tensor, pool_bytes: torch.Tensor, slots: torch.
 def _(fg, pool_bytes, slots, tables, bg_idx, top, left, apply, fg_lut, bg_mean, bg_std, alpha, layout, out_dtype=None):
     B, T, H, W, _ = fg.shape
     return fg.new_empty(_out_shape(B, T, H, W, layout), dtype=_out_spec("bgmix_blend_ragged", layout, out_dtype))
-
-
-@torch.library.custom_op("bgdebias::bgmix_blend_ragged_normfg", mutates_args=(), device_types="cuda")
-def bgmix_blend_ragged_normfg(fg_norm: torch.Tensor, pool_bytes: torch.Tensor, slots: torch.Tensor, tables: torch.Tensor,
-                              bg_idx: torch.Tensor, top: torch.Tensor, left: torch.Tensor, apply: torch.Tensor,
-                              bg_mean: torch.Tensor, bg_std: torch.Tensor, alpha: float, layout: str) -> torch.Tensor:
-    """Ragged-pool blend for a foreground that is already normalised (fp32 ``[B, T, 3, H, W]``)."""
-    _require(fg_norm.dtype == torch.float32 and fg_norm.dim() == 5 and fg_norm.shape[2] == 3,
-             "bgmix_blend_ragged_normfg: fg_norm must be float32 [B, T, 3, H, W]")
-    _require(layout in _cabi.LAYOUTS, f"bgmix_blend_ragged_normfg: layout must be one of {sorted(_cabi.LAYOUTS)}")
-    B, T, _, H, W = fg_norm.shape
-    dev = fg_norm.device
-    _check_ragged("bgmix_blend_ragged_normfg", B, dev, pool_bytes, slots, tables, bg_idx, top, left, apply)
-    fg_norm = fg_norm.contiguous()
-    bg_idx, top, left, apply, pool_bytes, slots, tables = (x.contiguous() for x in (bg_idx, top, left, apply, pool_bytes, slots, tables))
-    out = torch.empty(_out_shape(B, T, H, W, layout), dtype=torch.float32, device=dev)
-    with torch.cuda.device(dev):
-        _cabi.check(_cabi.lib().bgd_bgmix_blend_ragged_normfg_f32(
-            fg_norm.data_ptr(), B, T, H, W, pool_bytes.data_ptr(), slots.data_ptr(), slots.numel() // 40, tables.data_ptr(),
-            bg_idx.data_ptr(), top.data_ptr(), left.data_ptr(), apply.data_ptr(), _host3(bg_mean, "bg_mean"),
-            _host3(bg_std, "bg_std"), float(alpha), _cabi.LAYOUTS[layout], out.data_ptr(), _stream_ptr(dev)))
-    return out
-
-
-@bgmix_blend_ragged_normfg.register_fake
-def _(fg_norm, pool_bytes, slots, tables, bg_idx, top, left, apply, bg_mean, bg_std, alpha, layout):
-    B, T, _, H, W = fg_norm.shape
-    return fg_norm.new_empty(_out_shape(B, T, H, W, layout))
 
 
 # --------------------------------------------------------------------------- #
@@ -486,20 +462,15 @@ def bgmix_resize_blend(src: torch.Tensor, geom: torch.Tensor, T: int, H: int, W:
     B = g.shape[0]
     _require(bg_pool.dim() == 4 and bg_pool.shape[1] == 3 and bg_pool.dtype in (torch.float32, torch.uint8),
              "bgmix_resize_blend: bg_pool must be float32 or uint8 [P, 3, Hb, Wb]")
-    out_dt = _out_spec("bgmix_resize_blend", layout, out_dtype)
     P, _, Hb, Wb = bg_pool.shape
     dev = src.device
-    _check_draws("bgmix_resize_blend", B, dev, bg_idx, top, left, apply)
-    _check_lut("bgmix_resize_blend", fg_lut, dev)
+    out, _keep, tail = _blend_tail("bgmix_resize_blend", B, T, H, W, dev, bg_idx, top, left, apply, fg_lut, bg_mean, bg_std,
+                                   alpha, layout, out_dtype)
     _require(bg_pool.device == dev, "bgmix_resize_blend: bg_pool must be on the same device as src")
     bg_pool = bg_pool.contiguous()
-    bg_idx, top, left, apply, fg_lut = (x.contiguous() for x in (bg_idx, top, left, apply, fg_lut))
-    out = torch.empty(_out_shape(B, T, H, W, layout), dtype=out_dt, device=dev)
     with torch.cuda.device(dev):
-        _cabi.check(_cabi.lib().bgd_bgmix_resize_blend_out(
-            src.data_ptr(), src.numel(), gptr, B, T, H, W, bg_pool.data_ptr(), int(bg_pool.dtype == torch.uint8), P, Hb, Wb,
-            bg_idx.data_ptr(), top.data_ptr(), left.data_ptr(), apply.data_ptr(), fg_lut.data_ptr(), _host3(bg_mean, "bg_mean"),
-            _host3(bg_std, "bg_std"), float(alpha), _cabi.OUT_LAYOUTS[layout], _OUT_DTYPES[out_dt], out.data_ptr(), _stream_ptr(dev)))
+        _cabi.check(_cabi.lib().bgd_bgmix_resize_blend_out(src.data_ptr(), src.numel(), gptr, B, T, H, W, bg_pool.data_ptr(),
+                                                           int(bg_pool.dtype == torch.uint8), P, Hb, Wb, *tail, _stream_ptr(dev)))
     return out
 
 

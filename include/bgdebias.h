@@ -169,18 +169,10 @@ int bgd_bgmix_blend_f32(const uint8_t *d_fg, int64_t B, int64_t T, int64_t H, in
                         const float *h_bg_std, double alpha, int layout, float *d_out,
                         void *stream);
 
-/* Same with a uint8 background pool [P][3][Hb][Wb] (values already at crop scale, e.g. a pool
- * whose images need no Resize); 4x less pool memory and traffic. */
-int bgd_bgmix_blend_u8pool_f32(const uint8_t *d_fg, int64_t B, int64_t T, int64_t H, int64_t W,
-                               const uint8_t *d_bg_pool, int64_t P, int64_t Hb, int64_t Wb,
-                               const int32_t *d_bg_idx, const int32_t *d_top, const int32_t *d_left,
-                               const uint8_t *d_apply, const float *d_fg_lut,
-                               const float *h_bg_mean, const float *h_bg_std, double alpha,
-                               int layout, float *d_out, void *stream);
-
-/* bgd_bgmix_blend_f32 / bgd_bgmix_blend_u8pool_f32 with a choice of output: replaces the same reference code
+/* bgd_bgmix_blend_f32 with a choice of pool and output: replaces the same reference code
  * (libs/loader/comix_loader.py:138-145 with :72-75, and config ..._bgmix_plus_randAug.py:137-138) and hands the model
- * the tensor it consumes.  d_bg_pool is fp32 (pool_is_u8 == 0) or uint8 (pool_is_u8 != 0) [P][3][Hb][Wb];
+ * the tensor it consumes.  d_bg_pool is fp32 (pool_is_u8 == 0) or uint8 (pool_is_u8 != 0) [P][3][Hb][Wb]; a uint8 pool
+ * (values already at crop scale, images that need no Resize) takes 4x less memory and traffic;
  *   layout     BGD_LAYOUT_NTCHW, BGD_LAYOUT_NCTHW or BGD_LAYOUT_NTHWC ([B][T][H][W][3])
  *   out_dtype  BGD_OUT_F32, BGD_OUT_BF16 or BGD_OUT_F16: element type of d_out
  * Every other argument and the arithmetic as bgd_bgmix_blend_f32. */
@@ -262,13 +254,6 @@ int bgd_bgmix_blend_ragged_out(const uint8_t *d_fg, int64_t B, int64_t T, int64_
                                const int32_t *d_left, const uint8_t *d_apply, const float *d_fg_lut,
                                const float *h_bg_mean, const float *h_bg_std, double alpha, int layout,
                                int out_dtype, void *d_out, void *stream);
-
-/* Same for a foreground that is already normalised (fp32 [B][T][3][H][W], as bgd_bgmix_blend_normfg_f32). */
-int bgd_bgmix_blend_ragged_normfg_f32(const float *d_fg_norm, int64_t B, int64_t T, int64_t H, int64_t W,
-                                      const uint8_t *d_pool, const bgd_ragged_slot *d_slots, int64_t P,
-                                      const int32_t *d_tables, const int32_t *d_bg_idx, const int32_t *d_top,
-                                      const int32_t *d_left, const uint8_t *d_apply, const float *h_bg_mean,
-                                      const float *h_bg_std, double alpha, int layout, float *d_out, void *stream);
 
 /* ---- RandomResizedCrop of a batch of frames (simulated-camera-motion extraction) --------------------
  * Replaces, for every frame of many frame folders in one launch,
