@@ -30,6 +30,11 @@ Evaluation datasets (``test_mode=True``: val, test, the herding feature pass, th
 ``device_mix=True`` their pipeline stops after ``RawFrameDecode`` and ``device_test_pipeline`` takes the steps it no longer
 runs -- ``Resize(scale=(-1, S))``, ``CenterCrop`` or ``ThreeCrop``, ``Normalize`` and ``FormatShape('NCHW')``, see
 :class:`EvalPipeline` -- which ``device_finish`` runs on the native-size uint8 frames in one launch.
+
+Training datasets without a host-only step between decode and crop (no ``RandAugment``) can stop after ``RawFrameDecode``
+as well: ``device_train_pipeline`` takes ``Resize(scale=(-1, S))``, ``MultiScaleCrop``, the final ``Resize``,
+``Normalize`` and ``FormatShape('NCHW')`` (see :class:`TrainPipeline`); the worker draws the crop where MultiScaleCrop
+would, and ``device_finish`` runs both resizes inside the blend launch.
 """
 from __future__ import annotations
 
@@ -167,6 +172,66 @@ def draw_crop(h: int, w: int, crop) -> tuple:
     return top, left
 
 
+def _steps_in_order(who: str, steps: Sequence[dict], expected: tuple) -> List[dict]:
+    """The step dicts, checked to be of the ``expected`` types (a tuple of alternatives per position), in that order."""
+    steps = [dict(s) for s in steps]
+    for i, step in enumerate(steps):
+        if i >= len(expected) or step.get('type') not in expected[i]:
+            raise ValueError(f"{who}: step {i}, {step.get('type')!r}, has no device form (expected "
+                             f"{', '.join(' or '.join(e) for e in expected)}, in this order)")
+    if len(steps) < len(expected):
+        raise ValueError(f"{who}: the {' or '.join(expected[len(steps)])} step is missing")
+    return steps
+
+
+def _only(step: dict, **allowed) -> None:
+    """Keys other than ``type`` must be in ``allowed``; those with a non-None value there must equal it."""
+    for k, v in step.items():
+        if k == 'type':
+            continue
+        if k not in allowed or (allowed[k] is not None and v != allowed[k]):
+            raise ValueError(f"{step['type']}: {k}={v!r} has no device form")
+
+
+def _short_side(resize: dict) -> int:
+    """S of a ``Resize(scale=(-1, S))`` (or ``(S, -1)``) step, keep_ratio and bilinear."""
+    _only(resize, scale=None, keep_ratio=True, interpolation='bilinear', lazy=False)
+    scale = resize.get('scale')
+    if not (isinstance(scale, (tuple, list)) and len(scale) == 2 and min(scale) == -1 and max(scale) > 0
+            and all(isinstance(v, int) for v in scale)):
+        raise ValueError(f"Resize: only scale=(-1, S) or (S, -1) has a device form (got scale={scale!r})")
+    return int(max(scale))
+
+
+def rescale_short_side(h: int, w: int, short_side: int) -> tuple:
+    """``(Hr, Wr)`` of mmaction's ``Resize(scale=(-1, S))`` for an ``h x w`` frame: ``mmcv.rescale_size((w, h), (inf, S))``,
+    ``f = S / min(h, w)``, ``(int(w * f + 0.5), int(h * f + 0.5))``."""
+    f = short_side / min(h, w)
+    return int(h * f + 0.5), int(w * f + 0.5)
+
+
+def _size_hw(step: dict, key: str) -> tuple:
+    """``(h, w)`` of a size given as an int or mmaction's ``(w, h)`` pair."""
+    v = step.get(key)
+    w, h = (v, v) if isinstance(v, int) else tuple(v) if isinstance(v, (tuple, list)) and len(v) == 2 else (None, None)
+    if not (isinstance(w, int) and isinstance(h, int) and w > 0 and h > 0):
+        raise ValueError(f"{step['type']}: {key} must be a positive int or (w, h) (got {v!r})")
+    return h, w
+
+
+def _normalize(norm: dict) -> tuple:
+    _only(norm, mean=None, std=None, to_bgr=False, adjust_magnitude=False)
+    if len(norm.get('mean', ())) != 3 or len(norm.get('std', ())) != 3:
+        raise ValueError("Normalize: mean and std must have 3 values (RGB)")
+    return tuple(float(m) for m in norm['mean']), tuple(float(v) for v in norm['std'])
+
+
+def _format_nchw(fmt: dict) -> None:
+    _only(fmt, input_format=None, collapse=False)
+    if fmt.get('input_format') != 'NCHW':
+        raise ValueError(f"FormatShape: only input_format='NCHW' has a device form (got {fmt.get('input_format')!r})")
+
+
 class EvalPipeline:
     """The tail of an evaluation pipeline that the device runs on decoded uint8 frames (``resize_crop_normalize``):
 
@@ -193,43 +258,13 @@ class EvalPipeline:
     """
 
     def __init__(self, steps: Sequence[dict]):
-        steps = [dict(s) for s in steps]
-        expected = (('Resize',), ('CenterCrop', 'ThreeCrop'), ('Normalize',), ('FormatShape',))
-        for i, step in enumerate(steps):
-            if i >= len(expected) or step.get('type') not in expected[i]:
-                raise ValueError(f"device_test_pipeline: step {i}, {step.get('type')!r}, has no device form (expected "
-                                 "Resize, CenterCrop or ThreeCrop, Normalize, FormatShape, in this order)")
-        if len(steps) < len(expected):
-            raise ValueError(f"device_test_pipeline: the {' or '.join(expected[len(steps)])} step is missing")
-        resize, crop, norm, fmt = steps
-        self._only(resize, scale=None, keep_ratio=True, interpolation='bilinear', lazy=False)
-        scale = resize.get('scale')
-        if not (isinstance(scale, (tuple, list)) and len(scale) == 2 and min(scale) == -1 and max(scale) > 0
-                and all(isinstance(v, int) for v in scale)):
-            raise ValueError(f"Resize: only scale=(-1, S) or (S, -1) has a device form (got scale={scale!r})")
-        self.short_side = int(max(scale))
-        self._only(crop, crop_size=None, lazy=False)
-        cs = crop.get('crop_size')
-        cw, ch = (cs, cs) if isinstance(cs, int) else tuple(cs)
-        if not (isinstance(cw, int) and isinstance(ch, int) and cw > 0 and ch > 0):
-            raise ValueError(f"{crop['type']}: crop_size must be a positive int or (w, h) (got {cs!r})")
-        self.three, self.crop_hw = crop['type'] == 'ThreeCrop', (ch, cw)
-        self._only(norm, mean=None, std=None, to_bgr=False, adjust_magnitude=False)
-        if len(norm.get('mean', ())) != 3 or len(norm.get('std', ())) != 3:
-            raise ValueError("Normalize: mean and std must have 3 values (RGB)")
-        self.mean, self.std = tuple(float(m) for m in norm['mean']), tuple(float(v) for v in norm['std'])
-        self._only(fmt, input_format=None, collapse=False)
-        if fmt.get('input_format') != 'NCHW':
-            raise ValueError(f"FormatShape: only input_format='NCHW' has a device form (got {fmt.get('input_format')!r})")
-
-    @staticmethod
-    def _only(step: dict, **allowed) -> None:
-        """Keys other than ``type`` must be in ``allowed``; those with a non-None value there must equal it."""
-        for k, v in step.items():
-            if k == 'type':
-                continue
-            if k not in allowed or (allowed[k] is not None and v != allowed[k]):
-                raise ValueError(f"{step['type']}: {k}={v!r} has no device form")
+        resize, crop, norm, fmt = _steps_in_order('device_test_pipeline', steps,
+                                                  (('Resize',), ('CenterCrop', 'ThreeCrop'), ('Normalize',), ('FormatShape',)))
+        self.short_side = _short_side(resize)
+        _only(crop, crop_size=None, lazy=False)
+        self.three, self.crop_hw = crop['type'] == 'ThreeCrop', _size_hw(crop, 'crop_size')
+        self.mean, self.std = _normalize(norm)
+        _format_nchw(fmt)
 
     @property
     def n_crops(self) -> int:
@@ -237,8 +272,7 @@ class EvalPipeline:
 
     def windows(self, h: int, w: int) -> tuple:
         """``(Hr, Wr, [(top, left), ...])`` for a native ``h x w`` frame: the resized size and every crop's window."""
-        f = self.short_side / min(h, w)
-        Wr, Hr = int(w * f + 0.5), int(h * f + 0.5)
+        Hr, Wr = rescale_short_side(h, w, self.short_side)
         ch, cw = self.crop_hw
         if not self.three:
             if ch > Hr or cw > Wr:
@@ -262,13 +296,100 @@ class EvalPipeline:
         return torch.tensor(rows, dtype=torch.int64).reshape(-1, 9)
 
 
+class TrainPipeline:
+    """The geometric tail of a training pipeline that the device runs on decoded uint8 frames, fused with the BG-mix blend:
+
+        Resize(scale=(-1, S)) -> MultiScaleCrop(...) -> Resize(scale=(W, H), keep_ratio=False) -> Normalize -> FormatShape('NCHW')
+
+    ``steps`` are the mmaction step dicts of these five, in this order, moved verbatim out of ``train_pipeline``.  Any other
+    step, or another form of these (``lazy=True``, another interpolation, ``to_bgr=True``, NCTHW, ...), raises
+    ``ValueError`` naming the step; such a config keeps its CPU pipeline.  A pipeline with a host-only step between
+    ``RawFrameDecode`` and ``MultiScaleCrop`` (``RandAugment``) cannot use this route.
+
+    The rules restate mmaction2 0.x ``mmaction/datasets/pipelines/augmentations.py`` (``Resize``, ``MultiScaleCrop``,
+    ``Normalize``) and mmcv 1.x ``rescale_size`` / ``imresize``; neither package is a dependency:
+
+    * Resize(scale=(-1, S)): :func:`rescale_short_side`, as :class:`EvalPipeline`; pixels ``cv2.resize(img, (Wr, Hr),
+      interpolation=cv2.INTER_LINEAR)``.
+    * MultiScaleCrop(input_size, scales=(1,), max_wh_scale_gap=1, random_crop=False, num_fixed_crops=5), on the Hr x Wr
+      frame: ``base = min(Hr, Wr)``, ``crop_sizes = [int(base * s) for s in scales]``; the candidates are ``[w, h]`` for
+      every ``(i, h)``, ``(j, w)`` of ``enumerate(crop_sizes)`` (h outer, w inner) with ``abs(i - j) <= max_wh_scale_gap``;
+      ``crop_size = random.choice(candidates)`` (Python's ``random``); each side with ``abs(side - input_size[k]) < 3``
+      becomes ``input_size[k]`` (``input_size`` an int or ``(w, h)``, mmaction's ``_pair``).  The offset: with
+      ``random_crop``, ``x0 = random.randint(0, Wr - cw)`` then ``y0 = random.randint(0, Hr - ch)``; otherwise, with
+      ``w_step = (Wr - cw) // 4`` and ``h_step = (Hr - ch) // 4``, ``(x0, y0) = random.choice`` of the (x, y) offsets
+      ``(0, 0), (4w, 0), (0, 4h), (4w, 4h), (2w, 2h)`` and, for ``num_fixed_crops=13``, then ``(0, 2h), (4w, 2h), (2w, 4h),
+      (2w, 0), (w, h), (3w, h), (w, 3h), (3w, 3h)`` (w = w_step, h = h_step).  The crop is ``img[y0:y0 + ch, x0:x0 + cw]``.
+    * Resize(scale=(W, H), keep_ratio=False): ``cv2.resize(crop, (W, H), interpolation=cv2.INTER_LINEAR)``.
+    * Normalize, ``to_bgr=False``: :func:`ops.make_fg_lut` of ``(mean, std)``.  FormatShape('NCHW'): ``[T, 3, H, W]``.
+
+    The draws happen on the host (:meth:`draw`, in the worker, where the CPU pipeline would make them); the pixels of all
+    three geometric steps are one launch with the blend (``ops.TWO_STAGE_COLS``).
+    """
+
+    def __init__(self, steps: Sequence[dict]):
+        resize, msc, final, norm, fmt = _steps_in_order(
+            'device_train_pipeline', steps, (('Resize',), ('MultiScaleCrop',), ('Resize',), ('Normalize',), ('FormatShape',)))
+        self.short_side = _short_side(resize)
+        _only(msc, input_size=None, scales=None, max_wh_scale_gap=None, random_crop=None, num_fixed_crops=None, lazy=False)
+        self.input_hw = _size_hw(msc, 'input_size')
+        scales = msc.get('scales', (1,))
+        if not (isinstance(scales, (tuple, list)) and scales and all(isinstance(v, (int, float)) and 0 < v for v in scales)):
+            raise ValueError(f"MultiScaleCrop: scales must be a non-empty tuple of positive numbers (got {scales!r})")
+        self.scales = tuple(scales)
+        self.max_wh_scale_gap = msc.get('max_wh_scale_gap', 1)
+        if not isinstance(self.max_wh_scale_gap, int) or self.max_wh_scale_gap < 0:
+            raise ValueError(f"MultiScaleCrop: max_wh_scale_gap must be an int >= 0 (got {self.max_wh_scale_gap!r})")
+        self.random_crop = msc.get('random_crop', False)
+        if not isinstance(self.random_crop, bool):
+            raise ValueError(f"MultiScaleCrop: random_crop must be a bool (got {self.random_crop!r})")
+        self.num_fixed_crops = msc.get('num_fixed_crops', 5)
+        if self.num_fixed_crops not in (5, 13):
+            raise ValueError(f"MultiScaleCrop: num_fixed_crops must be 5 or 13 (got {self.num_fixed_crops!r})")
+        _only(final, scale=None, keep_ratio=False, interpolation='bilinear', lazy=False)
+        if final.get('keep_ratio', True) is not False:
+            raise ValueError("Resize: keep_ratio must be False in the Resize after MultiScaleCrop")
+        self.out_hw = _size_hw(final, 'scale')
+        self.mean, self.std = _normalize(norm)
+        _format_nchw(fmt)
+
+    def draw(self, h: int, w: int) -> tuple:
+        """``(Hr, Wr, y0, x0, ch, cw)`` for a native ``h x w`` frame, drawn from Python's ``random`` as MultiScaleCrop draws."""
+        Hr, Wr = rescale_short_side(h, w, self.short_side)
+        base = min(Hr, Wr)
+        crop_sizes = [int(base * s) for s in self.scales]
+        candidates = [[cw, ch] for i, ch in enumerate(crop_sizes) for j, cw in enumerate(crop_sizes)
+                      if abs(i - j) <= self.max_wh_scale_gap]
+        size = random.choice(candidates)
+        in_wh = (self.input_hw[1], self.input_hw[0])
+        for k in range(2):
+            if abs(size[k] - in_wh[k]) < 3:
+                size[k] = in_wh[k]
+        cw, ch = size
+        if ch > Hr or cw > Wr or ch < 1 or cw < 1:
+            raise ValueError(f"MultiScaleCrop: crop {ch}x{cw} does not fit the resized frame {Hr}x{Wr}")
+        if self.random_crop:
+            x0 = random.randint(0, Wr - cw)
+            y0 = random.randint(0, Hr - ch)
+        else:
+            ws, hs = (Wr - cw) // 4, (Hr - ch) // 4
+            offsets = [(0, 0), (4 * ws, 0), (0, 4 * hs), (4 * ws, 4 * hs), (2 * ws, 2 * hs)]
+            if self.num_fixed_crops == 13:
+                offsets += [(0, 2 * hs), (4 * ws, 2 * hs), (2 * ws, 4 * hs), (2 * ws, 0), (ws, hs), (3 * ws, hs), (ws, 3 * hs),
+                            (3 * ws, 3 * hs)]
+            x0, y0 = random.choice(offsets)
+        return Hr, Wr, y0, x0, ch, cw
+
+
 @_register(_DATASETS)
 class BackgroundMixDataset(_Base):
     """Same signature as the reference class (libs/loader/comix_loader.py:16-45) plus four
     keyword-only extensions: ``device`` (CUDA device of the pool and the blend), ``device_mix``
     (see module docstring), ``bg_reader`` (callable ``path -> uint8 [3,h,w]``, defaults to
-    ``torchvision.io.read_image(mode=RGB)`` as in the reference) and ``device_test_pipeline`` (the
-    step dicts of :class:`EvalPipeline`, required by ``device_mix=True`` with ``test_mode=True``)."""
+    ``torchvision.io.read_image(mode=RGB)`` as in the reference), ``device_test_pipeline`` (the
+    step dicts of :class:`EvalPipeline`, required by ``device_mix=True`` with ``test_mode=True``) and
+    ``device_train_pipeline`` (the step dicts of :class:`TrainPipeline`, for ``device_mix=True`` training
+    datasets whose pipeline then stops after ``RawFrameDecode``)."""
 
     def __init__(self,
                  ann_file,
@@ -301,13 +422,23 @@ class BackgroundMixDataset(_Base):
                  device_mix=False,
                  bg_reader: Optional[Callable] = None,
                  device_test_pipeline: Optional[Sequence[dict]] = None,
+                 device_train_pipeline: Optional[Sequence[dict]] = None,
                  **kwargs):
+        if device_train_pipeline is not None:
+            if device_test_pipeline is not None:
+                raise ValueError("device_train_pipeline and device_test_pipeline are exclusive: a dataset trains or evaluates")
+            if not device_mix or test_mode:
+                raise ValueError("device_train_pipeline is the training tail of device_mix=True with test_mode=False")
+            if with_randAug:
+                raise ValueError("device_train_pipeline cannot run with with_randAug=True: the gate reads the flag RandAugment "
+                                 "sets, and RandAugment runs on the host between RawFrameDecode and MultiScaleCrop")
         if device_test_pipeline is not None and not (device_mix and test_mode):
             raise ValueError("device_test_pipeline is the evaluation tail of device_mix=True with test_mode=True")
         if device_mix and test_mode and device_test_pipeline is None:
             raise ValueError("device_mix=True with test_mode=True needs device_test_pipeline: the Resize, crop, Normalize "
                              "and FormatShape steps moved out of test_pipeline")
         self._eval = EvalPipeline(device_test_pipeline) if device_test_pipeline is not None else None
+        self._train = TrainPipeline(device_train_pipeline) if device_train_pipeline is not None else None
         super().__init__(ann_file, pipeline, data_prefix, test_mode, filename_tmpl, with_offset, multi_class,
                          num_classes, start_index, modality, sample_by_class, power, dynamic_length, **kwargs)
         bg_dir = osp.realpath(bg_dir)                 # same reason as the reference, comix_loader.py:61-68
@@ -316,6 +447,9 @@ class BackgroundMixDataset(_Base):
         self.bg_dir.mkdir(exist_ok=True, parents=True)
         self.bg_resize = bg_resize
         self.bg_crop_size = tuple(bg_crop_size) if not isinstance(bg_crop_size, int) else (bg_crop_size, bg_crop_size)
+        if self._train is not None and self._train.out_hw != self.bg_crop_size:
+            raise ValueError(f"device_train_pipeline: the final Resize gives {self._train.out_hw} (h, w), bg_crop_size is "
+                             f"{self.bg_crop_size}; the blend needs them equal")
         self.bg_mean = [float(m) for m in bg_mean]
         self.bg_std = [float(s) for s in bg_std]
         self.alpha = alpha
@@ -436,6 +570,11 @@ class BackgroundMixDataset(_Base):
     def prepare_train_frames(self, idx):
         """Prepare the frames for training given the index (comix_loader.py:105-124)."""
         result = super().prepare_train_frames(idx)
+        if self._train is not None:
+            # MultiScaleCrop's draws, where the CPU pipeline makes them: before the gate's random.random()
+            imgs = result['imgs']
+            h, w = (imgs[0].shape[0], imgs[0].shape[1]) if isinstance(imgs, (list, tuple)) else tuple(imgs.shape[1:3])
+            result['fg_window'] = self._train.draw(int(h), int(w))
         result['bg_idx'] = -1
         if self.device_mix:
             result['bg_top'], result['bg_left'], result['bg_apply'] = 0, 0, 0
@@ -626,17 +765,25 @@ class BackgroundMixDataset(_Base):
         :meth:`device_finish` in the training process; with ``pin_memory=True`` the batch travels as uint8,
         a quarter of the bytes of the reference's fp32 batch (libs/cil/cil.py:203-210).
 
+        Samples of a ``device_train_pipeline`` dataset carry native-size frames: they are packed with ``ops.pack_clips``
+        and ``fg_geom`` is the ``[B, 11]`` two-stage geometry (``ops.TWO_STAGE_COLS``) of their MultiScaleCrop draws.
+
         Samples without draws (``test_mode=True``) make an evaluation batch: the native-size uint8 frames packed with
         ``ops.pack_clips`` (sizes may differ per video) and ``label``, for the eval route of :meth:`device_finish`."""
         clips = [torch.as_tensor(np.stack(s['imgs']) if isinstance(s['imgs'], (list, tuple)) else s['imgs']) for s in samples]
         out = {}
-        if 'bg_idx' not in samples[0]:
+        if 'fg_window' in samples[0]:
+            # device_train_pipeline: native-size frames and each sample's (Hr, Wr, y0, x0, ch, cw), the two-stage geometry
+            out['imgs'], g5 = ops.pack_clips(clips)
+            out['fg_geom'] = torch.cat([g5, torch.tensor([s['fg_window'] for s in samples], dtype=torch.int64)], 1)
+            out['fg_frames'] = int(clips[0].shape[0])
+        elif 'bg_idx' not in samples[0]:
             out['imgs'], out['fg_geom'] = ops.pack_clips(clips)
             out['fg_frames'] = int(clips[0].shape[0])
             if 'label' in samples[0]:
                 out['label'] = torch.stack([torch.as_tensor(s['label']) for s in samples])
             return out
-        if all(c.shape == clips[0].shape for c in clips):
+        elif all(c.shape == clips[0].shape for c in clips):
             out['imgs'] = torch.stack(clips)
         else:
             # the pipeline stopped before Resize((224, 224), keep_ratio=False) (config :136): MultiScaleCrop's crops differ in
@@ -680,8 +827,14 @@ class BackgroundMixDataset(_Base):
             # random-frame mode and no sample of the batch was mixed: a placeholder frame the blend never reads
             batch = dict(batch, bg_imgs=[torch.zeros((3, *self.bg_crop_size), dtype=torch.uint8)],
                          bg_slot=torch.zeros(len(batch['bg_idx']), dtype=torch.int32))
+        fg_geom = batch.get('fg_geom')
+        norm = {}
+        if fg_geom is not None and fg_geom.shape[1] == len(ops.TWO_STAGE_COLS):
+            if self._train is None:
+                raise ValueError("a batch with the two-stage geometry needs a dataset built with device_train_pipeline")
+            norm = dict(img_mean=self._train.mean, img_std=self._train.std)
         out['imgs'] = self.mix_batch_on_device(batch['imgs'], batch['bg_idx'], batch['bg_top'], batch['bg_left'],
-                                               batch['bg_apply'], layout=layout, fg_geom=batch.get('fg_geom'),
+                                               batch['bg_apply'], layout=layout, fg_geom=fg_geom, **norm,
                                                fg_frames=batch.get('fg_frames'), bg_imgs=batch.get('bg_imgs'),
                                                bg_slot=batch.get('bg_slot'), dtype=dtype, memory_format=memory_format)
         return out

@@ -677,7 +677,15 @@ int bgd_resize_bilinear_u8(const uint8_t *d_src, int64_t src_bytes, const int64_
 {
     DeviceProps dp;
     if (int rc = current_device_props(&dp)) return rc;
-    return launch_resize_u8(d_src, src_bytes, h_geom, B, T, H, W, d_out, static_cast<cudaStream_t>(stream));
+    return launch_resize_u8(d_src, src_bytes, h_geom, 5, B, T, H, W, d_out, static_cast<cudaStream_t>(stream));
+}
+
+int bgd_resize_bilinear_cols_u8(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int geom_cols, int64_t B,
+                                int64_t T, int64_t H, int64_t W, uint8_t *d_out, void *stream)
+{
+    DeviceProps dp;
+    if (int rc = current_device_props(&dp)) return rc;
+    return launch_resize_u8(d_src, src_bytes, h_geom, geom_cols, B, T, H, W, d_out, static_cast<cudaStream_t>(stream));
 }
 
 int bgd_bgmix_resize_blend_f32(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t B, int64_t T, int64_t H,
@@ -697,10 +705,21 @@ int bgd_bgmix_resize_blend_out(const uint8_t *d_src, int64_t src_bytes, const in
                                const float *d_fg_lut, const float *h_bg_mean, const float *h_bg_std, double alpha, int layout,
                                int out_dtype, void *d_out, void *stream)
 {
+    return bgd_bgmix_resize_blend_cols_out(d_src, src_bytes, h_geom, 5, B, T, H, W, d_bg_pool, pool_is_u8, P, Hb, Wb, d_bg_idx,
+                                           d_top, d_left, d_apply, d_fg_lut, h_bg_mean, h_bg_std, alpha, layout, out_dtype, d_out,
+                                           stream);
+}
+
+int bgd_bgmix_resize_blend_cols_out(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int geom_cols, int64_t B,
+                                    int64_t T, int64_t H, int64_t W, const void *d_bg_pool, int pool_is_u8, int64_t P, int64_t Hb,
+                                    int64_t Wb, const int32_t *d_bg_idx, const int32_t *d_top, const int32_t *d_left,
+                                    const uint8_t *d_apply, const float *d_fg_lut, const float *h_bg_mean,
+                                    const float *h_bg_std, double alpha, int layout, int out_dtype, void *d_out, void *stream)
+{
     DeviceProps dp;
     if (int rc = current_device_props(&dp)) return rc;
-    return launch_resize_blend(d_src, src_bytes, h_geom, B, T, H, W, d_bg_pool, pool_is_u8 != 0, P, Hb, Wb, d_bg_idx, d_top,
-                               d_left, d_apply, d_fg_lut, h_bg_mean, h_bg_std, alpha, layout, out_dtype, d_out,
+    return launch_resize_blend(d_src, src_bytes, h_geom, geom_cols, B, T, H, W, d_bg_pool, pool_is_u8 != 0, P, Hb, Wb, d_bg_idx,
+                               d_top, d_left, d_apply, d_fg_lut, h_bg_mean, h_bg_std, alpha, layout, out_dtype, d_out,
                                static_cast<cudaStream_t>(stream));
 }
 
@@ -750,7 +769,7 @@ int bgd_bgmix_resize_blend_f32_host(const uint8_t *h_src, int64_t src_bytes, con
     if (int rc = stage_host_blend("bgmix_resize", h_src, (size_t)src_bytes, B, H, W, P, Hb, Wb, h_bg_idx, h_top, h_left, h_apply,
                                   device, &g))
         return rc;
-    if (int rc = launch_resize_blend(g.fg, src_bytes, h_geom, B, T, H, W, d_bg_pool, false, P, Hb, Wb, g.bg_idx, g.top, g.left,
+    if (int rc = launch_resize_blend(g.fg, src_bytes, h_geom, 5, B, T, H, W, d_bg_pool, false, P, Hb, Wb, g.bg_idx, g.top, g.left,
                                      g.apply, d_fg_lut, h_bg_mean, h_bg_std, alpha, layout, BGD_OUT_F32, d_out, g.stream))
         return rc;
     return finish_host_blend(d_out, B * T * 3 * H * W, h_checksum, g.stream);

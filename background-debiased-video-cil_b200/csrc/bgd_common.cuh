@@ -138,10 +138,11 @@ int launch_bgmix(const uint8_t *d_fg, const float *d_fg_norm, int64_t B, int64_t
                  const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply,
                  const float *d_lut, const float *h_mean, const float *h_std, double alpha,
                  int layout, int out_dtype, void *d_out, cudaStream_t stream);
-int launch_resize_u8(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t B, int64_t T, int64_t H, int64_t W,
-                     uint8_t *d_out, cudaStream_t stream);
-int launch_resize_blend(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int64_t B, int64_t T, int64_t H,
-                        int64_t W, const void *d_pool, bool pool_is_u8, int64_t P, int64_t Hb, int64_t Wb,
+// geom_cols: 5 (h_geom [B][5]) or 11 (the two-stage form, [B][11]); see resize.cu
+int launch_resize_u8(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int geom_cols, int64_t B, int64_t T,
+                     int64_t H, int64_t W, uint8_t *d_out, cudaStream_t stream);
+int launch_resize_blend(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int geom_cols, int64_t B, int64_t T,
+                        int64_t H, int64_t W, const void *d_pool, bool pool_is_u8, int64_t P, int64_t Hb, int64_t Wb,
                         const int32_t *d_bg_idx, const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply,
                         const float *d_lut, const float *h_mean, const float *h_std, double alpha, int layout, int out_dtype,
                         void *d_out, cudaStream_t stream);

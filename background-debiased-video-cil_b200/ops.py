@@ -24,7 +24,9 @@ built library (``ImportError`` otherwise).  Ops are stream-ordered and never syn
     bgdebias::resize_bilinear(Tensor src, Tensor geom, int T, int H, int W) -> Tensor
     bgdebias::bgmix_resize_blend(Tensor src, Tensor geom, int T, int H, int W, <bgmix_blend arguments>) -> Tensor
         the pipeline's Resize((W, H), keep_ratio=False) (config ..._bgmix_plus_randAug.py:136; cv2 INTER_LINEAR, bit-exact)
-        on packed uint8 crops, alone or fused with the blend.
+        on packed uint8 crops, alone or fused with the blend.  With an 11-column ``geom`` (:data:`TWO_STAGE_COLS`), on
+        native-size frames: Resize(scale=(-1, S)) -> MultiScaleCrop -> Resize((W, H), keep_ratio=False), both resizes
+        bit-exact (``comix_loader.TrainPipeline`` builds the table).
     bgdebias::resize_crop_normalize(Tensor src, Tensor geom, int T, int H, int W, Tensor fg_lut, str layout,
                                     ScalarType? out_dtype=None) -> Tensor
         the evaluation tail Resize(scale=(-1, S)) -> CenterCrop / ThreeCrop -> Normalize -> FormatShape('NCHW') on packed
@@ -427,9 +429,14 @@ def pack_clips(clips, pin: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
     return buf, geom
 
 
-def _check_packed(name: str, src: torch.Tensor, geom: torch.Tensor, cols: int = 5):
+#: Columns of the two-stage geometry: the five of :func:`pack_clips`, the size the clip is resized to, the window of that
+#: resized clip (MultiScaleCrop's offset and crop size) that is resized to the output size.
+TWO_STAGE_COLS = ("offset", "h", "w", "row_stride", "frame_stride", "Hr", "Wr", "y0", "x0", "ch", "cw")
+
+
+def _check_packed(name: str, src: torch.Tensor, geom: torch.Tensor, cols: Tuple[int, ...] = (5,)):
     _require(src.dtype == torch.uint8 and src.dim() == 1, f"{name}: src must be a flat uint8 buffer")
-    _require(geom.dim() == 2 and geom.shape[1] == cols, f"{name}: geom must be int64 [B, {cols}]")
+    _require(geom.dim() == 2 and geom.shape[1] in cols, f"{name}: geom must be int64 [B, {' or '.join(map(str, cols))}]")
     _require(src.numel() % 4 == 0, f"{name}: src must be a multiple of 4 bytes long (ops.pack_clips pads)")
     g = geom.detach().to("cpu", torch.int64).contiguous()
     return src.contiguous(), g, ctypes.cast(g.data_ptr(), ctypes.POINTER(ctypes.c_int64))
@@ -438,17 +445,21 @@ def _check_packed(name: str, src: torch.Tensor, geom: torch.Tensor, cols: int = 
 @torch.library.custom_op("bgdebias::resize_bilinear", mutates_args=(), device_types="cuda")
 def resize_bilinear(src: torch.Tensor, geom: torch.Tensor, T: int, H: int, W: int) -> torch.Tensor:
     """Packed uint8 crops (see :func:`pack_clips`) -> uint8 ``[B, T, H, W, 3]``; every frame equals
-    ``cv2.resize(frame, (W, H), interpolation=cv2.INTER_LINEAR)``, the arithmetic of mmaction's ``Resize``."""
-    src, g, gptr = _check_packed("resize_bilinear", src, geom)
+    ``cv2.resize(frame, (W, H), interpolation=cv2.INTER_LINEAR)``, the arithmetic of mmaction's ``Resize``.
+
+    ``geom`` int64 ``[B, 11]`` (:data:`TWO_STAGE_COLS`): every frame equals
+    ``cv2.resize(cv2.resize(frame, (Wr, Hr))[y0:y0 + ch, x0:x0 + cw], (W, H))``, both INTER_LINEAR."""
+    src, g, gptr = _check_packed("resize_bilinear", src, geom, (5, len(TWO_STAGE_COLS)))
     out = torch.empty((g.shape[0], T, H, W, 3), dtype=torch.uint8, device=src.device)
     with torch.cuda.device(src.device):
-        _cabi.check(_cabi.lib().bgd_resize_bilinear_u8(src.data_ptr(), src.numel(), gptr, g.shape[0], T, H, W, out.data_ptr(),
-                                                       _stream_ptr(src.device)))
+        _cabi.check(_cabi.lib().bgd_resize_bilinear_cols_u8(src.data_ptr(), src.numel(), gptr, g.shape[1], g.shape[0], T, H, W,
+                                                            out.data_ptr(), _stream_ptr(src.device)))
     return out
 
 
 @resize_bilinear.register_fake
 def _(src, geom, T, H, W):
+    _require(geom.dim() == 2 and geom.shape[1] in (5, len(TWO_STAGE_COLS)), "resize_bilinear: geom must be int64 [B, 5 or 11]")
     return src.new_empty((geom.shape[0], T, H, W, 3))
 
 
@@ -457,8 +468,9 @@ def bgmix_resize_blend(src: torch.Tensor, geom: torch.Tensor, T: int, H: int, W:
                        bg_idx: torch.Tensor, top: torch.Tensor, left: torch.Tensor, apply: torch.Tensor, fg_lut: torch.Tensor,
                        bg_mean: torch.Tensor, bg_std: torch.Tensor, alpha: float, layout: str,
                        out_dtype: Optional[torch.dtype] = None) -> torch.Tensor:
-    """``bgmix_blend(resize_bilinear(src, geom, T, H, W), ...)`` in one launch (the resized uint8 batch never exists)."""
-    src, g, gptr = _check_packed("bgmix_resize_blend", src, geom)
+    """``bgmix_blend(resize_bilinear(src, geom, T, H, W), ...)`` in one launch (the resized uint8 batch never exists), for
+    either form of ``geom``."""
+    src, g, gptr = _check_packed("bgmix_resize_blend", src, geom, (5, len(TWO_STAGE_COLS)))
     B = g.shape[0]
     _require(bg_pool.dim() == 4 and bg_pool.shape[1] == 3 and bg_pool.dtype in (torch.float32, torch.uint8),
              "bgmix_resize_blend: bg_pool must be float32 or uint8 [P, 3, Hb, Wb]")
@@ -469,13 +481,15 @@ def bgmix_resize_blend(src: torch.Tensor, geom: torch.Tensor, T: int, H: int, W:
     _require(bg_pool.device == dev, "bgmix_resize_blend: bg_pool must be on the same device as src")
     bg_pool = bg_pool.contiguous()
     with torch.cuda.device(dev):
-        _cabi.check(_cabi.lib().bgd_bgmix_resize_blend_out(src.data_ptr(), src.numel(), gptr, B, T, H, W, bg_pool.data_ptr(),
-                                                           int(bg_pool.dtype == torch.uint8), P, Hb, Wb, *tail, _stream_ptr(dev)))
+        _cabi.check(_cabi.lib().bgd_bgmix_resize_blend_cols_out(src.data_ptr(), src.numel(), gptr, g.shape[1], B, T, H, W,
+                                                                bg_pool.data_ptr(), int(bg_pool.dtype == torch.uint8), P, Hb, Wb,
+                                                                *tail, _stream_ptr(dev)))
     return out
 
 
 @bgmix_resize_blend.register_fake
 def _(src, geom, T, H, W, bg_pool, bg_idx, top, left, apply, fg_lut, bg_mean, bg_std, alpha, layout, out_dtype=None):
+    _require(geom.dim() == 2 and geom.shape[1] in (5, len(TWO_STAGE_COLS)), "bgmix_resize_blend: geom must be int64 [B, 5 or 11]")
     B = geom.shape[0]
     return src.new_empty(_out_shape(B, T, H, W, layout), dtype=_out_spec("bgmix_resize_blend", layout, out_dtype))
 
@@ -488,7 +502,7 @@ def resize_crop_normalize(src: torch.Tensor, geom: torch.Tensor, T: int, H: int,
     ``cv2.resize(frame, (Wr, Hr), interpolation=cv2.INTER_LINEAR)[top:top + H, left:left + W]`` of every frame of its clip,
     normalised through ``fg_lut`` (:func:`make_fg_lut`).  ``layout`` "NTCHW" (``[n, T, 3, H, W]``) or "NTHWC"
     (``[n, T, H, W, 3]``); ``out_dtype`` as :func:`bgmix_blend`.  ``comix_loader.EvalPipeline.geometry`` builds the table."""
-    src, g, gptr = _check_packed("resize_crop_normalize", src, geom, 9)
+    src, g, gptr = _check_packed("resize_crop_normalize", src, geom, (9,))
     _require(layout in ("NTCHW", "NTHWC"), "resize_crop_normalize: layout must be 'NTCHW' or 'NTHWC'")
     out_dt = _out_spec("resize_crop_normalize", layout, out_dtype)
     _check_lut("resize_crop_normalize", fg_lut, src.device)

@@ -322,6 +322,23 @@ int bgd_bgmix_resize_blend_out(const uint8_t *d_src, int64_t src_bytes, const in
                                const float *d_fg_lut, const float *h_bg_mean, const float *h_bg_std,
                                double alpha, int layout, int out_dtype, void *d_out, void *stream);
 
+/* bgd_resize_bilinear_u8 and bgd_bgmix_resize_blend_out with a choice of geometry form: h_geom is HOST int64
+ * [B][geom_cols], geom_cols 5 (the form of those entry points, same results) or 11, the training pipeline's
+ * Resize(scale=(-1, S)) -> MultiScaleCrop -> Resize((W, H), keep_ratio=False) of mmaction2 0.x:
+ *   {the five columns of bgd_resize_bilinear_u8, Hr, Wr, y0, x0, ch, cw}
+ * Entry b is cv2.resize(cv2.resize(frame, (Wr, Hr))[y0:y0+ch, x0:x0+cw], (W, H)) of every frame of its clip, both
+ * resizes INTER_LINEAR and bit-exact, the first rounded to uint8 as cv2 rounds it; the intermediate images never exist.
+ * Needs Hr, Wr, ch, cw >= 1, y0, x0 >= 0, y0 + ch <= Hr, x0 + cw <= Wr and (h - 1) * row stride + 3 * max(w, 2) < 2^31.
+ * Every other argument as bgd_resize_bilinear_u8 / bgd_bgmix_resize_blend_out. */
+int bgd_resize_bilinear_cols_u8(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int geom_cols,
+                                int64_t B, int64_t T, int64_t H, int64_t W, uint8_t *d_out, void *stream);
+int bgd_bgmix_resize_blend_cols_out(const uint8_t *d_src, int64_t src_bytes, const int64_t *h_geom, int geom_cols,
+                                    int64_t B, int64_t T, int64_t H, int64_t W, const void *d_bg_pool,
+                                    int pool_is_u8, int64_t P, int64_t Hb, int64_t Wb, const int32_t *d_bg_idx,
+                                    const int32_t *d_top, const int32_t *d_left, const uint8_t *d_apply,
+                                    const float *d_fg_lut, const float *h_bg_mean, const float *h_bg_std,
+                                    double alpha, int layout, int out_dtype, void *d_out, void *stream);
+
 /* The evaluation pipeline's tail, with no blend: Resize(scale=(-1, S), keep_ratio=True) -> CenterCrop / ThreeCrop ->
  * Normalize(to_bgr=False) -> FormatShape('NCHW') of mmaction2 0.x (the val / test / feature datasets of a CIL run), so that
  * the DataLoader can ship the decoded uint8 frames.  Each output entry resizes one source clip to Hr x Wr (cv2.resize,
